@@ -2,7 +2,7 @@
 """Benchmark of the synthesis hot path (BASELINE.json metric: audio-sec/sec, JP-Extra 44.1 kHz,
 batch 32 per GPU; p50 latency of a 5 s utterance).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the full JP-Extra synthesizer (enc_p, duration predictors, length
 regulator, flow, HiFi-GAN decoder) over one batch of 32 synthetic ~8 s utterances (BASELINE config 4
@@ -191,6 +191,26 @@ def sources_digest() -> str:
     return h.hexdigest()
 
 
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs
+
+
+def dump_outputs(out_dir: str, waves, suffix: str = "") -> None:
+    """Writes one batch's waveforms as sbv2_batch_download hands them to its caller: the samples of every utterance back to
+    back (audio, float32) and the samples per utterance (audio_lengths, float64).  Past DUMP_LIMIT bytes, audio keeps a fixed,
+    seeded sample of the samples, in order, and audio_index (float64) gives their positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    audio = np.concatenate(waves).astype(np.float32, copy=False)
+    arrays = {"audio_lengths": np.array([w.size for w in waves], np.float64)}
+    if audio.nbytes + arrays["audio_lengths"].nbytes > DUMP_LIMIT:
+        k = (DUMP_LIMIT - arrays["audio_lengths"].nbytes - 1024) // 12  # 4 B per sample + 8 B per index; 1 KB for the headers
+        idx = np.sort(np.random.default_rng(0).choice(audio.size, size=k, replace=False))
+        arrays["audio_index"] = idx.astype(np.float64)
+        audio = audio[idx]
+    arrays["audio"] = audio
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def wall(fn, n, warm=3):
     for _ in range(warm):
         fn()
@@ -278,7 +298,14 @@ def main():
     ap.add_argument("--flow", default="transformer", choices=["transformer", "wn"],
                     help="flow variant of the synthetic model: JP-Extra's transformer coupling layers (the headline) or the WN "
                          "residual-coupling layers north_star names (non-JP-Extra Style-Bert-VITS2 models)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the waveforms of the last timed batch of replica 0 to DIR as .npy "
+                         "(see dump_outputs); the same arguments give the same inputs, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -388,6 +415,10 @@ def main():
     ms, launches = timed_kernel_run(R, args.steps)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        # replica 0 runs at least one of the timed steps, and its device noise is seeded and advances per run by an amount
+        # its inputs set, so its last batch depends on the arguments only
+        dump_outputs(args.dump_outputs, dbs[0].download(), f"_rank{rank}" if world > 1 else "")
     # one replica on one stream (no overlap between replicas): what a single in-flight batch achieves
     ms_single, _ = timed_kernel_run(1, max(2, args.steps // 2))
     single_steps = max(2, args.steps // 2)

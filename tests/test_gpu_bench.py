@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -12,9 +13,9 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
 
 
-def test_bench_line_has_the_contract_keys(lib_built):
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--batch", "4", "--steps", "2", "--warmup", "3", "--configs", "cfg1,cfg3"],
-                       capture_output=True, text=True, timeout=900)
+def test_bench_line_has_the_contract_keys(lib_built, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--batch", "4", "--steps", "2", "--warmup", "3", "--configs", "cfg1,cfg3",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
     for k in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
@@ -29,3 +30,8 @@ def test_bench_line_has_the_contract_keys(lib_built):
     assert line["single_stream"]["value"] > 0
     assert line["configs"]["cfg1"]["latency_ms_p50"] > 0 and line["configs"]["cfg3"]["decoder_ms"] > 0
     assert line["e2e"]["single_replica_rank0"] > 0 and line["e2e"]["single_replica_pageable_inputs_rank0"] > 0
+    # --dump-outputs: the last timed batch of 4 utterances, whole (well under the size limit), finite and not silent
+    audio, lengths = np.load(tmp_path / "audio.npy"), np.load(tmp_path / "audio_lengths.npy")
+    assert sorted(os.listdir(tmp_path)) == ["audio.npy", "audio_lengths.npy"]
+    assert audio.dtype == np.float32 and lengths.dtype == np.float64 and lengths.size == 4 and lengths.sum() == audio.size
+    assert np.isfinite(audio).all() and np.abs(audio).max() > 0
