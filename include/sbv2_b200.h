@@ -121,7 +121,9 @@ int sbv2_model_seed(sbv2_model* synth, uint64_t seed);
  * noise_zp: float32 [192, noise_zp_frames] channel-major (only the first T_y frames are used; the
  * call fails with SBV2_ERR_INVALID_ARGUMENT if T_y > noise_zp_frames).
  * out_durations: int32 [t_x] (= ceil(w)), out_frame2ph: int32, library-allocated [T_y],
- * both optional (NULL to skip). */
+ * both optional (NULL to skip).  out_frame2ph[j] is the phoneme that owns frame j, or -1 for a frame
+ * that belongs to no phoneme: when every duration is 0 (length_scale = 0) T_y is 1 and that frame
+ * is synthesized from a zero prior mean and log-scale, as the ONNX graph does. */
 int sbv2_synthesize_with_noise(sbv2_model* synth, const float* bert, const int64_t* x_tst,
                                const int64_t* tones, const int64_t* lang_ids, int64_t t_x, int64_t sid,
                                const float* style_vec, float sdp_ratio, float length_scale,

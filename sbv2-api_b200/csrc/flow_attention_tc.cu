@@ -438,6 +438,15 @@ __global__ void __launch_bounds__(288, 1) flow_attention_tc_kernel(__half* out, 
 
 }  // namespace
 
+std::vector<__half> pack_flow_rel_table(const float* table, int window, int head_dim) {
+  const int R = 2 * window + 1;
+  if (head_dim != D || R > RP) fail(SBV2_ERR_UNSUPPORTED, "tensor-core attention: head_dim must be 96 and window at most 7");
+  std::vector<__half> pk(size_t(DP) * RP * 8, __float2half(0.f));
+  for (int r = 0; r < R; ++r)
+    for (int d = 0; d < D; ++d) pk[(size_t(d / 8) * RP + r) * 8 + d % 8] = __float2half_rn(table[size_t(r) * D + d]);
+  return pk;
+}
+
 // rel_k_p / rel_v_p: fp16 [D/8][16][8] packings of emb_rel_k / emb_rel_v ([2w+1, D], rows >= 2w+1 zero)
 void launch_flow_attention_tc(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const __half* rel_k_p, const __half* rel_v_p,
                               int heads, int head_dim, int window, const PlanarSegs& s, long long* trace) {

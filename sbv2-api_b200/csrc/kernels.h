@@ -136,7 +136,7 @@ void launch_convflow_spline(const LaunchCtx& ctx, float* z, const float* proj, i
 void launch_sdp_affine(const LaunchCtx& ctx, float* z, const float* m, const float* logs, int rows);
 
 // durations: logw = sdp*ratio + dp*(1-ratio); w = exp(logw)*length_scale; d = ceil(w);
-// cum = inclusive scan per utterance; ylen[b] = max(1, sum d)
+// cum = inclusive scan per utterance; ylen[b] = min(max(1, sum d), INT_MAX) (the sum is formed in 64 bits)
 void launch_durations(const LaunchCtx& ctx, const float* logw_dp, const float* z_sdp /*[rows,2] or null*/,
                       const float* sdp_ratio_utt, const float* length_scale_utt, float* w_out, int* dur, int* cum,
                       int* ylen, const Segs& seg);
@@ -187,6 +187,8 @@ void launch_rel_attention_planar(const LaunchCtx& ctx, __half* ctx_out, const __
 // same on tcgen05 tensor cores (head_dim 96, window 4); rel_k_p / rel_v_p: fp16 [D/8][16][8] packings
 void launch_flow_attention_tc(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const __half* rel_k_p, const __half* rel_v_p,
                               int heads, int head_dim, int window, const PlanarSegs& s, long long* trace = nullptr);
+// host: fp32 relative table [2*window+1][head_dim] -> the fp16 [D/8][16][8] packing launch_flow_attention_tc reads
+std::vector<__half> pack_flow_rel_table(const float* table, int window, int head_dim);
 // z[row, C/2:] -= m32 (planar fp32, C/2 channels)
 void launch_coupling_sub_planar(const LaunchCtx& ctx, float* z, const float* m32, int C, const PlanarSegs& s);
 }  // namespace sbv2

@@ -2,6 +2,7 @@
 // alignment) and the glue around the tensor-core kernels.  See kernels.h for layouts.
 #include <math_constants.h>
 
+#include <climits>
 #include <cstdlib>
 
 #include "kernels.h"
@@ -630,7 +631,9 @@ __global__ void durations_kernel(const float* logw_dp, const float* z_sdp, const
   int len = seg.len[b];
   int base = seg.start[b];
   float ratio = sdp_ratio[b], ls = length_scale[b];
-  int carry = 0;
+  // 64-bit total: 2^20 phonemes of up to 1e6 frames each exceed int32.  ylen saturates at INT_MAX, which the host
+  // rejects as too long; whenever it accepts the batch, every prefix in cum fits in int32.
+  long long carry = 0;
   for (int t0 = 0; t0 < len; t0 += 32) {
     int t = t0 + lane;
     int d = 0;
@@ -657,11 +660,10 @@ __global__ void durations_kernel(const float* logw_dp, const float* z_sdp, const
       int n = __shfl_up_sync(0xffffffffu, s, o);
       if (lane >= o) s += n;
     }
-    s += carry;
-    if (t < len) cum[base + t] = s;
-    carry = __shfl_sync(0xffffffffu, s, 31);
+    if (t < len) cum[base + t] = (int)(carry + s);
+    carry += __shfl_sync(0xffffffffu, s, 31);  // one chunk: at most 32e6
   }
-  if (lane == 0) ylen[b] = carry > 1 ? carry : 1;
+  if (lane == 0) ylen[b] = (int)min(max(carry, 1LL), (long long)INT_MAX);
 }
 
 __global__ void expand_kernel(float* z_p, int* frame2ph, const float* stats, const int* cum, const float* eps,

@@ -877,9 +877,7 @@ sbv2_model* create_synth_model(const OnnxModel& m, int device) {
           CUDA_CHECK(cudaMemcpy(hk.data(), Lw.rel_k, hk.size() * 4, cudaMemcpyDeviceToHost));
           CUDA_CHECK(cudaMemcpy(hv.data(), Lw.rel_v, hv.size() * 4, cudaMemcpyDeviceToHost));
           auto pack = [&](const std::vector<float>& src) {
-            std::vector<__half> pk(size_t(D / 8) * 16 * 8, __float2half(0.f));
-            for (int r = 0; r < R; ++r)
-              for (int d = 0; d < D; ++d) pk[(size_t(d / 8) * 16 + r) * 8 + d % 8] = __float2half_rn(src[size_t(r) * D + d]);
+            const std::vector<__half> pk = pack_flow_rel_table(src.data(), E0.window, D);
             return static_cast<__half*>(M->upload_bytes(pk.data(), pk.size() * 2));
           };
           M->flow_tc[i].layers[l].rel_k_p = pack(hk);

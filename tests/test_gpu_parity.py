@@ -255,8 +255,27 @@ def test_error_paths(tiny, S):
     with pytest.raises(S.Sbv2Error) as e:
         S.Model(assets.model_proto({"foo": np.zeros(4, np.float32)}), bert=False)
     assert e.value.status == S.ERR_UNSUPPORTED
+    # 2201 phonemes at the 1e6-frame duration clamp: 2.2e9 frames, more than an int32 total (and 2^31 samples) can hold
+    long = dict(util.to_api(util.make_utterance(hp, 2201, seed=5, max_frames=1)), length_scale=1e30, noise_zp=None)
+    with pytest.raises(S.Sbv2Error) as e:
+        model.synthesize_batch([long])
+    assert e.value.status == S.ERR_INVALID_ARGUMENT and "too long" in e.value.message
     # the model is still usable after errors
     assert run_gpu(model, u)[0].size > 0
+
+
+def test_zero_durations(full):
+    """length_scale = 0: every duration is 0, T_y is clamped to 1 and that frame belongs to no phoneme (frame2ph -1); the
+    oracle synthesizes it from m_p = logs_p = 0."""
+    hp, oracle, model = full
+    u = util.make_utterance(hp, 7, seed=17, sdp_ratio=0.4, length_scale=0.0)
+    ref, inter = util.oracle_run(oracle, u)
+    audio, dur, f2p = run_gpu(model, u)
+    assert (dur == 0).all() and (inter["w_ceil"] == 0).all()
+    assert np.array_equal(f2p, [-1])
+    assert audio.shape[0] == ref.shape[-1] == 512
+    err = np.abs(audio - ref[0, 0].numpy()).max()
+    assert err <= WAVE_TOL, f"waveform max-abs {err:.3e}"
 
 
 def test_internal_noise_is_seeded(tiny):
