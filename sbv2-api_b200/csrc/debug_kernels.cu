@@ -1,12 +1,14 @@
 // Unit-test hooks of the synthesizer kernels between the text encoder and the decoder: the flow's window attention
 // (tensor-core and planar CUDA-core), the text encoder's fp32 attention, the inverse spline of the stochastic duration
-// predictor, and the length regulator.  Linked into libsbv2_b200_debug.so only (build.py DEBUG_ONLY).  Every hook runs
-// on its own stream, takes host arrays and returns host arrays before it returns; tests/test_gpu_synth_kernels.py
-// compares the results with float64 evaluations of oracle/vits.py.
+// predictor, the length regulator, and the HiFi-GAN decoder's tensor-core layers and conv_post.  Linked into
+// libsbv2_b200_debug.so only (build.py DEBUG_ONLY).  Every hook runs on its own stream, takes host arrays and returns host
+// arrays before it returns; tests/test_gpu_synth_kernels.py and tests/test_gpu_decoder_kernels.py compare the results
+// with float64 references.
 #include <cuda_fp16.h>
 
 #include <algorithm>
 #include <climits>
+#include <cstring>
 
 #include "model.h"
 #include "umma_conv.h"
@@ -208,5 +210,181 @@ extern "C" int sbv2_debug_durations(const float* logw_dp, const float* z_sdp, co
     launch_expand(ctx, d_zp, d_f2p, upload(owner, zero_f.data(), rows * 2), d_cum, d_zero_y, upload(owner, zero_f.data(), size_t(n)), 1, xseg,
                   yseg);
     download(owner, frame2ph, d_f2p, size_t(ny));
+  });
+}
+
+// ---- the decoder's tensor-core layers ---------------------------------------------------------------------------
+namespace {
+using namespace sbv2;
+
+constexpr uint16_t kHalfSentinel = 0x7D5A;       // an fp16 NaN payload: no kernel writes it
+constexpr uint32_t kFloatSentinel = 0x7FC0A5A5u;  // an fp32 NaN payload
+
+// packed fp32 [sum(lens), C] -> planar fp16 [C/8][rows_tot][8] with zero gaps (launch_zero_gaps, launch_to_planar)
+__half* planar_input(sbv2_model& owner, const float* packed, int C, const int* d_start, const Geom& g, int n) {
+  const LaunchCtx ctx = owner.ctx();
+  long long rows = 0;
+  for (int b = 0; b < n; ++b) rows += g.len[size_t(b)];
+  std::vector<uint16_t> zero(size_t(C / 8) * g.rows_tot * 8, 0);
+  __half* d = reinterpret_cast<__half*>(upload(owner, zero.data(), zero.size()));
+  launch_zero_gaps(ctx, d, C, g, n);
+  launch_to_planar(ctx, d, upload(owner, packed, size_t(rows) * C), C, C, d_start, g, n, ACT_NONE);
+  return d;
+}
+
+}  // namespace
+
+// One tensor-core layer (launch_umma) on a ragged batch, as the HiFi-GAN decoder runs it.
+//   up == 0: Conv1d, w [cout][cin][k], dilation dil: make_conv1d_layer(mt_pref, nb_max); utterance b has lens[b] rows.
+//   up == u: ConvTranspose1d, w [cin][cout][k], stride u, padding (k - u) / 2: make_upsample_layer(mt_pref), launched
+//            with out_mul = u; utterance b has lens[b] input rows and u * lens[b] output rows.
+// bias [cout] or null.  x: packed fp32 [sum(lens), cin], stored as planar fp16 with zero gaps and no activation (pass the
+// values the layer reads).  Epilogue inputs, all optional: bias_utt [n][cout]; residual = the input (cin == cout);
+// res2 / res3 (both or neither): packed fp32 [output rows, cout] stored the same way, with out_div; accum_mode (UAccum)
+// with accum: packed fp32 [output rows, cout] that pre-fills the planar fp32 accumulate buffer and receives it back, and
+// accum_div; act_out (Act).
+// out: packed fp32 [output rows, cout] <- the fp16 output (left untouched for UACC_SET / UACC_ADD, which store none).
+// The output buffer holds a sentinel in every row before the launch, the accumulate buffer outside the utterance rows:
+// pad_rows[0] / [1] count the planar rows outside every utterance that the layer wrote in either.  cfg[3]: the layer's
+// mt (128-row tiles per work item, in input rows), nb and n_nblk.
+extern "C" int sbv2_debug_umma_layer(const float* w, const float* bias, int cin, int cout, int k, int dil, int up, int mt_pref,
+                                     int nb_max, const float* x, const int* lens, int n, const float* bias_utt, int residual,
+                                     const float* res2, const float* res3, float out_div, int accum_mode, float* accum,
+                                     float accum_div, int act_out, float* out, long long* pad_rows, int* cfg) {
+  return guarded([&] {
+    SBV2_REQUIRE(w && x && lens && out && n > 0 && cin > 0 && cout > 0 && k > 0 && up >= 0, "bad arguments");
+    SBV2_REQUIRE(!residual || cin == cout, "the residual is the layer's input: needs cin == cout");
+    SBV2_REQUIRE(!res2 == !res3, "res2 and res3 go together");
+    SBV2_REQUIRE(accum_mode >= UACC_NONE && accum_mode <= UACC_FINAL && (accum_mode == UACC_NONE || accum),
+                 "an accumulate mode needs the accumulate buffer");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    HostConv hc;
+    hc.d0 = up ? cin : cout;
+    hc.d1 = up ? cout : cin;
+    hc.k = k;
+    hc.w.assign(w, w + size_t(cin) * cout * k);
+    if (bias) hc.b.assign(bias, bias + cout);
+    const ConvLayer L = up ? make_upsample_layer(&owner, hc, up, mt_pref) : make_conv1d_layer(&owner, hc, dil, mt_pref, nb_max);
+    if (cfg) {
+      cfg[0] = L.mt;
+      cfg[1] = L.nb;
+      cfg[2] = L.n_nblk;
+    }
+    const int mul = up ? up : 1;
+    std::vector<int> ystart(lens, lens + n), ostart(lens, lens + n), ylen(lens, lens + n), muls{1};
+    if (up) muls.push_back(up);
+    long long rows = 0;
+    for (int b = 0; b < n; ++b) {
+      SBV2_REQUIRE(lens[b] >= 1, "utterance lengths must be positive");
+      ystart[size_t(b)] = int(rows);
+      ostart[size_t(b)] = int(rows * mul);
+      rows += lens[b];
+      SBV2_REQUIRE(rows * mul < INT_MAX, "too many rows");
+    }
+    DBuf meta;
+    PinnedBuf pin;
+    meta.stream = owner.stream;
+    BatchGeom bg = build_geoms(&owner, meta, pin, ystart, ylen, muls);
+    const Geom& Gi = bg.g[0];
+    const Geom& Go = bg.g.back();
+    const int* d_ostart = upload(owner, ostart.data(), size_t(n));
+    const size_t oplane = size_t(Go.rows_tot) * 8;
+    std::vector<char> in_utt(size_t(Go.rows_tot), 0);
+    for (int b = 0; b < n; ++b)
+      for (int t = 0; t < Go.len[size_t(b)]; ++t) in_utt[size_t(Go.pstart[size_t(b)]) + t] = 1;
+
+    ConvCall c;
+    c.in = planar_input(owner, x, cin, bg.d_ystart, Gi, n);
+    if (residual) c.residual = c.in;
+    if (res2) {
+      c.residual2 = planar_input(owner, res2, cout, d_ostart, Go, n);
+      c.residual3 = planar_input(owner, res3, cout, d_ostart, Go, n);
+      c.out_div = out_div;
+    }
+    if (bias_utt) c.bias_utt = upload(owner, bias_utt, size_t(n) * cout);
+    std::vector<uint16_t> ho(size_t(cout / 8) * oplane, kHalfSentinel);
+    __half* d_out = reinterpret_cast<__half*>(upload(owner, ho.data(), ho.size()));
+    const bool stores = accum_mode != UACC_SET && accum_mode != UACC_ADD;
+    c.out = stores ? d_out : nullptr;
+    std::vector<uint32_t> ha;
+    float* d_acc = nullptr;
+    if (accum_mode != UACC_NONE) {
+      ha.assign(size_t(cout / 8) * oplane, kFloatSentinel);
+      for (int b = 0; b < n; ++b)
+        for (int t = 0; t < Go.len[size_t(b)]; ++t)
+          for (int co = 0; co < cout; ++co)
+            memcpy(&ha[size_t(co / 8) * oplane + (size_t(Go.pstart[size_t(b)]) + t) * 8 + co % 8],
+                   accum + (size_t(ostart[size_t(b)]) + t) * cout + co, 4);
+      d_acc = reinterpret_cast<float*>(upload(owner, ha.data(), ha.size()));
+      c.accum = d_acc;
+      c.accum_mode = accum_mode;
+      c.accum_div = accum_div;
+    }
+    c.act_out = act_out;
+    c.out_mul = mul;
+    launch_umma(ctx, L, Gi, Go, c, n);
+    download(owner, ho.data(), reinterpret_cast<const uint16_t*>(d_out), ho.size());
+    if (d_acc) download(owner, ha.data(), reinterpret_cast<const uint32_t*>(d_acc), ha.size());
+    for (int b = 0; b < n; ++b)
+      for (int t = 0; t < Go.len[size_t(b)]; ++t) {
+        const size_t pr = size_t(Go.pstart[size_t(b)]) + t, orow = size_t(ostart[size_t(b)]) + t;
+        for (int co = 0; co < cout; ++co) {
+          const size_t e = size_t(co / 8) * oplane + pr * 8 + co % 8;
+          if (stores) out[orow * cout + co] = __half2float(__ushort_as_half(ho[e]));
+          if (d_acc) memcpy(accum + orow * cout + co, &ha[e], 4);
+        }
+      }
+    long long written[2] = {0, 0};
+    for (size_t pr = 0; pr < size_t(Go.rows_tot); ++pr) {
+      if (in_utt[pr]) continue;
+      bool wo = false, wa = false;
+      for (int e = 0; e < cout; ++e) {
+        const size_t i = size_t(e / 8) * oplane + pr * 8 + e % 8;
+        wo |= ho[i] != kHalfSentinel;
+        wa |= d_acc && ha[i] != kFloatSentinel;
+      }
+      written[0] += wo ? 1 : 0;
+      written[1] += wa ? 1 : 0;
+    }
+    if (pad_rows) {
+      pad_rows[0] = written[0];
+      pad_rows[1] = written[1];
+    }
+  });
+}
+
+// The decoder's conv_post (launch_dec_post_planar) on a ragged batch.  x: packed fp32 [sum(lens), C] (the lrelu(0.01)
+// values it reads), stored as planar fp16 with zero gaps; w fp32 [C][k]; utterance b's samples go to
+// wave[wstart[b] .. wstart[b] + lens[b]).  wave [wave_len] in / out: the whole buffer goes up and comes back, so every
+// sample outside the utterances keeps what the caller put there unless the kernel wrote it.  force_generic: the generic
+// kernel also at C = 16, k = 7.
+extern "C" int sbv2_debug_dec_post(const float* x, const int* lens, const long long* wstart, int n, const float* w, int C, int k,
+                                   int force_generic, float* wave, long long wave_len) {
+  return guarded([&] {
+    SBV2_REQUIRE(x && lens && wstart && w && wave && n > 0 && C > 0 && C % 8 == 0 && k > 0 && k % 2 == 1, "bad arguments");
+    sbv2_model owner;
+    open_owner(owner);
+    std::vector<int> ystart(lens, lens + n), ylen(lens, lens + n), muls{1};
+    std::vector<long long> ws(wstart, wstart + n);
+    long long rows = 0;
+    for (int b = 0; b < n; ++b) {
+      SBV2_REQUIRE(lens[b] >= 1, "utterance lengths must be positive");
+      SBV2_REQUIRE(wstart[b] >= 0 && wstart[b] + lens[b] <= wave_len, "utterance outside the waveform buffer");
+      ystart[size_t(b)] = int(rows);
+      rows += lens[b];
+      SBV2_REQUIRE(rows < INT_MAX, "too many rows");
+    }
+    DBuf meta;
+    PinnedBuf pin;
+    meta.stream = owner.stream;
+    BatchGeom bg = build_geoms(&owner, meta, pin, ystart, ylen, muls, nullptr, false, &ws);
+    const Geom& G = bg.g[0];
+    const __half* d_x = planar_input(owner, x, C, bg.d_ystart, G, n);
+    const std::vector<float> wh(w, w + size_t(C) * k);
+    float* d_wave = upload(owner, wave, size_t(wave_len));
+    launch_dec_post_planar(owner.ctx(), d_wave, d_x, G, bg.d_wstart, n, upload(owner, wh.data(), wh.size()), wh, C, k, force_generic != 0);
+    download(owner, wave, d_wave, size_t(wave_len));
   });
 }

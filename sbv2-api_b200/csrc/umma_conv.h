@@ -190,5 +190,11 @@ void umma_decoder_free(UmmaDecoder* d);
 void umma_decoder_run(UmmaDecoder* d, sbv2_model* owner, const float* z, const float* g, int B,
                       const std::vector<int>& ystart, const std::vector<int>& ylen, float* wave,
                       const std::vector<long long>* wstart = nullptr);
+// The decoder's conv_post: wave[wstart[b] + t] = tanh(sum_j sum_c w[c][j] * x[t + j - (k-1)/2][c]) for t < len[b] of
+// geometry g.  x: planar fp16, already lrelu(0.01)-activated, zero gap rows (the kernels read the halo without a bounds
+// test).  d_w: device fp32 [C][k]; w_host: the same values, which the 16 x 7 kernel takes as constant-bank operands.
+// force_generic: run the generic kernel at 16 x 7 too (it sums in the same order: bit-identical results).
+void launch_dec_post_planar(const LaunchCtx& ctx, float* wave, const __half* x, const Geom& g, const int* d_wstart, int n_utt,
+                            const float* d_w, const std::vector<float>& w_host, int C, int k, bool force_generic);
 
 }  // namespace sbv2

@@ -101,6 +101,22 @@ __global__ void __launch_bounds__(POST_T) post_planar_const_kernel(float* wave, 
 
 }  // namespace
 
+void launch_dec_post_planar(const LaunchCtx& ctx, float* wave, const __half* x, const Geom& g, const int* d_wstart, int n_utt,
+                            const float* d_w, const std::vector<float>& w_host, int C, int k, bool force_generic) {
+  dim3 grid((g.max_len + POST_T - 1) / POST_T, n_utt);
+  if (C == 16 && k == 7 && !force_generic) {
+    PostWeights<16, 7> pw;
+    for (int c = 0; c < 16; ++c)
+      for (int j = 0; j < 7; ++j) pw.w[j][c] = w_host[size_t(c) * 7 + j];
+    post_planar_const_kernel<16, 7><<<grid, POST_T, 0, ctx.stream>>>(wave, x, g.rows_tot * 8, pw, g.d_pstart, d_wstart, g.d_len);
+  } else {
+    const size_t smem = ((sizeof(float) * C * k + 15) & ~size_t(15)) + size_t(C / 8) * (POST_T + k - 1) * 16;
+    post_planar_kernel<<<grid, POST_T, smem, ctx.stream>>>(wave, x, g.rows_tot * 8, d_w, C, k, g.d_pstart, d_wstart, g.d_len);
+  }
+  CUDA_CHECK(cudaGetLastError());
+  ctx.count();
+}
+
 // ---- decoder plan -----------------------------------------------------------------------------------------
 struct UmmaDecoder {
   int gin = 0, cin0 = 0, c0 = 0, n_stages = 0, per = 0, post_c = 0, post_k = 0;
@@ -362,22 +378,7 @@ void umma_decoder_run(UmmaDecoder* D, sbv2_model* owner, const float* z, const f
       }
     }
   }
-  const Geom& GL = bg.g.back();
-  {
-    dim3 grid((GL.max_len + POST_T - 1) / POST_T, B);
-    if (D->post_c == 16 && D->post_k == 7) {
-      PostWeights<16, 7> pw;
-      for (int c = 0; c < 16; ++c)
-        for (int j = 0; j < 7; ++j) pw.w[j][c] = D->post_w_host[size_t(c) * 7 + j];
-      post_planar_const_kernel<16, 7><<<grid, POST_T, 0, ctx.stream>>>(wave, xs, GL.rows_tot * 8, pw, GL.d_pstart, bg.d_wstart, GL.d_len);
-    } else {
-      const size_t smem = ((sizeof(float) * D->post_c * D->post_k + 15) & ~size_t(15)) + size_t(D->post_c / 8) * (POST_T + D->post_k - 1) * 16;
-      post_planar_kernel<<<grid, POST_T, smem, ctx.stream>>>(wave, xs, GL.rows_tot * 8, D->post_w, D->post_c, D->post_k, GL.d_pstart,
-                                                             bg.d_wstart, GL.d_len);
-    }
-    CUDA_CHECK(cudaGetLastError());
-    ctx.count();
-  }
+  launch_dec_post_planar(ctx, wave, xs, bg.g.back(), bg.d_wstart, B, D->post_w, D->post_w_host, D->post_c, D->post_k, false);
   // the pinned geometry blob is rewritten by the next run: make sure its upload finished
   // (it did: every kernel above depends on it and the caller synchronises before returning results)
 }

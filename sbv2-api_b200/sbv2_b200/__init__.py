@@ -132,8 +132,8 @@ _debug_lib = None
 
 def debug_lib() -> C.CDLL:
     """libsbv2_b200_debug.so: the same objects plus the kernel unit-test / tracing hooks (sbv2_debug_conv_compare,
-    _conv_trace, _pair_compare, _attn_trace, _mma_rate*, _flow_attention, _rel_attention, _convflow_spline, _durations),
-    which the product library does not export."""
+    _conv_trace, _pair_compare, _attn_trace, _mma_rate*, _flow_attention, _rel_attention, _convflow_spline, _durations,
+    _umma_layer, _dec_post), which the product library does not export."""
     global _debug_lib
     if _debug_lib is None:
         path = os.path.join(_HERE, "libsbv2_b200_debug.so")

@@ -1,8 +1,9 @@
 """GPU unit tests of individual tensor-core kernels through their debug hooks (run with -m gpu on a B200).
 
 * fused ResBlock pair (umma_pair.cu) against the two unfused tensor-core convs (bit-identical: same fp16
-  rounding points, same fp32 accumulation order) and against a numpy fp32 evaluation of
-  oracle/vits.py ResBlock1 (one conv1/conv2 pair), on ragged batches that exercise tile boundaries;
+  rounding points, same fp32 accumulation order), against a numpy fp32 evaluation of
+  oracle/vits.py ResBlock1 (one conv1/conv2 pair), and per element against a float64 evaluation with the bars of
+  test_gpu_decoder_kernels.py, on ragged batches that exercise tile boundaries;
 * split-fp16 text-encoder convs against the CUDA-core fp32 path of the same model.
 """
 import ctypes as C
@@ -12,6 +13,7 @@ import numpy as np
 import pytest
 
 import util
+from test_gpu_decoder_kernels import KAPPA, conv_offs, taps_ref, ulp16, xrec
 from util import ov
 
 pytestmark = pytest.mark.gpu
@@ -52,7 +54,8 @@ def f16(a):
 
 
 @pytest.mark.parametrize("c,k,dil,mrf", [(16, 3, 1, 0), (16, 11, 5, 0), (16, 7, 3, 1), (32, 3, 5, 0), (32, 11, 1, 0), (32, 7, 5, 1),
-                                         (64, 3, 1, 0), (64, 7, 3, 0), (64, 11, 5, 0), (64, 11, 5, 1)])
+                                         (64, 3, 1, 0), (64, 7, 3, 0), (64, 11, 5, 0), (64, 11, 5, 1),
+                                         (128, 3, 1, 0), (128, 7, 3, 0), (128, 3, 5, 1), (128, 7, 5, 1)])
 def test_fused_resblock_pair(S, c, k, dil, mrf):
     rng = np.random.default_rng(c * 100 + k * 10 + dil)
     lens = np.asarray([50, 1, 700, 1300, 129, 2500, 1022, 1023], np.int32)  # tile-edge lengths included
@@ -86,6 +89,26 @@ def test_fused_resblock_pair(S, c, k, dil, mrf):
         ref = (xr + np.where(yb >= 0, yb, yb * 10.0) + ref) / 3.0
     ref = lrelu(ref)
     assert np.abs(fused - ref).max() <= 4e-3 * max(1.0, np.abs(ref).max())  # fp16 output rounding of values up to ~6
+    # float64 per element.  t1 is rounded to fp16 as the kernel stores it; the kernel's fp32 t1 (off by up to KAPPA * its
+    # sum of |terms|) may round to the neighbouring fp16 value, which conv2 weighs with |w2|.
+    p1, m1 = taps_ref(y, w1, conv_offs(k, dil), lens)
+    p1 += b1
+    m1 += np.abs(b1)
+    t1 = f16(lrelu(p1))
+    e1 = KAPPA * m1 + ulp16(np.abs(t1) + KAPPA * m1)
+    v, mag = taps_ref(t1, w2, conv_offs(k, 1), lens)
+    v += b2 + xr
+    mag += np.abs(b2) + np.abs(xr)
+    if mrf:
+        rb = xrec(f16(x))
+        v = ((xr + rb) + v) / 3.0
+        mag += np.abs(xr) + np.abs(rb)
+    ref64 = lrelu(v)
+    bar = ulp16(ref64) + KAPPA * mag + taps_ref(e1, np.abs(w2), conv_offs(k, 1), lens)[0]
+    err = np.abs(fused - ref64) - bar
+    i = np.unravel_index(np.argmax(err), err.shape)
+    print(f"pair C{c} k{k} d{dil} mrf{mrf}: max |err| / bar = {float((np.abs(fused - ref64) / bar).max()):.3f}")
+    assert err[i] <= 0, f"element {i}: fused {fused[i]!r}, float64 {ref64[i]!r}, bar {bar[i]:.3e}"
 
 
 def test_text_split_convs_match_fp32_path(S):
