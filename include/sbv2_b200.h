@@ -85,13 +85,14 @@ int sbv2_model_describe(const sbv2_model* model, const char** json);
 /* input_ids, attention_mask: int64 [t_tok].  out: float32 [t_tok, hidden] (hidden = 1024 for
  * deberta-v2-large), caller-allocated.  Output = hidden_states[-3] of batch element 0
  * (scripts/convert/convert_deberta.py:34).
- * Restrictions the ONNX graph does not have: at most 512 tokens (the checkpoint's max_position_embeddings; longer inputs
- * return SBV2_ERR_INVALID_ARGUMENT), and attention_mask must be a prefix of ones (right padding; a mask with holes returns
+ * Restrictions the ONNX graph does not have: at most 32768 tokens per sequence (longer inputs return
+ * SBV2_ERR_INVALID_ARGUMENT; every relative distance beyond +-512 reads the outermost position bucket, as in the graph),
+ * and attention_mask must be a prefix of ones (right padding; a mask with holes returns
  * SBV2_ERR_UNSUPPORTED) — the reference's tokenizer only ever produces all-ones masks (tts_util.rs:120-128).
  * Numerics: SBV2_B200_BERT (read at sbv2_model_create) = "exact" (default: two-term fp16 operand splits, fp32 activations;
  * features reproduce HF fp32 to ~3e-4 and the synthesizer's durations exactly) or "fp16" (single-term operands, ~2x
  * faster, ~1 duration in 2000 differs downstream).  The disentangled attention runs on the tensor cores in both modes for
- * every length up to 512 (SBV2_B200_BERT_ATTN=simt: CUDA-core cross-check kernels). */
+ * every length (SBV2_B200_BERT_ATTN=simt: CUDA-core cross-check kernels). */
 int sbv2_bert_predict(sbv2_model* bert, const int64_t* input_ids, const int64_t* attention_mask,
                       int64_t t_tok, float* out);
 /* Extension (the reference is batch 1): ids/mask int64 [batch, s] with right padding expressed by

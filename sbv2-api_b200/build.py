@@ -44,11 +44,11 @@ def _digest(path: str) -> str:
 
 
 # Debug hooks (sbv2_debug_conv_compare / _conv_trace / _pair_compare / _attn_trace, the MMA micro-benchmarks, the
-# attention / spline / duration / decoder-layer hooks of debug_kernels.cu) are compiled only with -DSBV2_DEBUG_HOOKS and
+# attention / spline / duration / decoder-layer / DeBERTa hooks of debug_kernels.cu) are compiled only with -DSBV2_DEBUG_HOOKS and
 # linked only into libsbv2_b200_debug.so, which the kernel unit tests and tools/ load.
 # The product library libsbv2_b200.so carries the C ABI of include/sbv2_b200.h and nothing else.
 DEBUG_ONLY = {"umma_microbench.cu", "debug_kernels.cu"}     # whole file is a debug facility
-DEBUG_VARIANT = {"umma_decoder.cu", "flow_attention_tc.cu"}  # contain #ifdef SBV2_DEBUG_HOOKS sections
+DEBUG_VARIANT = {"umma_decoder.cu", "flow_attention_tc.cu", "bert_attention_tc.cu"}  # contain #ifdef SBV2_DEBUG_HOOKS sections
 DEBUG_LIB = os.path.join(OUT_DIR, "libsbv2_b200_debug.so")
 
 

@@ -1,5 +1,5 @@
-// DeBERTa-v2 disentangled attention on tcgen05 tensor cores for sequences of at most 128 tokens (one query tile and one
-// key tile per (utterance, head); longer sequences use deberta_attention_kernel in bert_kernels.cu).
+// DeBERTa-v2 disentangled attention on tcgen05 tensor cores: one query tile and one key tile per (utterance, head) for
+// sequences of at most 128 tokens, 128 x 128 tile pairs with an online softmax beyond (the multi-tile kernels below).
 //
 //   score[i][j] = (Q_i.K_j + Q_i.posK[b(i-j)] + K_j.posQ[b(i-j)]) / sqrt(3 D),   out = softmax(score) V
 //
@@ -14,6 +14,8 @@
 // oracle: oracle/deberta.py (HF DebertaV2Model, DisentangledSelfAttention).
 #include <cuda_fp16.h>
 #include <math_constants.h>
+
+#include <cassert>
 
 #include "kernels.h"
 
@@ -81,6 +83,9 @@ __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t* v) {
         "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
       : "r"(taddr)
       : "memory");
+}
+__device__ __forceinline__ void tc_ld1(uint32_t taddr, uint32_t& v) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(v) : "r"(taddr) : "memory");
 }
 __device__ __forceinline__ void tc_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ uint32_t elect_one_sync() {
@@ -318,15 +323,39 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_kernel(__half* ou
 }
 
 
-// Sequences of 129..512 tokens: one CTA per (head, utterance, 128-query tile), key tiles visited in order with an online
+// Multi-tile kernels.  A (query tile, key tile) pair's 256-row window covers rel in [(qt-kt)*T - (T-1), (qt-kt)*T + T].  The
+// bucket table saturates at +-max_rel (bert_bucket_table), so when that whole range lies at or beyond one of the bounds
+// every window row is the same position row: C2P is one value per query row (Q_i.posK[pr]) and P2C one value per key
+// (K_j.posQ[pr]).  Such a FAR pair gathers WF rows instead of W, issues both bias products with N = WF, reads column 0 of
+// each, and skips the skewed copies; the scores are then formed with the roundings and order of the generic path, so the
+// two paths agree bit for bit.  The class depends only on (qt, kt) and max_rel, the same for the control warp and the
+// softmax threads, and every barrier is arrived on and waited for once per key tile on either path.
+constexpr int WF = 16;
+__device__ __forceinline__ bool far_pair(int qt, int kt, int max_rel) {
+  const int d = (qt - kt) * T;
+  return d - (T - 1) >= max_rel || d + T <= -max_rel;
+}
+// position row of window row w of pair (qt, kt)
+__device__ __forceinline__ int window_row(const int* bucket_idx, int max_rel, int n_pos, int qt, int kt, int w, bool far) {
+  int rel = (qt - kt) * T + w - (T - 1);
+  rel = rel < -max_rel ? -max_rel : (rel > max_rel ? max_rel : rel);
+  const int pr = bucket_idx[rel + max_rel];
+#ifdef SBV2_DEBUG_HOOKS
+  assert(pr >= 0 && pr < n_pos);
+  if (far) assert(pr == bucket_idx[(qt > kt ? max_rel : -max_rel) + max_rel]);
+#endif
+  return pr;
+}
+
+// Sequences of more than 128 tokens: one CTA per (head, utterance, 128-query tile), key tiles visited in order with an online
 // softmax (running maximum / sum per row, O kept in registers and rescaled per key tile).  A (query tile, key tile) pair
 // sees 255 consecutive relative positions rel = i - j; beyond |rel| = span / 2 HF's log buckets map several of them to
 // one position row, so the two 256-row position windows are GATHERED through bucket_idx (row w = position of
 // rel = (qt - kt) * 128 + w - 127) instead of bulk-copied.  With the windows in rel order, the products, the skewed
-// copies and the softmax are those of the single-tile kernel.
+// copies and the softmax are those of the single-tile kernel.  Far pairs: see far_pair; the P2C column goes to row 0 of Ds.
 __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__half* out, const __half* qkv, const __half* pos_k_p,
                                                                             const __half* pos_q_p, int n_pos, const int* bucket_idx,
-                                                                            int max_rel, int heads, PlanarSegs s) {
+                                                                            int max_rel, int heads, bool far_pairs, PlanarSegs s) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
   const int h = blockIdx.x, b = blockIdx.y, qt = blockIdx.z;
@@ -375,9 +404,10 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
     const uint64_t dpk = make_desc(sPK, W * 16, 128), dpq = make_desc(sPQ, W * 16, 128);
     const uint64_t dp = make_desc(sP, T * 16, 128);
     const uint64_t dv = make_desc(sV, 128, T * 16);
-    constexpr uint32_t ID_S = idesc_f16(T, 0), ID_B = idesc_f16(W, 0), ID_O = idesc_f16(D, 1);
+    constexpr uint32_t ID_S = idesc_f16(T, 0), ID_B = idesc_f16(W, 0), ID_BF = idesc_f16(WF, 0), ID_O = idesc_f16(D, 1);
     for (int kt = 0; kt < nk; ++kt) {
       const uint32_t par = kt & 1;
+      const uint32_t id_b = far_pairs && far_pair(qt, kt, max_rel) ? ID_BF : ID_B;
       // every MMA of the previous key tile has completed (bar_o below): its K / V tiles can be overwritten
       if (lane == 0) mbar_expect_tx(bar_kv, 2 * QKV_BYTES);
       __syncwarp();
@@ -395,7 +425,7 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
 #pragma unroll
         for (int k = 0; k < D / 16; ++k) tc_mma_f16(tmem + TM_S, dq + (uint64_t)(k * 2 * T), dk + (uint64_t)(k * 2 * T), ID_S, k > 0 ? 1u : 0u);
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) tc_mma_f16(tmem + TM_B, dq + (uint64_t)(k * 2 * T), dpk + (uint64_t)(k * 2 * W), ID_B, k > 0 ? 1u : 0u);
+        for (int k = 0; k < D / 16; ++k) tc_mma_f16(tmem + TM_B, dq + (uint64_t)(k * 2 * T), dpk + (uint64_t)(k * 2 * W), id_b, k > 0 ? 1u : 0u);
         tc_commit(bar_s1);
       }
       __syncwarp();
@@ -403,7 +433,7 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
       tc_fence_after();
       if (elect_one_sync()) {
 #pragma unroll
-        for (int k = 0; k < D / 16; ++k) tc_mma_f16(tmem + TM_B, dk + (uint64_t)(k * 2 * T), dpq + (uint64_t)(k * 2 * W), ID_B, k > 0 ? 1u : 0u);
+        for (int k = 0; k < D / 16; ++k) tc_mma_f16(tmem + TM_B, dk + (uint64_t)(k * 2 * T), dpq + (uint64_t)(k * 2 * W), id_b, k > 0 ? 1u : 0u);
         tc_commit(bar_s2);
       }
       __syncwarp();
@@ -432,12 +462,11 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
     for (int kt = 0; kt < nk; ++kt) {
       const uint32_t par = kt & 1;
       const int klen = len - kt * T;  // keys of this tile below klen are real
+      const bool fr = far_pairs && far_pair(qt, kt, max_rel);
       // position windows of this tile pair (the previous pair's MMAs have completed: bar_o was waited for)
 #pragma unroll 1
-      for (int w = row; w < W; w += T) {
-        int rel = (qt - kt) * T + w - (T - 1);
-        rel = rel < -max_rel ? -max_rel : (rel > max_rel ? max_rel : rel);
-        const int pr = bucket_idx[rel + max_rel];
+      for (int w = row; w < (fr ? WF : W); w += T) {
+        const int pr = window_row(bucket_idx, max_rel, n_pos, qt, kt, w, fr);
 #pragma unroll
         for (int pl = 0; pl < DPL; ++pl) {
           const size_t src = ((size_t)(h * DPL + pl) * n_pos + pr) * 8;
@@ -455,33 +484,49 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
       }
       mbar_wait(bar_s1, par);
       tc_fence_after();
-#pragma unroll 1
-      for (int q = 0; q < W / 32; ++q) {
-        uint32_t v[32];
-        tc_ld32(lane_addr + TM_B + q * 32, v);
+      float c_far = 0.f;  // far pair: c2p of this query row, rounded to fp16 as Cs holds it
+      if (fr) {
+        uint32_t v;
+        tc_ld1(lane_addr + TM_B, v);
         tc_wait_ld();
+        c_far = __half2float(__float2half_rn(__uint_as_float(v)));
+      } else {
+#pragma unroll 1
+        for (int q = 0; q < W / 32; ++q) {
+          uint32_t v[32];
+          tc_ld32(lane_addr + TM_B + q * 32, v);
+          tc_wait_ld();
 #pragma unroll
-        for (int e = 0; e < 32; ++e) {
-          const int jj = q * 32 + e - row;
-          if (jj >= 0 && jj < T) Cs[row * PCS + jj] = __float2half_rn(__uint_as_float(v[e]));
+          for (int e = 0; e < 32; ++e) {
+            const int jj = q * 32 + e - row;
+            if (jj >= 0 && jj < T) Cs[row * PCS + jj] = __float2half_rn(__uint_as_float(v[e]));
+          }
         }
       }
       tc_fence_before();
       mbar_arrive(bar_c);
       mbar_wait(bar_s2, par);
       tc_fence_after();
-#pragma unroll 1
-      for (int q = 0; q < W / 32; ++q) {
-        uint32_t v[32];
-        tc_ld32(lane_addr + TM_B + q * 32, v);
+      if (fr) {
+        uint32_t v;
+        tc_ld1(lane_addr + TM_B, v);
         tc_wait_ld();
+        Ds[row] = __float2half_rn(__uint_as_float(v));  // p2c of key `row`, the same for every query
+      } else {
+#pragma unroll 1
+        for (int q = 0; q < W / 32; ++q) {
+          uint32_t v[32];
+          tc_ld32(lane_addr + TM_B + q * 32, v);
+          tc_wait_ld();
 #pragma unroll
-        for (int e = 0; e < 32; ++e) {
-          const int ii = q * 32 + e + row - (T - 1);
-          if (ii >= 0 && ii < T) Ds[ii * PCS + row] = __float2half_rn(__uint_as_float(v[e]));
+          for (int e = 0; e < 32; ++e) {
+            const int ii = q * 32 + e + row - (T - 1);
+            if (ii >= 0 && ii < T) Ds[ii * PCS + row] = __float2half_rn(__uint_as_float(v[e]));
+          }
         }
       }
       asm volatile("bar.sync 1, 128;" ::: "memory");
+      const __half* dr = fr ? Ds : drow;
       float mt = -CUDART_INF_F;
 #pragma unroll 1
       for (int q = 0; q < T / 32; ++q) {
@@ -491,7 +536,7 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
 #pragma unroll
         for (int e = 0; e < 32; ++e) {
           const int j = q * 32 + e;
-          const float sc = __uint_as_float(v[e]) + __half2float(crow[T - 1 - j]) + __half2float(drow[j]);
+          const float sc = __uint_as_float(v[e]) + (fr ? c_far : __half2float(crow[T - 1 - j])) + __half2float(dr[j]);
           mt = fmaxf(mt, j < klen ? sc : -CUDART_INF_F);
         }
       }
@@ -509,7 +554,7 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
 #pragma unroll
         for (int e = 0; e < 32; ++e) {
           const int j = q * 32 + e;
-          const float sc = __uint_as_float(v[e]) + __half2float(crow[T - 1 - j]) + __half2float(drow[j]);
+          const float sc = __uint_as_float(v[e]) + (fr ? c_far : __half2float(crow[T - 1 - j])) + __half2float(dr[j]);
           const float p = j < klen ? ex2_approx(fmaf(sc, c_scale, -mc)) : 0.f;
           pv[e] = p;
           lt += p;
@@ -830,14 +875,15 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_exact_kernel(__ha
 }
 
 
-// Exact numerics, 129..512 tokens: the tile-pair loop / online softmax / gathered log-bucket windows of
+// Exact numerics, more than 128 tokens: the tile-pair loop / online softmax / gathered log-bucket windows of
 // deberta_attention_tc_multi_kernel with the split operands, fp32 bias tile and split probabilities of
 // deberta_attention_tc_exact_kernel.  Per key tile the 64 KB window buffer holds the gathered posK terms, then the gathered
-// posQ terms, then the two P terms.
+// posQ terms, then the two P terms.  Far pairs (far_pair): c2p stays in a register, the p2c column goes to row 0 of Bs, and
+// the bias is fl(c2p + p2c) as the generic path's Bs holds it.
 __global__ void __launch_bounds__(160, 1)
     deberta_attention_tc_exact_multi_kernel(__half* out_s, long long out_blk, const __half* qkv_s, long long qkv_blk, const __half* pos_k_s,
                                             const __half* pos_q_s, int n_pos, const int* bucket_idx, int max_rel, int heads, float inv_sc2,
-                                            PlanarSegs s) {
+                                            bool far_pairs, PlanarSegs s) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;
   const int h = blockIdx.x, b = blockIdx.y, qt = blockIdx.z;
@@ -892,7 +938,7 @@ __global__ void __launch_bounds__(160, 1)
     const uint64_t dw0 = make_desc(sW0, W * 16, 128), dw1 = make_desc(sW1, W * 16, 128);
     const uint64_t dp0 = make_desc(sW0, T * 16, 128), dp1 = make_desc(sW1, T * 16, 128);
     const uint64_t dv0 = make_desc(sV0, 128, T * 16), dv1 = make_desc(sV1, 128, T * 16);
-    constexpr uint32_t ID_S = idesc_f16(T, 0), ID_B = idesc_f16(W, 0), ID_O = idesc_f16(D, 1);
+    constexpr uint32_t ID_S = idesc_f16(T, 0), ID_B = idesc_f16(W, 0), ID_BF = idesc_f16(WF, 0), ID_O = idesc_f16(D, 1);
     auto cross = [&](uint32_t tm, uint64_t a0, uint64_t a1, uint64_t b0, uint64_t b1, uint32_t astep, uint32_t bstep, uint32_t id, int nk16) {
       for (int k = 0; k < nk16; ++k) tc_mma_f16(tm, a0 + (uint64_t)(k * astep), b0 + (uint64_t)(k * bstep), id, k > 0 ? 1u : 0u);
       for (int k = 0; k < nk16; ++k) tc_mma_f16(tm, a0 + (uint64_t)(k * astep), b1 + (uint64_t)(k * bstep), id, 1u);
@@ -900,6 +946,7 @@ __global__ void __launch_bounds__(160, 1)
     };
     for (int kt = 0; kt < nk; ++kt) {
       const uint32_t par = kt & 1;
+      const uint32_t id_b = far_pairs && far_pair(qt, kt, max_rel) ? ID_BF : ID_B;
       if (lane == 0) mbar_expect_tx(bar_kv, 4 * QKV_BYTES);
       __syncwarp();
       {
@@ -915,14 +962,14 @@ __global__ void __launch_bounds__(160, 1)
       tc_fence_after();
       if (elect_one_sync()) {
         cross(tmem + TM_S, dq0, dq1, dk0, dk1, 2 * T, 2 * T, ID_S, D / 16);
-        cross(tmem + TM_B, dq0, dq1, dw0, dw1, 2 * T, 2 * W, ID_B, D / 16);
+        cross(tmem + TM_B, dq0, dq1, dw0, dw1, 2 * T, 2 * W, id_b, D / 16);
         tc_commit(bar_s1);
       }
       __syncwarp();
       mbar_wait(bar_g2, par);  // C2P copied out of TMEM, posQ terms gathered
       tc_fence_after();
       if (elect_one_sync()) {
-        cross(tmem + TM_B, dk0, dk1, dw0, dw1, 2 * T, 2 * W, ID_B, D / 16);
+        cross(tmem + TM_B, dk0, dk1, dw0, dw1, 2 * T, 2 * W, id_b, D / 16);
         tc_commit(bar_s2);
       }
       __syncwarp();
@@ -952,12 +999,11 @@ __global__ void __launch_bounds__(160, 1)
     for (int kt = 0; kt < nk; ++kt) {
       const uint32_t par = kt & 1;
       const int klen = len - kt * T;
+      const bool fr = far_pairs && far_pair(qt, kt, max_rel);
       auto gather = [&](const __half* tab) {
 #pragma unroll 1
-        for (int w = row; w < W; w += T) {
-          int rel = (qt - kt) * T + w - (T - 1);
-          rel = rel < -max_rel ? -max_rel : (rel > max_rel ? max_rel : rel);
-          const int pr = bucket_idx[rel + max_rel];
+        for (int w = row; w < (fr ? WF : W); w += T) {
+          const int pr = window_row(bucket_idx, max_rel, n_pos, qt, kt, w, fr);
 #pragma unroll
           for (int i = 0; i < 2 * DPL; ++i) {
             const int term = i >> 3, pl = i & 7;
@@ -980,15 +1026,23 @@ __global__ void __launch_bounds__(160, 1)
       }
       mbar_wait(bar_s1, par);
       tc_fence_after();
-#pragma unroll 1
-      for (int q = 0; q < W / 32; ++q) {
-        uint32_t v[32];
-        tc_ld32(lane_addr + TM_B + q * 32, v);
+      float c_far = 0.f;  // far pair: c2p of this query row
+      if (fr) {
+        uint32_t v;
+        tc_ld1(lane_addr + TM_B, v);
         tc_wait_ld();
+        c_far = __uint_as_float(v);
+      } else {
+#pragma unroll 1
+        for (int q = 0; q < W / 32; ++q) {
+          uint32_t v[32];
+          tc_ld32(lane_addr + TM_B + q * 32, v);
+          tc_wait_ld();
 #pragma unroll
-        for (int e = 0; e < 32; ++e) {
-          const int j = row + (T - 1) - (q * 32 + e);
-          if (j >= 0 && j < T) Bs[row * BCS + j] = __uint_as_float(v[e]);
+          for (int e = 0; e < 32; ++e) {
+            const int j = row + (T - 1) - (q * 32 + e);
+            if (j >= 0 && j < T) Bs[row * BCS + j] = __uint_as_float(v[e]);
+          }
         }
       }
       tc_fence_before();
@@ -997,18 +1051,26 @@ __global__ void __launch_bounds__(160, 1)
       asm volatile("bar.sync 1, 128;" ::: "memory");  // every c2p entry is written before any p2c entry is added
       mbar_wait(bar_s2, par);
       tc_fence_after();
-#pragma unroll 1
-      for (int q = 0; q < W / 32; ++q) {
-        uint32_t v[32];
-        tc_ld32(lane_addr + TM_B + q * 32, v);
+      if (fr) {
+        uint32_t v;
+        tc_ld1(lane_addr + TM_B, v);
         tc_wait_ld();
+        Bs[row] = __uint_as_float(v);  // p2c of key `row`, the same for every query
+      } else {
+#pragma unroll 1
+        for (int q = 0; q < W / 32; ++q) {
+          uint32_t v[32];
+          tc_ld32(lane_addr + TM_B + q * 32, v);
+          tc_wait_ld();
 #pragma unroll
-        for (int e = 0; e < 32; ++e) {
-          const int ii = q * 32 + e + row - (T - 1);
-          if (ii >= 0 && ii < T) Bs[ii * BCS + row] += __uint_as_float(v[e]);
+          for (int e = 0; e < 32; ++e) {
+            const int ii = q * 32 + e + row - (T - 1);
+            if (ii >= 0 && ii < T) Bs[ii * BCS + row] += __uint_as_float(v[e]);
+          }
         }
       }
       asm volatile("bar.sync 1, 128;" ::: "memory");
+      const float* br = fr ? Bs : brow;
       float mt = -CUDART_INF_F;
 #pragma unroll 1
       for (int q = 0; q < T / 32; ++q) {
@@ -1017,8 +1079,8 @@ __global__ void __launch_bounds__(160, 1)
         tc_wait_ld();
 #pragma unroll
         for (int e4 = 0; e4 < 8; ++e4) {
-          const float4 bb = *reinterpret_cast<const float4*>(brow + q * 32 + 4 * e4);
-          const float bv[4] = {bb.x, bb.y, bb.z, bb.w};
+          const float4 bb = *reinterpret_cast<const float4*>(br + q * 32 + 4 * e4);
+          const float bv[4] = {fr ? c_far + bb.x : bb.x, fr ? c_far + bb.y : bb.y, fr ? c_far + bb.z : bb.z, fr ? c_far + bb.w : bb.w};
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int j = q * 32 + 4 * e4 + u;
@@ -1040,8 +1102,8 @@ __global__ void __launch_bounds__(160, 1)
         float pv[32];
 #pragma unroll
         for (int e4 = 0; e4 < 8; ++e4) {
-          const float4 bb = *reinterpret_cast<const float4*>(brow + q * 32 + 4 * e4);
-          const float bv[4] = {bb.x, bb.y, bb.z, bb.w};
+          const float4 bb = *reinterpret_cast<const float4*>(br + q * 32 + 4 * e4);
+          const float bv[4] = {fr ? c_far + bb.x : bb.x, fr ? c_far + bb.y : bb.y, fr ? c_far + bb.z : bb.z, fr ? c_far + bb.w : bb.w};
 #pragma unroll
           for (int u = 0; u < 4; ++u) {
             const int j = q * 32 + 4 * e4 + u;
@@ -1118,7 +1180,7 @@ __global__ void __launch_bounds__(160, 1)
 
 bool deberta_attention_tc_supported(int head_dim, int span, int max_len) { return head_dim == D && span >= 254 && max_len <= T; }
 
-bool deberta_attention_tc_multi_supported(int head_dim, int max_rel, int max_len) { return head_dim == D && max_len - 1 <= max_rel; }
+bool deberta_attention_tc_multi_supported(int head_dim) { return head_dim == D; }
 
 void launch_deberta_attention_tc(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const __half* pos_k_p, const __half* pos_q_p,
                                  int n_pos, int span, int heads, const PlanarSegs& s) {
@@ -1136,15 +1198,15 @@ void launch_deberta_attention_tc(const LaunchCtx& ctx, __half* ctx_out, const __
 }
 
 void launch_deberta_attention_tc_multi(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const __half* pos_k_p, const __half* pos_q_p,
-                                       int n_pos, const int* bucket_idx, int max_rel, int heads, const PlanarSegs& s) {
+                                       int n_pos, const int* bucket_idx, int max_rel, int heads, bool far_pairs, const PlanarSegs& s) {
   if (s.n <= 0 || s.max_len <= 0) return;
-  if (!deberta_attention_tc_multi_supported(D, max_rel, s.max_len))
+  if (!deberta_attention_tc_multi_supported(D) || s.max_len > kMaxBertTokens)
     fail(SBV2_ERR_INTERNAL, "tensor-core DeBERTa attention (multi-tile): unsupported shape");
   const size_t smem = 3 * QKV_BYTES + 2 * POS_BYTES + P_BYTES + 2 * SKEW_BYTES + 128;
   static PerDeviceOnce attr_once;
   attr_once.run([&] { CUDA_CHECK(cudaFuncSetAttribute(deberta_attention_tc_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); });
   dim3 grid(heads, s.n, (s.max_len + T - 1) / T);
-  deberta_attention_tc_multi_kernel<<<grid, 160, smem, ctx.stream>>>(ctx_out, qkv, pos_k_p, pos_q_p, n_pos, bucket_idx, max_rel, heads, s);
+  deberta_attention_tc_multi_kernel<<<grid, 160, smem, ctx.stream>>>(ctx_out, qkv, pos_k_p, pos_q_p, n_pos, bucket_idx, max_rel, heads, far_pairs, s);
   CUDA_CHECK(cudaGetLastError());
   ctx.count();
 }
@@ -1170,9 +1232,9 @@ void launch_deberta_attention_tc_exact(const LaunchCtx& ctx, __half* ctx_s, long
 
 void launch_deberta_attention_tc_exact_multi(const LaunchCtx& ctx, __half* ctx_s, long long ctx_blk, const __half* qkv_s, long long qkv_blk,
                                              const __half* pos_k_s, const __half* pos_q_s, int n_pos, const int* bucket_idx, int max_rel,
-                                             int heads, float sc, const PlanarSegs& s) {
+                                             int heads, float sc, bool far_pairs, const PlanarSegs& s) {
   if (s.n <= 0 || s.max_len <= 0) return;
-  if (!deberta_attention_tc_multi_supported(D, max_rel, s.max_len))
+  if (!deberta_attention_tc_multi_supported(D) || s.max_len > kMaxBertTokens)
     fail(SBV2_ERR_INTERNAL, "tensor-core DeBERTa attention (exact, multi-tile): unsupported shape");
   static PerDeviceOnce attr_once;
   attr_once.run([&] {
@@ -1180,7 +1242,7 @@ void launch_deberta_attention_tc_exact_multi(const LaunchCtx& ctx, __half* ctx_s
   });
   dim3 grid(heads, s.n, (s.max_len + T - 1) / T);
   deberta_attention_tc_exact_multi_kernel<<<grid, 160, EX_SMEM, ctx.stream>>>(ctx_s, ctx_blk, qkv_s, qkv_blk, pos_k_s, pos_q_s, n_pos, bucket_idx,
-                                                                               max_rel, heads, 1.0f / (sc * sc), s);
+                                                                               max_rel, heads, 1.0f / (sc * sc), far_pairs, s);
   CUDA_CHECK(cudaGetLastError());
   ctx.count();
 }

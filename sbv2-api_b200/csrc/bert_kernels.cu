@@ -371,8 +371,9 @@ __global__ void __launch_bounds__(256) deberta_attention_kernel(void* out_v, con
         from_f32(Vs[r * BD + pl * 8 + e], vf[e]);
       }
     }
-    // position range of this tile pair: delta = i - j in [q0-k0-63, q0-k0+63]
-    const int dmin = max(q0 - k0 - (BK - 1), -max_rel), dmax = min(q0 - k0 + (BQ - 1), max_rel);
+    // position range of this tile pair: delta = i - j in [q0-k0-63, q0-k0+63], both ends clamped to the table's +-max_rel
+    // (beyond max_rel + 63 tokens apart a whole range lies outside it)
+    const int dmin = min(max(q0 - k0 - (BK - 1), -max_rel), max_rel), dmax = min(max(q0 - k0 + (BQ - 1), -max_rel), max_rel);
     const int pmin = bucket_idx[dmin + max_rel], pmax = bucket_idx[dmax + max_rel];
     const int np = pmax - pmin + 1;  // <= 127
     for (int phase = 0; phase < 2; ++phase) {

@@ -9,8 +9,9 @@
 //                    synthesizer, and durations must match the reference bit for bit: single-term fp16 operands perturb
 //                    the features by 1.4e-3 (relative) and flip ~1 duration in 1000 (tests/test_gpu_fullsize.py chain test).
 //   fp16             single-term fp16 operands and planar fp16 activations (3x fewer tensor FLOPs), tensor-core
-//                    disentangled attention for sequences <= 128 tokens: the throughput mode, feature error ~1e-3.
+//                    disentangled attention: the throughput mode, feature error ~1e-3.
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <sstream>
 
@@ -34,7 +35,7 @@ struct BertLayer {
 };
 
 struct BertModel : sbv2_model {
-  int hidden = 0, heads = 0, inter = 0, vocab = 0, n_layers_total = 0, n_run = 0, span = 0, max_rel = 511;
+  int hidden = 0, heads = 0, inter = 0, vocab = 0, n_layers_total = 0, n_run = 0, span = 0, max_rel = 0;
   float eps = 1e-7f;
   float* word_emb = nullptr;
   float *emb_g = nullptr, *emb_b = nullptr;
@@ -42,7 +43,7 @@ struct BertModel : sbv2_model {
   bool has_conv = false;
   ConvLayer conv, conv_s;
   float *conv_g = nullptr, *conv_b = nullptr;
-  int* bucket_idx = nullptr;  // device [2*max_rel+1]
+  int* bucket_idx = nullptr;  // device [2*max_rel+1] (bert_bucket_table)
   DBuf ids, h, embp, hp, qkvp, ctxp, f1p, y32, meta, outd;
   uint64_t qkvp_cleared_gen = 0;  // DBuf::gen of the qkv buffer that was zero-filled last (its tail rows must be finite)
   bool use_tc_attn = true;       // SBV2_B200_BERT_ATTN=simt (read at model creation) keeps the CUDA-core attention
@@ -78,6 +79,24 @@ int log_bucket(int rel, int bucket_size, int max_position) {
 }
 
 }  // namespace
+
+std::vector<int> bert_bucket_table(int span, int* max_rel) {
+  if (span < 2) fail(SBV2_ERR_UNSUPPORTED, "DeBERTa position_buckets must be at least 2");
+  const int hi = 2 * span - 1;
+  auto idx = [&](int d) { return std::min(std::max(log_bucket(d, span, 2 * span) + span, 0), hi); };  // max_position = 2*span
+  // the log buckets grow without bound, so the clamp saturates both ends; R = the first distance where both have
+  // (HF span 256: idx(-512) = 0 but idx(-511) = 1, idx(d) = 511 from d = 506 on, so R = 512)
+  int R = 1;
+  while (idx(R) != hi || idx(-R) != 0)
+    if (++R > 4 * kMaxBertTokens) fail(SBV2_ERR_UNSUPPORTED, "DeBERTa position buckets do not saturate");
+  // every distance a sequence within the cap can form must read the same row as R once clamped to it
+  for (int d = R; d < kMaxBertTokens; ++d)
+    if (idx(d) != hi || idx(-d) != 0) fail(SBV2_ERR_INTERNAL, "DeBERTa bucket table is not saturated beyond its bound");
+  std::vector<int> tab(size_t(2) * R + 1);
+  for (int d = -R; d <= R; ++d) tab[size_t(d + R)] = idx(d);
+  *max_rel = R;
+  return tab;
+}
 
 sbv2_model* create_bert_model(const OnnxModel& m, int device) {
   std::unique_ptr<BertModel> M(new BertModel());
@@ -267,13 +286,8 @@ sbv2_model* create_bert_model(const OnnxModel& m, int device) {
     M->conv_b = vec("encoder.conv.LayerNorm.bias", H);
     M->has_conv = true;
   }
-  // bucket index table: clamp(bucket(delta) + span, 0, 2*span-1), delta in [-max_rel, max_rel]
   {
-    std::vector<int> tab(size_t(2) * M->max_rel + 1);
-    for (int d = -M->max_rel; d <= M->max_rel; ++d) {
-      int bkt = log_bucket(d, M->span, 2 * M->span) + M->span;  // position_buckets = span, max_position = 2*span
-      tab[size_t(d + M->max_rel)] = std::min(std::max(bkt, 0), 2 * M->span - 1);
-    }
+    const std::vector<int> tab = bert_bucket_table(M->span, &M->max_rel);
     M->bucket_idx = static_cast<int*>(M->upload_bytes(tab.data(), tab.size() * 4));
   }
   for (DBuf* b : {&M->ids, &M->h, &M->embp, &M->hp, &M->qkvp, &M->ctxp, &M->f1p, &M->y32, &M->meta, &M->outd, &M->x_emb, &M->x_qkv, &M->x_qkvs, &M->x_ctx,
@@ -297,7 +311,7 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
   auto* Mp = static_cast<BertModel*>(mm);
   BertModel& M = *Mp;
   SBV2_REQUIRE(batch > 0 && S > 0, "empty input");
-  SBV2_REQUIRE(S <= M.max_rel + 1, "sequence longer than 512 tokens is not supported");
+  SBV2_REQUIRE(S <= kMaxBertTokens, "sequence longer than 32768 tokens");
   M.bind_device();
   const int H = M.hidden;
   // right-padded masks only: 1..1 0..0
@@ -310,6 +324,7 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
     for (int64_t t = l; t < S; ++t)
       if (mask[b * S + t] != 0) fail(SBV2_ERR_UNSUPPORTED, "attention_mask must be a prefix of ones (right padding)");
     len[b] = l;
+    SBV2_REQUIRE(n + l <= INT_MAX, "too many tokens in one call");  // packed rows are indexed in int32
     start[b] = int(n);
     n += l;
     max_len = std::max(max_len, l);
@@ -366,8 +381,7 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
     // attention on the tensor cores with split operands (one tile up to 128 tokens, tile pairs beyond;
     // SBV2_B200_BERT_ATTN=simt: fp32 CUDA-core kernel); q|k|v then leave their GEMM as split planes instead of fp32 rows
     const bool tc_single = deberta_attention_tc_supported(64, M.span, max_len);
-    const bool tc_exact = M.use_tc_attn && M.hidden / M.heads == 64 && sc == kSplitScale &&
-                          (tc_single || deberta_attention_tc_multi_supported(64, M.max_rel, max_len));
+    const bool tc_exact = M.use_tc_attn && M.hidden / M.heads == 64 && sc == kSplitScale && (tc_single || deberta_attention_tc_multi_supported(64));
     __half* sp_qkv = nullptr;
     const long long qkv_blk = (long long)(3 * H / 8) * ps.plane_stride, ctx_blk = (long long)(H / 8) * ps.plane_stride;
     if (tc_exact) {
@@ -405,7 +419,7 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
           launch_deberta_attention_tc_exact(ctx, sp_b, ctx_blk, sp_qkv, qkv_blk, B.pos_k_s, B.pos_q_s, 2 * M.span, M.span, M.heads, sc, ps);
         else
           launch_deberta_attention_tc_exact_multi(ctx, sp_b, ctx_blk, sp_qkv, qkv_blk, B.pos_k_s, B.pos_q_s, 2 * M.span, M.bucket_idx, M.max_rel,
-                                                  M.heads, sc, ps);
+                                                  M.heads, sc, true, ps);
       } else {
         gemm(small ? B.qkv_s : B.qkv, l == 0 ? sp_e : sp_a, qkv, 3 * H, nullptr, ACT_NONE);
         launch_deberta_attention_f32(ctx, nullptr, sp_b, sc, qkv, B.pos_k, B.pos_q, 2 * M.span, M.bucket_idx, M.max_rel, M.heads, 64, ps);
@@ -458,8 +472,8 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
   };
   // sequences of at most 128 tokens: disentangled attention on the tensor cores (SBV2_B200_BERT_ATTN=simt: CUDA cores)
   const bool tc_attn = M.use_tc_attn && M.hidden / M.heads == 64 && deberta_attention_tc_supported(64, M.span, max_len);
-  // 129..512 tokens: the multi-tile kernel (log-bucket position windows gathered per tile pair)
-  const bool tc_multi = !tc_attn && M.use_tc_attn && M.hidden / M.heads == 64 && deberta_attention_tc_multi_supported(64, M.max_rel, max_len);
+  // longer sequences: the multi-tile kernel (log-bucket position windows gathered per tile pair)
+  const bool tc_multi = !tc_attn && M.use_tc_attn && M.hidden / M.heads == 64 && deberta_attention_tc_multi_supported(64);
   if ((tc_attn || tc_multi) && M.qkvp.gen != M.qkvp_cleared_gen) {
     // rows past an utterance's end are read by the tensor-core attention: they must hold finite values
     CUDA_CHECK(cudaMemsetAsync(M.qkvp.p, 0, M.qkvp.cap, M.stream));
@@ -471,7 +485,7 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
     const __half* in = l == 0 ? embp : hp;
     umma(small ? B.qkv_s : B.qkv, in, qkvp, nullptr, ACT_NONE);
     if (tc_attn) launch_deberta_attention_tc(ctx, ctxp, qkvp, B.pos_k_p, B.pos_q_p, 2 * M.span, M.span, M.heads, ps);
-    else if (tc_multi) launch_deberta_attention_tc_multi(ctx, ctxp, qkvp, B.pos_k_p, B.pos_q_p, 2 * M.span, M.bucket_idx, M.max_rel, M.heads, ps);
+    else if (tc_multi) launch_deberta_attention_tc_multi(ctx, ctxp, qkvp, B.pos_k_p, B.pos_q_p, 2 * M.span, M.bucket_idx, M.max_rel, M.heads, true, ps);
     else launch_deberta_attention(ctx, ctxp, qkvp, B.pos_k, B.pos_q, 2 * M.span, M.bucket_idx, M.max_rel, M.heads, 64, ps);
     umma(small ? B.o_s : B.o, ctxp, nullptr, y32, ACT_NONE);
     launch_ln_planar_wide(ctx, h, hp, nullptr, y32, B.ln1_g, B.ln1_b, M.eps, H, ps);

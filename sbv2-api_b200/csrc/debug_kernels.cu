@@ -9,6 +9,7 @@
 #include <algorithm>
 #include <climits>
 #include <cstring>
+#include <functional>
 
 #include "model.h"
 #include "umma_conv.h"
@@ -386,5 +387,128 @@ extern "C" int sbv2_debug_dec_post(const float* x, const int* lens, const long l
     float* d_wave = upload(owner, wave, size_t(wave_len));
     launch_dec_post_planar(owner.ctx(), d_wave, d_x, G, bg.d_wstart, n, upload(owner, wh.data(), wh.size()), wh, C, k, force_generic != 0);
     download(owner, wave, d_wave, size_t(wave_len));
+  });
+}
+
+// ---- DeBERTa ----------------------------------------------------------------------------------------------------
+// The relative-position bucket table the model builds at load (bert_bucket_table), on the host: *max_rel = its saturation
+// bound R; out (null: R only) receives the 2R + 1 entries for delta = -R..R.  Needs no device.
+extern "C" int sbv2_debug_bert_bucket_table(int span, int* max_rel, int* out) {
+  return guarded([&] {
+    SBV2_REQUIRE(max_rel != nullptr, "bad arguments");
+    const std::vector<int> tab = bert_bucket_table(span, max_rel);
+    if (out) memcpy(out, tab.data(), tab.size() * sizeof(int));
+  });
+}
+
+// One DeBERTa disentangled attention launch (head dim 64) on a ragged batch, with the bucket table of `span`.
+//   qkv   fp16 row-major [terms][sum(lens)][3 * heads * 64] (q | k | v, channel h * 64 + d)
+//   pos_k, pos_q  fp16 row-major [terms][2 * span][heads * 64]: the position projections
+//   mode  0: single-tile tensor-core kernel (<= 128 tokens), 1: multi-tile tensor-core kernel, 2: its exact variant, whose
+//         operands are the two fp16 terms (terms = 2) of values scaled by sc, 3: CUDA-core kernel; terms = 1 except in mode 2
+//   far_pairs  modes 1 and 2: far tile pairs take the reduced path (0: the generic path for every pair)
+//   out   fp16 row-major [terms][sum(lens)][heads * 64]: the context (mode 2: the two terms of context * sc)
+//   reps > 0: the launch is then repeated `reps` times between two CUDA events and *ms receives the mean time per launch
+// The planar rows of no utterance hold zeros, as the model keeps them.
+extern "C" int sbv2_debug_deberta_attention(const uint16_t* qkv, const uint16_t* pos_k, const uint16_t* pos_q, const int* lens, int n,
+                                            int heads, int span, int mode, int far_pairs, float sc, int reps, float* ms, uint16_t* out) {
+  return guarded([&] {
+    SBV2_REQUIRE(qkv && pos_k && pos_q && lens && out && n > 0 && heads > 0 && mode >= 0 && mode <= 3, "bad arguments");
+    SBV2_REQUIRE(mode != 2 || sc > 0.f, "the exact kernel needs the split scale");
+    SBV2_REQUIRE(reps <= 0 || ms != nullptr, "timing needs *ms");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    std::vector<int> ystart(lens, lens + n), ylen(lens, lens + n), muls{1};
+    long long rows = 0;
+    for (int b = 0; b < n; ++b) {
+      SBV2_REQUIRE(lens[b] >= 1 && lens[b] <= kMaxBertTokens, "utterance lengths must be in [1, 32768]");
+      ystart[size_t(b)] = int(rows);
+      rows += lens[b];
+      SBV2_REQUIRE(rows < INT_MAX, "too many rows");
+    }
+    int max_rel = 0;
+    const std::vector<int> tab = bert_bucket_table(span, &max_rel);
+    DBuf meta;
+    PinnedBuf pin;
+    meta.stream = owner.stream;
+    BatchGeom bg = build_geoms(&owner, meta, pin, ystart, ylen, muls);
+    const Geom& G = bg.g[0];
+    const int H = heads * 64, C3 = 3 * H, terms = mode == 2 ? 2 : 1, n_pos = 2 * span;
+    const size_t plane = size_t(G.rows_tot) * 8, qkv_blk = size_t(C3 / 8) * plane, ctx_blk = size_t(H / 8) * plane;
+    std::vector<uint16_t> hq(terms * qkv_blk, 0);
+    for (int term = 0; term < terms; ++term)
+      for (int b = 0; b < n; ++b)
+        for (int t = 0; t < lens[b]; ++t) {
+          const size_t pr = size_t(G.pstart[size_t(b)]) + t;
+          const uint16_t* src = qkv + (size_t(term) * rows + ystart[size_t(b)] + t) * C3;
+          for (int c = 0; c < C3; ++c) hq[term * qkv_blk + size_t(c / 8) * plane + pr * 8 + c % 8] = src[c];
+        }
+    std::vector<uint16_t> ho(3 * ctx_blk, 0);
+    const __half* d_qkv = reinterpret_cast<const __half*>(upload(owner, hq.data(), hq.size()));
+    __half* d_out = reinterpret_cast<__half*>(upload(owner, ho.data(), ho.size()));
+    const int* d_tab = upload(owner, tab.data(), tab.size());
+    PlanarSegs ps;
+    ps.start = bg.d_ystart;
+    ps.pstart = G.d_pstart;
+    ps.len = G.d_len;
+    ps.order = bg.d_order;
+    ps.n = n;
+    ps.max_len = G.max_len;
+    ps.plane_stride = G.rows_tot * 8;
+    std::function<void()> launch;
+    if (mode == 3) {
+      // the CUDA-core kernel reads fp32 tables transposed to [heads * 64][n_pos]
+      std::vector<float> tk(size_t(H) * n_pos), tq(tk.size());
+      for (int r = 0; r < n_pos; ++r)
+        for (int c = 0; c < H; ++c) {
+          tk[size_t(c) * n_pos + r] = __half2float(__ushort_as_half(pos_k[size_t(r) * H + c]));
+          tq[size_t(c) * n_pos + r] = __half2float(__ushort_as_half(pos_q[size_t(r) * H + c]));
+        }
+      const float* d_tk = upload(owner, tk.data(), tk.size());
+      const float* d_tq = upload(owner, tq.data(), tq.size());
+      launch = [&, d_tk, d_tq] { launch_deberta_attention(ctx, d_out, d_qkv, d_tk, d_tq, n_pos, d_tab, max_rel, heads, 64, ps); };
+    } else {
+      // the tensor-core kernels read [terms][heads][8][n_pos][8]
+      auto pack = [&](const uint16_t* pos) {
+        std::vector<uint16_t> p(size_t(terms) * H * n_pos);
+        for (int term = 0; term < terms; ++term)
+          for (int r = 0; r < n_pos; ++r)
+            for (int c = 0; c < H; ++c)
+              p[size_t(term) * H * n_pos + (size_t(c / 8) * n_pos + r) * 8 + c % 8] = pos[(size_t(term) * n_pos + r) * H + c];
+        return reinterpret_cast<const __half*>(upload(owner, p.data(), p.size()));
+      };
+      const __half* d_pk = pack(pos_k);
+      const __half* d_pq = pack(pos_q);
+      launch = [&, d_pk, d_pq] {
+        if (mode == 0) launch_deberta_attention_tc(ctx, d_out, d_qkv, d_pk, d_pq, n_pos, span, heads, ps);
+        else if (mode == 1) launch_deberta_attention_tc_multi(ctx, d_out, d_qkv, d_pk, d_pq, n_pos, d_tab, max_rel, heads, far_pairs != 0, ps);
+        else
+          launch_deberta_attention_tc_exact_multi(ctx, d_out, (long long)ctx_blk, d_qkv, (long long)qkv_blk, d_pk, d_pq, n_pos, d_tab, max_rel,
+                                                  heads, sc, far_pairs != 0, ps);
+      };
+    }
+    launch();
+    if (reps > 0) {
+      cudaEvent_t e0, e1;
+      CUDA_CHECK(cudaEventCreate(&e0));
+      CUDA_CHECK(cudaEventCreate(&e1));
+      CUDA_CHECK(cudaEventRecord(e0, owner.stream));
+      for (int r = 0; r < reps; ++r) launch();
+      CUDA_CHECK(cudaEventRecord(e1, owner.stream));
+      CUDA_CHECK(cudaEventSynchronize(e1));
+      CUDA_CHECK(cudaEventElapsedTime(ms, e0, e1));
+      *ms /= float(reps);
+      CUDA_CHECK(cudaEventDestroy(e0));
+      CUDA_CHECK(cudaEventDestroy(e1));
+    }
+    download(owner, ho.data(), reinterpret_cast<const uint16_t*>(d_out), ho.size());
+    for (int term = 0; term < terms; ++term)
+      for (int b = 0; b < n; ++b)
+        for (int t = 0; t < lens[b]; ++t) {
+          const size_t pr = size_t(G.pstart[size_t(b)]) + t;
+          uint16_t* dst = out + (size_t(term) * rows + ystart[size_t(b)] + t) * H;
+          for (int c = 0; c < H; ++c) dst[c] = ho[term * ctx_blk + size_t(c / 8) * plane + pr * 8 + c % 8];
+        }
   });
 }

@@ -201,9 +201,15 @@ void launch_ln_planar_wide(const LaunchCtx& ctx, float* h, __half* hp, __half* h
                            const float* beta, float eps, int C, const PlanarSegs& s);
 // h[row, :] = table[ids[row], :]
 void launch_embed_rows(const LaunchCtx& ctx, float* h, const float* table, const int* ids, int C, int n_vocab, int64_t rows);
+// Longest sequence the DeBERTa forward accepts (tokens); longer inputs return SBV2_ERR_INVALID_ARGUMENT.
+constexpr int kMaxBertTokens = 32768;
+// Relative-position bucket table of HF make_log_bucket_position(delta, span, 2 * span): entry delta + R holds
+// clamp(bucket(delta) + span, 0, 2*span-1) for delta = -R..R, R (*max_rel) being the saturation bound: every |delta| >= R reads
+// the same row as +-R (span 256: R = 512, idx(-512) = 0, idx(-511) = 1).  So kernels clamp delta to +-R and index the table.
+// Checked for every |delta| < kMaxBertTokens.
+std::vector<int> bert_bucket_table(int span, int* max_rel);
 // DeBERTa-v2 disentangled attention (c2p + p2c, shared keys) on planar fp16 q|k|v -> planar fp16 ctx.
-// pos_k/pos_q: fp32 [2*span, heads*64] projections of the normalised relative embeddings;
-// bucket_idx: int [2*max_rel+1] = clamp(bucket(delta) + span, 0, 2*span-1) for delta = -max_rel..max_rel.
+// pos_k/pos_q: fp32 [2*span, heads*64] projections of the normalised relative embeddings; bucket_idx / max_rel: bert_bucket_table.
 void launch_deberta_attention(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const float* pos_k_t, const float* pos_q_t,
                               int n_pos, const int* bucket_idx, int max_rel, int heads, int head_dim, const PlanarSegs& s);
 // "exact" mode: the same kernel on fp32 row-major q|k|v [rows, 3*heads*64] -> fp32 row-major context [rows, heads*64]
@@ -223,13 +229,16 @@ void launch_deberta_attention_tc(const LaunchCtx& ctx, __half* ctx_out, const __
 void launch_deberta_attention_tc_exact(const LaunchCtx& ctx, __half* ctx_s, long long ctx_blk, const __half* qkv_s, long long qkv_blk,
                                        const __half* pos_k_s, const __half* pos_q_s, int n_pos, int span, int heads, float sc,
                                        const PlanarSegs& s);
+// Any length: 128-query tiles x 128-key tiles with an online softmax; position windows gathered through bucket_idx.
+// far_pairs: a tile pair whose relative positions all lie at or beyond +-max_rel (|qt - kt| >= 5 for span 256) reads one
+// position row, and takes the reduced path (16 gathered rows, N = 16 bias products, no skewed copies), bit-identical to
+// the generic path; false forces the generic path (the debug hook compares the two).
+bool deberta_attention_tc_multi_supported(int head_dim);
 void launch_deberta_attention_tc_exact_multi(const LaunchCtx& ctx, __half* ctx_s, long long ctx_blk, const __half* qkv_s, long long qkv_blk,
                                              const __half* pos_k_s, const __half* pos_q_s, int n_pos, const int* bucket_idx, int max_rel,
-                                             int heads, float sc, const PlanarSegs& s);
-// 129..512 tokens: 128-query tiles x 128-key tiles with an online softmax; position windows gathered through bucket_idx
-bool deberta_attention_tc_multi_supported(int head_dim, int max_rel, int max_len);
+                                             int heads, float sc, bool far_pairs, const PlanarSegs& s);
 void launch_deberta_attention_tc_multi(const LaunchCtx& ctx, __half* ctx_out, const __half* qkv, const __half* pos_k_p, const __half* pos_q_p,
-                                       int n_pos, const int* bucket_idx, int max_rel, int heads, const PlanarSegs& s);
+                                       int n_pos, const int* bucket_idx, int max_rel, int heads, bool far_pairs, const PlanarSegs& s);
 // out[b, t, :] = h[start[b] + t, :] for t < len[b], zeros elsewhere (out: [n, S, C] fp32)
 void launch_scatter_rows(const LaunchCtx& ctx, float* out, const float* h, int C, int S, const PlanarSegs& s);
 }  // namespace sbv2

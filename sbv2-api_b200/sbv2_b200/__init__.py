@@ -133,7 +133,7 @@ _debug_lib = None
 def debug_lib() -> C.CDLL:
     """libsbv2_b200_debug.so: the same objects plus the kernel unit-test / tracing hooks (sbv2_debug_conv_compare,
     _conv_trace, _pair_compare, _attn_trace, _mma_rate*, _flow_attention, _rel_attention, _convflow_spline, _durations,
-    _umma_layer, _dec_post), which the product library does not export."""
+    _umma_layer, _dec_post, _bert_bucket_table, _deberta_attention), which the product library does not export."""
     global _debug_lib
     if _debug_lib is None:
         path = os.path.join(_HERE, "libsbv2_b200_debug.so")
@@ -142,6 +142,45 @@ def debug_lib() -> C.CDLL:
         _debug_lib = C.CDLL(path)
         _debug_lib.sbv2_last_error.restype = C.c_char_p
     return _debug_lib
+
+
+def _debug_check(status: int) -> None:
+    if status != OK:
+        raise Sbv2Error(status, debug_lib().sbv2_last_error().decode("utf-8", "replace"))
+
+
+def debug_bert_bucket_table(span: int) -> np.ndarray:
+    """The DeBERTa relative-position bucket table of `span` position buckets as the model builds it at load: entry
+    d + R for d = -R..R, R = (len - 1) // 2 being the bound beyond which every distance reads the row of +-R."""
+    D = debug_lib()
+    r = C.c_int(0)
+    _debug_check(D.sbv2_debug_bert_bucket_table(C.c_int(span), C.byref(r), None))
+    out = np.zeros(2 * r.value + 1, np.int32)
+    _debug_check(D.sbv2_debug_bert_bucket_table(C.c_int(span), C.byref(r), out.ctypes.data_as(C.POINTER(C.c_int))))
+    return out
+
+
+DEBERTA_ATTN_MODES = {"single": 0, "multi": 1, "exact-multi": 2, "simt": 3}
+
+
+def debug_deberta_attention(qkv: np.ndarray, pos_k: np.ndarray, pos_q: np.ndarray, lens, heads: int, mode: str,
+                            far_pairs: bool = True, sc: float = 16.0, reps: int = 0):
+    """One DeBERTa attention launch (sbv2_debug_deberta_attention) on a ragged batch: qkv fp16 [terms, sum(lens), 3*heads*64],
+    pos_k / pos_q fp16 [terms, 2*span, heads*64]; terms = 2 (the split terms of values scaled by sc) for mode "exact-multi",
+    else 1.  Returns the context, fp16 [terms, sum(lens), heads*64] (exact-multi: the two terms of context * sc); with
+    reps > 0, (context, mean ms of `reps` more launches timed with CUDA events)."""
+    terms = 2 if mode == "exact-multi" else 1
+    lens_a = np.ascontiguousarray(lens, dtype=np.int32)
+    qkv = np.ascontiguousarray(qkv, dtype=np.float16).reshape(terms, int(lens_a.sum()), 3 * heads * 64)
+    pos_k = np.ascontiguousarray(pos_k, dtype=np.float16).reshape(terms, -1, heads * 64)
+    pos_q = np.ascontiguousarray(pos_q, dtype=np.float16).reshape(pos_k.shape)
+    out = np.zeros((terms, int(lens_a.sum()), heads * 64), np.float16)
+    u16, ms = C.POINTER(C.c_uint16), C.c_float(0.0)
+    _debug_check(debug_lib().sbv2_debug_deberta_attention(
+        qkv.ctypes.data_as(u16), pos_k.ctypes.data_as(u16), pos_q.ctypes.data_as(u16), lens_a.ctypes.data_as(C.POINTER(C.c_int)),
+        len(lens_a), heads, pos_k.shape[1] // 2, DEBERTA_ATTN_MODES[mode], int(bool(far_pairs)), C.c_float(sc), reps, C.byref(ms),
+        out.ctypes.data_as(u16)))
+    return (out, ms.value) if reps > 0 else out
 
 
 def _check(status: int) -> None:
