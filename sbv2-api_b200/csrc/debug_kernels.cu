@@ -1,9 +1,9 @@
 // Unit-test hooks of the synthesizer kernels between the text encoder and the decoder: the flow's window attention
 // (tensor-core and planar CUDA-core), the text encoder's fp32 attention, the inverse spline of the stochastic duration
-// predictor, the length regulator, and the HiFi-GAN decoder's tensor-core layers and conv_post.  Linked into
-// libsbv2_b200_debug.so only (build.py DEBUG_ONLY).  Every hook runs on its own stream, takes host arrays and returns host
-// arrays before it returns; tests/test_gpu_synth_kernels.py and tests/test_gpu_decoder_kernels.py compare the results
-// with float64 references.
+// predictor, the length regulator, the HiFi-GAN decoder's tensor-core layers and conv_post, the split-fp16 layers, the
+// WaveNet gate and DeBERTa's kernels.  Linked into libsbv2_b200_debug.so only (build.py DEBUG_ONLY).  Every hook runs on
+// its own stream, takes host arrays and returns host arrays before it returns; tests/test_gpu_synth_kernels.py,
+// tests/test_gpu_decoder_kernels.py and tests/test_gpu_split_gemm.py compare the results with float64 references.
 #include <cuda_fp16.h>
 
 #include <algorithm>
@@ -387,6 +387,275 @@ extern "C" int sbv2_debug_dec_post(const float* x, const int* lens, const long l
     float* d_wave = upload(owner, wave, size_t(wave_len));
     launch_dec_post_planar(owner.ctx(), d_wave, d_x, G, bg.d_wstart, n, upload(owner, wh.data(), wh.size()), wh, C, k, force_generic != 0);
     download(owner, wave, d_wave, size_t(wave_len));
+  });
+}
+
+// ---- split-fp16 layers, the WaveNet gate, DeBERTa's LayerNorms -----------------------------------------------------
+namespace {
+
+// A ragged batch packed back to back (ystart) and its planar geometry (one time resolution).
+struct Ragged {
+  DBuf meta;
+  PinnedBuf pin;
+  BatchGeom bg;
+  std::vector<int> ystart;
+  long long rows = 0;
+  std::vector<char> in_utt;  // planar rows that belong to an utterance
+  const Geom& g() const { return bg.g[0]; }
+};
+
+void ragged(sbv2_model& owner, const int* lens, int n, Ragged* r) {
+  SBV2_REQUIRE(lens && n > 0, "need at least one utterance");
+  r->ystart.assign(lens, lens + n);
+  const std::vector<int> ylen(lens, lens + n), muls{1};
+  for (int b = 0; b < n; ++b) {
+    SBV2_REQUIRE(lens[b] >= 1, "utterance lengths must be positive");
+    r->ystart[size_t(b)] = int(r->rows);
+    r->rows += lens[b];
+    SBV2_REQUIRE(r->rows < INT_MAX, "too many rows");
+  }
+  r->meta.stream = owner.stream;
+  r->bg = build_geoms(&owner, r->meta, r->pin, r->ystart, ylen, muls);
+  r->in_utt.assign(size_t(r->g().rows_tot), 0);
+  for (int b = 0; b < n; ++b)
+    for (int t = 0; t < lens[b]; ++t) r->in_utt[size_t(r->g().pstart[size_t(b)]) + t] = 1;
+}
+
+PlanarSegs planar_segs(const Ragged& r, int n) {
+  PlanarSegs ps;
+  ps.start = r.bg.d_ystart;
+  ps.pstart = r.g().d_pstart;
+  ps.len = r.g().d_len;
+  ps.order = r.bg.d_order;
+  ps.n = n;
+  ps.max_len = r.g().max_len;
+  ps.plane_stride = r.g().rows_tot * 8;
+  return ps;
+}
+
+// planar 16-bit [planes][rows_tot][8] -> packed [rows][planes * 8] (utterance rows only)
+void unplanar(uint16_t* dst, const std::vector<uint16_t>& buf, int planes, const Ragged& r, int n) {
+  const Geom& G = r.g();
+  const size_t plane = size_t(G.rows_tot) * 8;
+  for (int b = 0; b < n; ++b)
+    for (int t = 0; t < G.len[size_t(b)]; ++t) {
+      const size_t pr = size_t(G.pstart[size_t(b)]) + t;
+      uint16_t* row = dst + (size_t(r.ystart[size_t(b)]) + t) * planes * 8;
+      for (int c = 0; c < planes * 8; ++c) row[c] = buf[size_t(c / 8) * plane + pr * 8 + c % 8];
+    }
+}
+
+// planar rows outside every utterance in which some element of the fp16 buffer no longer holds kHalfSentinel
+long long stray_rows(const std::vector<uint16_t>& buf, int planes, const Ragged& r) {
+  const size_t plane = size_t(r.g().rows_tot) * 8;
+  long long n = 0;
+  for (size_t pr = 0; pr < size_t(r.g().rows_tot); ++pr) {
+    if (r.in_utt[pr]) continue;
+    bool w = false;
+    for (int pl = 0; pl < planes && !w; ++pl)
+      for (int e = 0; e < 8; ++e) w |= buf[size_t(pl) * plane + pr * 8 + e] != kHalfSentinel;
+    n += w ? 1 : 0;
+  }
+  return n;
+}
+
+}  // namespace
+
+// One split-fp16 layer (make_split_conv1d_layer(terms, mt_pref, nb_max), dilation dil) on a ragged batch, as the text
+// encoder and exact-mode DeBERTa run it.  w [cout][cin][k], bias [cout] or null, x packed fp32 [sum(lens), cin] (the
+// values the layer receives): the input split planes come from launch_split_planar, with zero gaps (launch_zero_gaps),
+// in a buffer that holds kHalfSentinel everywhere before.  bias_utt [n][cout] or null; act_out ACT_NONE / ACT_RELU /
+// ACT_GELU; tmap, splitk, cluster as the ConvCall fields.
+//   rm:    out fp32 [sum(lens), cout] <- the row-major output (each element holds an fp32 NaN payload before the launch)
+//   split: out_split [sum(lens)][3 * cout] <- the ConvCall::split_out plane blocks [h0 | h1 | h0], scaled by split_scale
+// in_split [sum(lens)][3 or 6 * cin] <- the input plane blocks.  pad_rows[0] / [1]: planar rows outside every utterance
+// written by launch_split_planar / into split_out (both buffers start as kHalfSentinel).  cfg[4]: the layer's mt, nb,
+// n_nblk, nkc; scales[2]: in_scale, out_scale; report[4]: what launch_umma chose (UmmaLaunchReport: variant, cluster,
+// splitk, tmap).
+extern "C" int sbv2_debug_split_layer(const float* w, const float* bias, int cin, int cout, int k, int dil, int terms, int mt_pref, int nb_max,
+                                      const float* x, const int* lens, int n, const float* bias_utt, int act_out, int rm, int split,
+                                      float split_scale, int tmap, int splitk, int cluster, float* out, uint16_t* out_split,
+                                      uint16_t* in_split, long long* pad_rows, int* cfg, float* scales, int* report) {
+  return guarded([&] {
+    SBV2_REQUIRE(w && x && in_split && cin > 0 && cout > 0 && k > 0 && (terms == 2 || terms == 3), "bad arguments");
+    SBV2_REQUIRE((rm || split) && (!rm || out) && (!split || out_split), "the layer needs an output");
+    SBV2_REQUIRE(act_out == ACT_NONE || act_out == ACT_RELU || act_out == ACT_GELU, "the row-major epilogue applies none, relu or gelu");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    HostConv hc;
+    hc.d0 = cout;
+    hc.d1 = cin;
+    hc.k = k;
+    hc.w.assign(w, w + size_t(cin) * cout * k);
+    if (bias) hc.b.assign(bias, bias + cout);
+    const ConvLayer L = make_split_conv1d_layer(&owner, hc, dil, mt_pref, terms, nb_max);
+    if (cfg) {
+      cfg[0] = L.mt;
+      cfg[1] = L.nb;
+      cfg[2] = L.n_nblk;
+      cfg[3] = L.nkc;
+    }
+    if (scales) {
+      scales[0] = L.in_scale;
+      scales[1] = L.out_scale;
+    }
+    Ragged R;
+    ragged(owner, lens, n, &R);
+    const Geom& G = R.g();
+    const int nblk = terms == 3 ? 6 : 3;
+    const size_t plane = size_t(G.rows_tot) * 8;
+    std::vector<uint16_t> hi(size_t(nblk) * (cin / 8) * plane, kHalfSentinel);
+    __half* d_in = reinterpret_cast<__half*>(upload(owner, hi.data(), hi.size()));
+    launch_split_planar(ctx, d_in, upload(owner, x, size_t(R.rows) * cin), cin, cin, R.bg.d_ystart, G, n, terms, L.in_scale);
+    download(owner, hi.data(), reinterpret_cast<const uint16_t*>(d_in), hi.size());
+    unplanar(in_split, hi, nblk * cin / 8, R, n);
+    const long long stray_in = stray_rows(hi, nblk * cin / 8, R);
+    launch_zero_gaps(ctx, d_in, nblk * cin, G, n);
+
+    ConvCall c;
+    c.in = d_in;
+    c.act_out = act_out;
+    if (bias_utt) c.bias_utt = upload(owner, bias_utt, size_t(n) * cout);
+    std::vector<uint32_t> ho;
+    if (rm) {
+      ho.assign(size_t(R.rows) * cout, kFloatSentinel);
+      c.rm_out = reinterpret_cast<float*>(upload(owner, ho.data(), ho.size()));
+      c.rm_ld = cout;
+      c.rm_start = R.bg.d_ystart;
+    }
+    std::vector<uint16_t> hs;
+    if (split) {
+      hs.assign(size_t(3) * (cout / 8) * plane, kHalfSentinel);
+      c.split_out = reinterpret_cast<__half*>(upload(owner, hs.data(), hs.size()));
+      c.split_scale = split_scale;
+    }
+    c.tmap = tmap != 0;
+    c.splitk = splitk != 0;
+    c.cluster = cluster;
+    UmmaLaunchReport rep;
+    c.report = &rep;
+    launch_umma(ctx, L, G, G, c, n);
+    if (rm) {
+      download(owner, ho.data(), reinterpret_cast<const uint32_t*>(c.rm_out), ho.size());
+      memcpy(out, ho.data(), ho.size() * 4);
+    }
+    long long stray_out = 0;
+    if (split) {
+      download(owner, hs.data(), reinterpret_cast<const uint16_t*>(c.split_out), hs.size());
+      unplanar(out_split, hs, 3 * cout / 8, R, n);
+      stray_out = stray_rows(hs, 3 * cout / 8, R);
+    }
+    if (pad_rows) {
+      pad_rows[0] = stray_in;
+      pad_rows[1] = stray_out;
+    }
+    if (report) {
+      report[0] = rep.variant;
+      report[1] = rep.cluster;
+      report[2] = rep.splitk;
+      report[3] = rep.tmap;
+    }
+  });
+}
+
+// One WaveNet in_layer (make_gated_conv1d_layer, Conv1d cin -> 2 * hidden, k taps, dilation dil) on a ragged batch,
+// launched as the WN flow launches it: gate_half, and the conditioning as bias_utt with a row stride (bias_utt_ld) wider
+// than 2 * hidden.  w [2 * hidden][cin][k] and bias [2 * hidden] (or null) in the original channel order: channels
+// [0, hidden) feed tanh, [hidden, 2 * hidden) the sigmoid.  cond [n][2 * hidden]: each utterance's conditioning, also in
+// the original order; the hook permutes it with the layer's perm as the model permutes cond_layer.  x packed fp32
+// [sum(lens), cin], stored as planar fp16 with zero gaps.  out [sum(lens)][hidden] <- tanh(.) * sigmoid(.) as fp16
+// values; pad_rows[0]: planar output rows outside every utterance written.  cfg[4]: gate_half, nb, n_nblk, mt.
+extern "C" int sbv2_debug_gated_layer(const float* w, const float* bias, int cin, int hidden, int k, int dil, int mt_pref, const float* x,
+                                      const int* lens, int n, const float* cond, float* out, long long* pad_rows, int* cfg) {
+  return guarded([&] {
+    SBV2_REQUIRE(w && x && cond && out && cin > 0 && hidden > 0 && k > 0, "bad arguments");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    HostConv hc;
+    hc.d0 = 2 * hidden;
+    hc.d1 = cin;
+    hc.k = k;
+    hc.w.assign(w, w + size_t(cin) * 2 * hidden * k);
+    if (bias) hc.b.assign(bias, bias + 2 * hidden);
+    int gate_half = 0;
+    std::vector<int> perm;
+    const ConvLayer L = make_gated_conv1d_layer(&owner, hc, dil, mt_pref, &gate_half, &perm);
+    if (cfg) {
+      cfg[0] = gate_half;
+      cfg[1] = L.nb;
+      cfg[2] = L.n_nblk;
+      cfg[3] = L.mt;
+    }
+    Ragged R;
+    ragged(owner, lens, n, &R);
+    const Geom& G = R.g();
+    const int ld = 2 * hidden + 32;
+    std::vector<float> cp(size_t(n) * ld, 0.f);
+    for (int b = 0; b < n; ++b)
+      for (int i = 0; i < 2 * hidden; ++i) cp[size_t(b) * ld + i] = cond[size_t(b) * 2 * hidden + perm[size_t(i)]];
+    const size_t plane = size_t(G.rows_tot) * 8;
+    std::vector<uint16_t> ho(size_t(hidden / 8) * plane, kHalfSentinel);
+    ConvCall c;
+    c.in = planar_input(owner, x, cin, R.bg.d_ystart, G, n);
+    c.out = reinterpret_cast<__half*>(upload(owner, ho.data(), ho.size()));
+    c.gate_half = gate_half;
+    c.bias_utt = upload(owner, cp.data(), cp.size());
+    c.bias_utt_ld = ld;
+    launch_umma(ctx, L, G, G, c, n);
+    download(owner, ho.data(), reinterpret_cast<const uint16_t*>(c.out), ho.size());
+    std::vector<uint16_t> packed(size_t(R.rows) * hidden);
+    unplanar(packed.data(), ho, hidden / 8, R, n);
+    for (size_t i = 0; i < packed.size(); ++i) out[i] = __half2float(__ushort_as_half(packed[i]));
+    if (pad_rows) pad_rows[0] = stray_rows(ho, hidden / 8, R);
+  });
+}
+
+// One of DeBERTa's LayerNorms on a ragged batch: a, addin packed fp32 [sum(lens), C] (addin may be null), gamma / beta [C].
+//   mode 0: launch_ln_split(out, split, split_scale, a, addin): out [sum(lens)][C] <- LN(a + addin) (each element holds an
+//           fp32 NaN payload before), planes [sum(lens)][3 * C] <- the split blocks [h0 | h1 | h0]
+//   mode 1: launch_ln_planar_wide(h = a, hp, hp2, y32 = addin as planar fp32): out <- h, planes [sum(lens)][2 * C] <- hp | hp2
+// pad_rows[0]: planar rows outside every utterance written into the planes (which hold kHalfSentinel before).
+extern "C" int sbv2_debug_bert_layernorm(int mode, const float* a, const float* addin, const float* gamma, const float* beta, float eps, int C,
+                                         const int* lens, int n, float split_scale, float* out, uint16_t* planes, long long* pad_rows) {
+  return guarded([&] {
+    SBV2_REQUIRE(a && gamma && beta && out && planes && (mode == 0 || mode == 1) && C > 0, "bad arguments");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    Ragged R;
+    ragged(owner, lens, n, &R);
+    const Geom& G = R.g();
+    const PlanarSegs ps = planar_segs(R, n);
+    const size_t plane = size_t(G.rows_tot) * 8, elems = size_t(R.rows) * C;
+    const int nbuf = mode == 0 ? 3 : 2;
+    std::vector<uint16_t> hp(size_t(nbuf) * (C / 8) * plane, kHalfSentinel);
+    __half* d_hp = reinterpret_cast<__half*>(upload(owner, hp.data(), hp.size()));
+    const float* d_g = upload(owner, gamma, size_t(C));
+    const float* d_b = upload(owner, beta, size_t(C));
+    float* d_out;
+    if (mode == 0) {
+      const std::vector<uint32_t> sentinel(elems, kFloatSentinel);
+      d_out = reinterpret_cast<float*>(upload(owner, sentinel.data(), elems));
+      launch_ln_split(ctx, d_out, d_hp, split_scale, upload(owner, a, elems), addin ? upload(owner, addin, elems) : nullptr, d_g, d_b, eps, C, ps);
+    } else {
+      d_out = upload(owner, a, elems);
+      const float* d_y = nullptr;
+      if (addin) {
+        std::vector<float> y((C / 8) * plane, 0.f);
+        for (int b = 0; b < n; ++b)
+          for (int t = 0; t < lens[b]; ++t)
+            for (int c = 0; c < C; ++c)
+              y[size_t(c / 8) * plane + (size_t(G.pstart[size_t(b)]) + t) * 8 + c % 8] = addin[(size_t(R.ystart[size_t(b)]) + t) * C + c];
+        d_y = upload(owner, y.data(), y.size());
+      }
+      launch_ln_planar_wide(ctx, d_out, d_hp, d_hp + size_t(C / 8) * plane, d_y, d_g, d_b, eps, C, ps);
+    }
+    download(owner, out, d_out, elems);
+    download(owner, hp.data(), reinterpret_cast<const uint16_t*>(d_hp), hp.size());
+    unplanar(planes, hp, nbuf * C / 8, R, n);
+    if (pad_rows) pad_rows[0] = stray_rows(hp, nbuf * C / 8, R);
   });
 }
 

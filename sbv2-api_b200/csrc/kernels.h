@@ -195,7 +195,7 @@ void launch_coupling_sub_planar(const LaunchCtx& ctx, float* z, const float* m32
 
 // ---- DeBERTa glue (bert_kernels.cu) ----------------------------------------------------------------
 namespace sbv2 {
-// h = LN(h + y32) * gamma + beta for any C <= 1024 (multiple of 256 or <= 256); y32 planar fp32 or null;
+// h = LN(h + y32) * gamma + beta for any C that is a multiple of 8 and <= 1024; y32 planar fp32 or null;
 // also writes the planar fp16 copy hp (and hp2 if not null).
 void launch_ln_planar_wide(const LaunchCtx& ctx, float* h, __half* hp, __half* hp2, const float* y32, const float* gamma,
                            const float* beta, float eps, int C, const PlanarSegs& s);
@@ -218,6 +218,7 @@ void launch_deberta_attention_f32(const LaunchCtx& ctx, float* ctx_out, __half* 
                                   const float* pos_k_t, const float* pos_q_t, int n_pos, const int* bucket_idx, int max_rel, int heads,
                                   int head_dim, const PlanarSegs& s);
 // out = LN(a + addin) (fp32 row-major [rows, C], out optional) and the split-planar operand of the consuming GEMM in one pass
+// (any C that is a multiple of 8 and <= 1024)
 bool ln_split_supported(int C);
 void launch_ln_split(const LaunchCtx& ctx, float* out, __half* split, float split_scale, const float* a, const float* addin,
                      const float* gamma, const float* beta, float eps, int C, const PlanarSegs& s);

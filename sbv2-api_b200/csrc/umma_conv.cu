@@ -1006,7 +1006,8 @@ ConvLayer make_split_conv1d_layer(sbv2_model* owner, const HostConv& c, int dil,
     wexp = 13 - wexp;
   }
   const float wscale = std::ldexp(1.0f, wexp);
-  const float in_scale = 16.f;  // activations up to ~4000 in magnitude stay finite in fp16
+  // activations with |x| < 4095 stay finite in fp16: 16 * 4094.97 rounds to 65504, 16 * 4095 = 65520 rounds to infinity
+  const float in_scale = 16.f;
   for (int co = 0; co < c.d0; ++co)
     for (int ci = 0; ci < c.d1; ++ci)
       for (int j = 0; j < c.k; ++j) {
@@ -1121,6 +1122,7 @@ void launch_umma(const LaunchCtx& ctx, const ConvLayer& L, const Geom& gi, const
   a.split_npl = L.cout / 8;
   a.split_scale = c.split_scale;
   a.trace = g_trace;
+  if (c.report) *c.report = UmmaLaunchReport{};
   if (gi.n_tiles[slot] <= 0) return;
   static int num_sms = 0;
   if (num_sms == 0) {
@@ -1196,7 +1198,10 @@ void launch_umma(const LaunchCtx& ctx, const ConvLayer& L, const Geom& gi, const
     grid = dim3(a.n_items * splitk);  // one item per cluster
   }
   void (*kernel)(UmmaConvArgs) = nullptr;
-  switch ((c.gate_half > 0 ? 1 : 0) | (pair ? 8 : (splitk > 1 ? 16 : (nc > 1 ? 2 : 0))) | ((c.rm_out != nullptr || c.split_out != nullptr) ? 4 : 0)) {
+  const int variant =
+      (c.gate_half > 0 ? 1 : 0) | (pair ? 8 : (splitk > 1 ? 16 : (nc > 1 ? 2 : 0))) | ((c.rm_out != nullptr || c.split_out != nullptr) ? 4 : 0);
+  if (c.report) *c.report = UmmaLaunchReport{variant, nc, splitk, a.use_tmap};
+  switch (variant) {
     case 0: kernel = umma_conv_kernel<0>; break;
     case 1: kernel = umma_conv_kernel<1>; break;
     case 2: kernel = umma_conv_kernel<2>; break;

@@ -102,10 +102,17 @@ BatchGeom build_geoms(sbv2_model* owner, DBuf& dev, PinnedBuf& pin, const std::v
 // accumulator by ConvLayer::out_scale = 1 / (in_scale * weight scale) — exact.
 // The layer's input is the planar tensor written by launch_split_planar with the same `terms` and in_scale.
 ConvLayer make_split_conv1d_layer(sbv2_model* owner, const HostConv& c, int dil, int mt_pref, int terms, int nb_max = 256);
-// packed fp32 [rows, in_ld] (first C columns) * in_scale -> planar fp16 split terms; gap rows are not written
+// packed fp32 [rows, in_ld] (first C columns) * in_scale -> planar fp16 split terms in plane blocks [h0 | h1 | h0]
+// (terms = 2) or [h0 | h1 | h2 | h0 | h1 | h0] (terms = 3), each block C / 8 planes; gap rows are not written
 void launch_split_planar(const LaunchCtx& ctx, __half* out, const float* in, int in_ld, int C, const int* d_start, const Geom& g,
                          int n_utt, int terms, float in_scale);
 enum UAccum { UACC_NONE = 0, UACC_SET = 1, UACC_ADD = 2, UACC_FINAL = 3 };
+// What launch_umma chose for one call (ConvCall::report): the umma_conv_kernel VARIANT, CTAs per thread-block cluster
+// (multicast, CTA pair or split-K; 1: none), the split-K factor S (1: none) and whether activation chunks came by tensor
+// map.  All zero when the launch had no rows.
+struct UmmaLaunchReport {
+  int variant = 0, cluster = 0, splitk = 0, tmap = 0;
+};
 struct ConvCall {
   const __half* in = nullptr;
   __half* out = nullptr;          // planar fp16 (optional)
@@ -125,7 +132,7 @@ struct ConvCall {
   int gate_half = 0;
   int out_mul = 1, out_off = 0;
   // fp32 row-major output [packed rows, rm_ld] instead of the planar ones (text encoder): packed row = rm_start[b] + t;
-  // act_out ACT_NONE / ACT_RELU only
+  // act_out ACT_NONE / ACT_RELU / ACT_GELU only
   float* rm_out = nullptr;
   int rm_ld = 0;
   const int* rm_start = nullptr;
@@ -145,6 +152,8 @@ struct ConvCall {
   // split K over a thread-block cluster when the launch has few items (see launch_umma): the fp32 sums are formed in a
   // different order than without the split, so callers that promise batch == single results bit for bit must not ask
   bool splitk = false;
+  // tests: receives what launch_umma chose (null in production calls)
+  UmmaLaunchReport* report = nullptr;
 };
 void launch_umma(const LaunchCtx& ctx, const ConvLayer& L, const Geom& gi, const Geom& go, const ConvCall& c, int n_utt);
 void launch_zero_gaps(const LaunchCtx& ctx, __half* buf, int C, const Geom& g, int n_utt);
