@@ -169,6 +169,38 @@ int sbv2_synthesize_from_tokens_batch(sbv2_model* synth, sbv2_model* bert, const
                                       const int64_t* pause_after /* [batch] or NULL */, float** out_samples,
                                       int64_t* out_total, int64_t* out_n_samples /* [batch] or NULL */);
 
+/* Style-Bert-VITS2's assist text (`assist_text`, `assist_text_weight`; style_bert_vits2/nlp/japanese/bert_feature.py
+ * extract_bert_feature): the tone of a sentence is steered toward another text by mixing that text's mean DeBERTa row into
+ * the feature of every phoneme.  The assist text is normalised and tokenised by the caller exactly as the main text
+ * (CLS ... SEP); an empty assist text means no blend (pass none).
+ *
+ * Numerics (bit for bit, on the device and in the host restatement of host/tts.hpp, tts_util::assist_mean /
+ * expand_bert_features):
+ *   F_a[t][c]   DeBERTa rows of the assist (hidden_states[-3], fp32), n_a = t_tok tokens, CLS and SEP included
+ *   mean_a[c] = (float)((sum_{t=0..n_a-1} (double)F_a[t][c]) / (double)n_a), one fp64 accumulator per column, token order
+ *   c_row     = (float)(1.0 - (double)weight), c_mean = weight
+ *   row of phoneme p (token t) = fl(fl(F[t][c] * c_row) + fl(mean_a[c] * c_mean)), no fused multiply-add
+ * The weight must be finite; any finite value is accepted (the reference does not clamp it).  A weight of 0 (or no
+ * assist) takes the plain gather and never sends the assist through DeBERTa, so the result is bit-identical to
+ * sbv2_synthesize_from_tokens_batch.
+ * DeBERTa batch of one call: [sentences..., used assists...] right-padded to the longest row, where the used assists are
+ * those some sentence names with a non-zero weight, in index order.  (Which rows share a call decides the GEMM path, and
+ * thereby the last bits of every row: see DESIGN.md §4.) */
+typedef struct sbv2_assist_text {
+  const int64_t* input_ids;      /* [t_tok], the assist text through the same tokenizer */
+  const int64_t* attention_mask; /* [t_tok], all ones */
+  int64_t t_tok;                 /* 1 .. 32768 */
+  float weight;                  /* assist_text_weight; 0 = no blend (DeBERTa is not run on it) */
+} sbv2_assist_text;
+/* sbv2_synthesize_from_tokens_batch with assist texts: sentence i blends assists[assist_of[i]] (-1 = none; assist_of NULL =
+ * none for all).  Each sentence may carry its own assist, as it carries its own sid / style_vec / sdp_ratio.
+ * SBV2_ERR_INVALID_ARGUMENT: assist_of out of [-1, n_assists), an assist with null arrays, t_tok outside 1 .. 32768, a mask
+ * with a zero, or a non-finite weight (every entry of `assists` is checked, used or not). */
+int sbv2_synthesize_from_tokens_assist(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                       const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of /* [batch] or NULL */,
+                                       const int64_t* pause_after /* [batch] or NULL */, float** out_samples, int64_t* out_total,
+                                       int64_t* out_n_samples /* [batch] or NULL */);
+
 /* Batched, variable-length extension.  Per-utterance pointer arrays of length `batch`; every
  * utterance's result is bit-identical to its own batch-1 call.  Results land in one pinned block:
  * `*out_samples` float32 [sum n_samples[b]] back to back, `out_n_samples` int64 [batch] caller
@@ -265,6 +297,10 @@ int sbv2_holder_get_style_vector(sbv2_holder* h, const char* ident, int32_t styl
  * (tts_util.rs:120-154).  out: float32 [hidden, sum(word2ph)] library-allocated. */
 int sbv2_holder_bert_features(sbv2_holder* h, const int64_t* token_ids, const int64_t* attention_mask,
                               int64_t t_tok, const int32_t* word2ph, float** out, int64_t* t_x);
+/* The same with an assist text (NULL = none): one DeBERTa batch [sentence, assist] (the layout of
+ * sbv2_synthesize_from_tokens_assist), then the blend on the host with the numerics stated there. */
+int sbv2_holder_bert_features_assist(sbv2_holder* h, const int64_t* token_ids, const int64_t* attention_mask, int64_t t_tok,
+                                     const int32_t* word2ph, const sbv2_assist_text* assist, float** out, int64_t* t_x);
 /* easy_synthesize from already-parsed sentences (one entry per non-empty '\n'-separated line):
  * find_and_load_model, get_style_vector, per-sentence synthesize, 22050 zero samples between
  * sentences (`total_lines` is the number of lines of the original text incl. empty ones and
@@ -301,6 +337,12 @@ int sbv2_holder_easy_synthesize_tokens(sbv2_holder* h, const char* ident, const 
                                        int n_sentences, int64_t total_lines, int32_t style_id, int64_t speaker_id,
                                        float sdp_ratio, float length_scale, float style_weight,
                                        void** wav_bytes, size_t* wav_n);
+/* The same with an assist text (NULL = none) that applies to every line, as the reference's TTSModel.infer passes it to
+ * each line of a request. */
+int sbv2_holder_easy_synthesize_tokens_assist(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences,
+                                              int n_sentences, int64_t total_lines, int32_t style_id, int64_t speaker_id,
+                                              float sdp_ratio, float length_scale, float style_weight,
+                                              const sbv2_assist_text* assist, void** wav_bytes, size_t* wav_n);
 
 #ifdef __cplusplus
 }

@@ -513,6 +513,29 @@ __global__ void __launch_bounds__(256) deberta_attention_kernel(void* out_v, con
   }
 }
 
+// mean[a, c] = (float)((sum_t (double)feat[row0 + a][t][c]) / len[row0 + a]), t = 0 .. len-1 in order.  One thread per
+// column: the threads of a warp read 32 consecutive floats of one token row (coalesced), and every group of TM_UNROLL
+// loads is issued before the dependent fp64 adds consume it.  The sequential fp64 sum is what the host restates bit for bit.
+constexpr int TM_THREADS = 128, TM_UNROLL = 8;
+__global__ void __launch_bounds__(TM_THREADS) token_mean_kernel(float* __restrict__ mean, const float* __restrict__ feat,
+                                                                const int* __restrict__ len, int row0, int S, int H) {
+  const int a = blockIdx.y, c = blockIdx.x * TM_THREADS + threadIdx.x;
+  if (c >= H) return;
+  const int n = len[row0 + a];
+  const float* p = feat + (size_t)(row0 + a) * S * H + c;
+  double acc = 0.0;
+  int t = 0;
+  for (; t + TM_UNROLL <= n; t += TM_UNROLL) {
+    float v[TM_UNROLL];
+#pragma unroll
+    for (int k = 0; k < TM_UNROLL; ++k) v[k] = __ldg(p + (size_t)(t + k) * H);
+#pragma unroll
+    for (int k = 0; k < TM_UNROLL; ++k) acc += (double)v[k];
+  }
+  for (; t < n; ++t) acc += (double)__ldg(p + (size_t)t * H);
+  mean[(size_t)a * H + c] = (float)(acc / (double)n);
+}
+
 }  // namespace
 
 #define POST_LAUNCH(ctx)            \
@@ -558,6 +581,13 @@ void launch_scatter_rows(const LaunchCtx& ctx, float* out, const float* h, int C
   if (s.n <= 0 || S <= 0) return;
   dim3 grid(S, s.n);
   scatter_rows_kernel<<<grid, 128, 0, ctx.stream>>>(out, h, C, S, s);
+  POST_LAUNCH(ctx);
+}
+
+void launch_token_mean(const LaunchCtx& ctx, float* mean, const float* feat, const int* len, int row0, int n, int S, int H) {
+  if (n <= 0 || H <= 0) return;
+  dim3 grid((H + TM_THREADS - 1) / TM_THREADS, n);
+  token_mean_kernel<<<grid, TM_THREADS, 0, ctx.stream>>>(mean, feat, len, row0, S, H);
   POST_LAUNCH(ctx);
 }
 

@@ -45,6 +45,10 @@ struct BertModel : sbv2_model {
   float *conv_g = nullptr, *conv_b = nullptr;
   int* bucket_idx = nullptr;  // device [2*max_rel+1] (bert_bucket_table)
   DBuf ids, h, embp, hp, qkvp, ctxp, f1p, y32, meta, outd;
+  DBuf meand;                  // bert_token_mean's output; like outd, valid until the model's next call
+  const int* out_len = nullptr;  // device [batch]: valid tokens of each row of outd (in `meta`)
+  int out_batch = 0;
+  int64_t out_S = 0;
   uint64_t qkvp_cleared_gen = 0;  // DBuf::gen of the qkv buffer that was zero-filled last (its tail rows must be finite)
   bool use_tc_attn = true;       // SBV2_B200_BERT_ATTN=simt (read at model creation) keeps the CUDA-core attention
   bool exact = true;             // SBV2_B200_BERT=fp16 selects the single-term fp16 path
@@ -290,7 +294,7 @@ sbv2_model* create_bert_model(const OnnxModel& m, int device) {
     const std::vector<int> tab = bert_bucket_table(M->span, &M->max_rel);
     M->bucket_idx = static_cast<int*>(M->upload_bytes(tab.data(), tab.size() * 4));
   }
-  for (DBuf* b : {&M->ids, &M->h, &M->embp, &M->hp, &M->qkvp, &M->ctxp, &M->f1p, &M->y32, &M->meta, &M->outd, &M->x_emb, &M->x_qkv, &M->x_qkvs, &M->x_ctx,
+  for (DBuf* b : {&M->ids, &M->h, &M->embp, &M->hp, &M->qkvp, &M->ctxp, &M->f1p, &M->y32, &M->meta, &M->outd, &M->meand, &M->x_emb, &M->x_qkv, &M->x_qkvs, &M->x_ctx,
                   &M->x_f1, &M->x_y, &M->x_split})
     b->stream = M->stream;
   std::ostringstream js;
@@ -356,6 +360,9 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
   ps.max_len = max_len;
   ps.plane_stride = G.rows_tot * 8;
   const size_t R = size_t(G.rows_tot);
+  M.out_len = G.d_len;
+  M.out_batch = batch;
+  M.out_S = S;
   M.h.ensure(size_t(n) * H * 4);
   M.region_begin("bert");
   if (M.exact) {
@@ -502,6 +509,15 @@ const float* bert_forward_device(sbv2_model* mm, const int64_t* ids, const int64
   M.region_end("bert");
   M.debug["bert_h"] = DebugView{h, n, H, 4};
   return M.outd.as<float>();
+}
+
+const float* bert_token_mean(sbv2_model* mm, int row0, int n) {
+  auto& M = *static_cast<BertModel*>(mm);
+  M.bind_device();
+  SBV2_REQUIRE(M.out_len && row0 >= 0 && n > 0 && row0 + n <= M.out_batch, "token mean over rows the last forward did not produce");
+  M.meand.ensure(size_t(n) * M.hidden * 4);
+  launch_token_mean(M.ctx(), M.meand.as<float>(), M.outd.as<float>(), M.out_len, row0, n, int(M.out_S), M.hidden);
+  return M.meand.as<float>();
 }
 
 void bert_predict(sbv2_model* mm, const int64_t* ids, const int64_t* mask, int batch, int64_t S, float* out) {

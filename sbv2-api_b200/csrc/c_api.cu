@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 
 #include "container.h"
 #include "model.h"
@@ -250,25 +251,59 @@ int sbv2_synthesize_from_tokens(sbv2_model* synth, sbv2_model* bert, const int64
 
 int sbv2_synthesize_from_tokens_batch(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
                                       const int64_t* pause_after, float** out_samples, int64_t* out_total, int64_t* out_n_samples) {
+  return sbv2_synthesize_from_tokens_assist(synth, bert, utts, batch, nullptr, 0, nullptr, pause_after, out_samples, out_total,
+                                            out_n_samples);
+}
+
+int sbv2_synthesize_from_tokens_assist(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                       const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of,
+                                       const int64_t* pause_after, float** out_samples, int64_t* out_total, int64_t* out_n_samples) {
   return guarded([&] {
     SBV2_REQUIRE(synth && bert && utts && out_samples && out_total, "null argument");
     SBV2_REQUIRE(!synth->is_bert, "synthesize called on a BERT model");
     SBV2_REQUIRE(bert->is_bert, "bert_predict called on a synthesizer model");
     SBV2_REQUIRE(synth->device == bert->device, "the BERT and synthesizer models must live on the same device");
     SBV2_REQUIRE(batch > 0, "empty batch");
+    SBV2_REQUIRE(n_assists >= 0 && (assists || n_assists == 0), "null assists with n_assists > 0");
     *out_samples = nullptr;
     *out_total = 0;
-    // one right-padded DeBERTa batch over all sentences (bert.rs:6-24 per sentence in the reference)
+    for (int a = 0; a < n_assists; ++a) {
+      const sbv2_assist_text& x = assists[a];
+      SBV2_REQUIRE(x.input_ids && x.attention_mask, "null assist-text input");
+      SBV2_REQUIRE(x.t_tok > 0 && x.t_tok <= kMaxBertTokens, "assist text must have 1 .. 32768 tokens");
+      SBV2_REQUIRE(std::isfinite(x.weight), "assist_text_weight must be finite");
+      for (int64_t t = 0; t < x.t_tok; ++t)
+        SBV2_REQUIRE(x.attention_mask[t] != 0, "attention_mask of an assist text must be all ones (padding is added by the library)");
+    }
+    // DeBERTa batch: [sentences..., used assists...] right-padded to the longest row.  An assist is used when some
+    // sentence names it with a non-zero weight; used assists follow in index order and take slots 0, 1, ...
+    std::vector<char> named(size_t(n_assists), 0);
+    for (int i = 0; i < batch; ++i) {
+      const int a = assist_of ? assist_of[i] : -1;
+      SBV2_REQUIRE(a >= -1 && a < n_assists, "assist_of entry out of range");
+      if (a >= 0 && assists[a].weight != 0.f) named[size_t(a)] = 1;
+    }
+    std::vector<int> slot_of(size_t(n_assists), -1), used;
+    for (int a = 0; a < n_assists; ++a)
+      if (named[size_t(a)]) {
+        slot_of[size_t(a)] = int(used.size());
+        used.push_back(a);
+      }
+    const int rows_b = batch + int(used.size());
     int64_t s_max = 0, nx = 0;
     for (int i = 0; i < batch; ++i) {
       SBV2_REQUIRE(utts[i].input_ids && utts[i].attention_mask && utts[i].word2ph && utts[i].t_tok > 0 && utts[i].t_x > 0, "empty input");
       s_max = std::max(s_max, utts[i].t_tok);
       nx += utts[i].t_x;
     }
-    std::vector<int64_t> ids(size_t(batch) * s_max, 0), mask(size_t(batch) * s_max, 0), ph2tok;
+    for (int a : used) s_max = std::max(s_max, assists[a].t_tok);
+    std::vector<int64_t> ids(size_t(rows_b) * s_max, 0), mask(size_t(rows_b) * s_max, 0), ph2tok;
+    std::vector<int32_t> ph_slot;
     ph2tok.reserve(size_t(nx));
+    if (!used.empty()) ph_slot.reserve(size_t(nx));
     for (int i = 0; i < batch; ++i) {
       const sbv2_token_utterance& u = utts[i];
+      const int32_t slot = assist_of && assist_of[i] >= 0 ? slot_of[size_t(assist_of[i])] : -1;
       int64_t n_ph = 0;
       for (int64_t t = 0; t < u.t_tok; ++t) {
         SBV2_REQUIRE(u.attention_mask[t] != 0, "attention_mask of a sentence must be all ones (padding is added by the library)");
@@ -280,9 +315,27 @@ int sbv2_synthesize_from_tokens_batch(sbv2_model* synth, sbv2_model* bert, const
         n_ph += u.word2ph[t];
       }
       SBV2_REQUIRE(n_ph == u.t_x, "sum(word2ph) must equal the number of phonemes");
+      if (!used.empty()) ph_slot.insert(ph_slot.end(), size_t(n_ph), slot);
     }
-    const float* rows = bert_forward_device(bert, ids.data(), mask.data(), batch, s_max);
+    std::vector<float> coef(used.size() * 2);
+    for (size_t k = 0; k < used.size(); ++k) {
+      const sbv2_assist_text& x = assists[used[k]];
+      for (int64_t t = 0; t < x.t_tok; ++t) {
+        ids[(size_t(batch) + k) * s_max + t] = x.input_ids[t];
+        mask[(size_t(batch) + k) * s_max + t] = 1;
+      }
+      coef[2 * k] = float(1.0 - double(x.weight));
+      coef[2 * k + 1] = x.weight;
+    }
+    const float* rows = bert_forward_device(bert, ids.data(), mask.data(), rows_b, s_max);
     SBV2_REQUIRE(rows != nullptr, "attention_mask selects no token");
+    DeviceBert dev;
+    if (!used.empty()) {
+      dev.n_slots = int(used.size());
+      dev.means = bert_token_mean(bert, batch, int(used.size()));
+      dev.slot = ph_slot.data();
+      dev.coef = coef.data();
+    }
     cudaEvent_t ready = nullptr;
     CUDA_CHECK(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
     struct EventGuard {
@@ -290,9 +343,8 @@ int sbv2_synthesize_from_tokens_batch(sbv2_model* synth, sbv2_model* bert, const
       ~EventGuard() { cudaEventDestroy(e); }
     } guard{ready};
     CUDA_CHECK(cudaEventRecord(ready, bert->stream));
-    DeviceBert dev;
     dev.rows = rows;
-    dev.n_rows = int64_t(batch) * s_max;
+    dev.n_rows = int64_t(rows_b) * s_max;
     dev.hidden = bert_hidden(bert);
     dev.ph2tok = ph2tok.data();
     dev.ready = ready;

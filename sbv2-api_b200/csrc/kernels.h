@@ -108,6 +108,10 @@ void launch_embed_combine(const LaunchCtx& ctx, float* h, const int* x, const in
                           int n_tones, int n_lang, const Segs& seg);
 // gather rows: out[b, :] = table[idx[b], :]
 void launch_gather_rows(const LaunchCtx& ctx, float* out, const float* table, const int64_t* idx, int n, int C, int n_rows);
+// assist-text blend: out[b, :] = __fadd_rn(__fmul_rn(table[idx[b], :], coef[s].x), __fmul_rn(mean[s, :], coef[s].y)), s = slot[b];
+// slot -1 copies the row as launch_gather_rows does.  16-byte loads when C % 4 == 0.
+void launch_gather_rows_blend(const LaunchCtx& ctx, float* out, const float* table, const int64_t* idx, const int* slot, const float* mean,
+                              const float2* coef, int n, int C, int n_rows, int n_slots);
 // x[row, c] (+)= v[b, c]; out may alias x.
 void launch_add_utt_vec(const LaunchCtx& ctx, float* out, const float* x, const float* v, int C, int v_ld, const Segs& seg);
 
@@ -242,4 +246,7 @@ void launch_deberta_attention_tc_multi(const LaunchCtx& ctx, __half* ctx_out, co
                                        int n_pos, const int* bucket_idx, int max_rel, int heads, bool far_pairs, const PlanarSegs& s);
 // out[b, t, :] = h[start[b] + t, :] for t < len[b], zeros elsewhere (out: [n, S, C] fp32)
 void launch_scatter_rows(const LaunchCtx& ctx, float* out, const float* h, int C, int S, const PlanarSegs& s);
+// mean[a, :] = (float)((sum over t < len[row0 + a] of (double)feat[row0 + a, t, :]) / len[row0 + a]) for a < n, summed in
+// token order with one fp64 accumulator per column (feat: [batch, S, H] fp32, len: device [batch])
+void launch_token_mean(const LaunchCtx& ctx, float* mean, const float* feat, const int* len, int row0, int n, int S, int H);
 }  // namespace sbv2

@@ -198,6 +198,40 @@ __global__ void gather_rows_kernel(float* out, const float* table, const int64_t
   for (int c = threadIdx.x; c < C; c += blockDim.x) out[(size_t)b * C + c] = table[(size_t)i * C + c];
 }
 
+// out[b, :] = table[idx[b], :] * c_row + mean[slot[b], :] * c_mean with coef[s] = (c_row, c_mean), rounded after each
+// product and after the sum (no FMA contraction: the host restatement reproduces it bit for bit); slot -1 copies the row.
+template <bool VEC>
+__global__ void gather_rows_blend_kernel(float* __restrict__ out, const float* __restrict__ table, const int64_t* __restrict__ idx,
+                                         const int* __restrict__ slot, const float* __restrict__ mean, const float2* __restrict__ coef,
+                                         int C, int n_rows, int n_slots) {
+  const int b = blockIdx.x;
+  int64_t i = idx[b];
+  if (i < 0) i = 0;
+  if (i >= n_rows) i = n_rows - 1;
+  const int s = slot[b];
+  const float* src = table + (size_t)i * C;
+  float* dst = out + (size_t)b * C;
+  if (s < 0 || s >= n_slots) {
+    if (VEC)
+      for (int c = threadIdx.x; c < C / 4; c += blockDim.x) reinterpret_cast<float4*>(dst)[c] = __ldg(reinterpret_cast<const float4*>(src) + c);
+    else
+      for (int c = threadIdx.x; c < C; c += blockDim.x) dst[c] = src[c];
+    return;
+  }
+  const float2 k = coef[s];
+  const float* m = mean + (size_t)s * C;
+  if (VEC) {
+    for (int c = threadIdx.x; c < C / 4; c += blockDim.x) {
+      const float4 x = __ldg(reinterpret_cast<const float4*>(src) + c), y = __ldg(reinterpret_cast<const float4*>(m) + c);
+      reinterpret_cast<float4*>(dst)[c] =
+          make_float4(__fadd_rn(__fmul_rn(x.x, k.x), __fmul_rn(y.x, k.y)), __fadd_rn(__fmul_rn(x.y, k.x), __fmul_rn(y.y, k.y)),
+                      __fadd_rn(__fmul_rn(x.z, k.x), __fmul_rn(y.z, k.y)), __fadd_rn(__fmul_rn(x.w, k.x), __fmul_rn(y.w, k.y)));
+    }
+  } else {
+    for (int c = threadIdx.x; c < C; c += blockDim.x) dst[c] = __fadd_rn(__fmul_rn(src[c], k.x), __fmul_rn(m[c], k.y));
+  }
+}
+
 __global__ void add_utt_vec_kernel(float* out, const float* x, const float* v, int C, int v_ld, Segs seg) {
   int b = blockIdx.y;
   int t = blockIdx.x;
@@ -853,6 +887,15 @@ void launch_embed_combine(const LaunchCtx& ctx, float* h, const int* x, const in
 void launch_gather_rows(const LaunchCtx& ctx, float* out, const float* table, const int64_t* idx, int n, int C, int n_rows) {
   if (n <= 0) return;
   gather_rows_kernel<<<n, 128, 0, ctx.stream>>>(out, table, idx, n, C, n_rows);
+  POST_LAUNCH(ctx);
+}
+
+void launch_gather_rows_blend(const LaunchCtx& ctx, float* out, const float* table, const int64_t* idx, const int* slot, const float* mean,
+                              const float2* coef, int n, int C, int n_rows, int n_slots) {
+  if (n <= 0) return;
+  const bool vec = C % 4 == 0 && ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(table) | reinterpret_cast<uintptr_t>(mean)) & 15) == 0;
+  if (vec) gather_rows_blend_kernel<true><<<n, 128, 0, ctx.stream>>>(out, table, idx, slot, mean, coef, C, n_rows, n_slots);
+  else gather_rows_blend_kernel<false><<<n, 128, 0, ctx.stream>>>(out, table, idx, slot, mean, coef, C, n_rows, n_slots);
   POST_LAUNCH(ctx);
 }
 

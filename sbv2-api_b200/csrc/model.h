@@ -101,7 +101,12 @@ struct DeviceBert {
   int64_t n_rows = 0;
   int hidden = 0;
   const int64_t* ph2tok = nullptr;  // host, [sum t_x]: BERT row (index into `rows`) of each phoneme of the batch
-  cudaEvent_t ready = nullptr;      // recorded on the producer's stream after the rows were written
+  cudaEvent_t ready = nullptr;      // recorded on the producer's stream after the rows (and `means`) were written
+  // assist texts (sbv2_synthesize_from_tokens_assist); n_slots == 0: plain gather
+  int n_slots = 0;
+  const float* means = nullptr;     // device [n_slots, hidden]: mean DeBERTa row of each assist
+  const int32_t* slot = nullptr;    // host [sum t_x]: assist slot of each phoneme, -1 = the plain row
+  const float* coef = nullptr;      // host [n_slots][2]: (c_row, c_mean) = ((float)(1 - (double)w), w)
 };
 sbv2_device_batch* synth_upload(sbv2_model* m, const sbv2_utterance* utts, int batch, const DeviceBert* dev_bert = nullptr);
 void synth_run(sbv2_model* m, sbv2_device_batch* b);
@@ -122,5 +127,8 @@ void bert_predict(sbv2_model* m, const int64_t* ids, const int64_t* mask, int ba
 // features stay on the device ([batch, s, hidden], zero rows where the mask is 0); null when no token is valid
 const float* bert_forward_device(sbv2_model* m, const int64_t* ids, const int64_t* mask, int batch, int64_t s);
 int bert_hidden(const sbv2_model* m);
+// launch_token_mean over rows [row0, row0 + n) of the last bert_forward_device output, on the model's stream; the result
+// [n, hidden] lives in a model-owned buffer that stays valid until the model's next call
+const float* bert_token_mean(sbv2_model* m, int row0, int n);
 
 }  // namespace sbv2

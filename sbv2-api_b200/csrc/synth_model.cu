@@ -200,6 +200,11 @@ struct sbv2_device_batch {
   const float* dev_bert_rows = nullptr;
   int64_t dev_bert_n = 0;
   cudaEvent_t dev_bert_ready = nullptr;
+  // assist-text blend of the gathered rows: per-phoneme slot (int32 [sum t_x]) and per-slot (c_row, c_mean) staged after
+  // ph2tok at these offsets; dev_bert_means == null: plain gather
+  const float* dev_bert_means = nullptr;
+  int dev_bert_slots = 0;
+  size_t o_slot = 0, o_coef = 0;
 };
 
 namespace sbv2 {
@@ -1007,6 +1012,13 @@ sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int 
     b->dev_bert_rows = dev_bert->rows;
     b->dev_bert_n = dev_bert->n_rows;
     b->dev_bert_ready = dev_bert->ready;
+    if (dev_bert->n_slots > 0) {
+      SBV2_REQUIRE(dev_bert->means && dev_bert->slot && dev_bert->coef && dev_bert->n_slots <= batch, "inconsistent assist-text blend");
+      for (int64_t t = 0; t < nx; ++t)
+        SBV2_REQUIRE(dev_bert->slot[t] >= -1 && dev_bert->slot[t] < dev_bert->n_slots, "assist slot out of range");
+      b->dev_bert_means = dev_bert->means;
+      b->dev_bert_slots = dev_bert->n_slots;
+    }
   }
 
   // blob layout
@@ -1078,9 +1090,17 @@ sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int 
   CUDA_CHECK(cudaMemcpyAsync(b->in.p, h, b->o_bert, cudaMemcpyHostToDevice, M->stream));
   CUDA_CHECK(cudaMemcpyAsync(b->in.as<uint8_t>() + b->o_nsdp, h + b->o_nsdp, size_t(nx) * 2 * 4, cudaMemcpyHostToDevice, M->stream));
   if (dev_bert) {
-    // the feature region only carries the phoneme -> token-row map
-    memcpy(hbert, dev_bert->ph2tok, size_t(nx) * 8);
-    CUDA_CHECK(cudaMemcpyAsync(b->in.as<uint8_t>() + b->o_bert, hbert, size_t(nx) * 8, cudaMemcpyHostToDevice, M->stream));
+    // the feature region only carries the phoneme -> token-row map (and the assist slots and coefficients)
+    size_t n_bytes = size_t(nx) * 8;
+    memcpy(hbert, dev_bert->ph2tok, n_bytes);
+    if (b->dev_bert_means) {
+      b->o_slot = b->o_bert + align_up(n_bytes, 16);
+      b->o_coef = b->o_slot + align_up(size_t(nx) * 4, 16);
+      n_bytes = b->o_coef - b->o_bert + size_t(b->dev_bert_slots) * 8;
+      memcpy(h + b->o_slot, dev_bert->slot, size_t(nx) * 4);
+      memcpy(h + b->o_coef, dev_bert->coef, size_t(b->dev_bert_slots) * 8);
+    }
+    CUDA_CHECK(cudaMemcpyAsync(b->in.as<uint8_t>() + b->o_bert, hbert, n_bytes, cudaMemcpyHostToDevice, M->stream));
   } else
   for (int i = 0; i < batch; ++i) {
     const size_t off_f = size_t(b->xstart[i]) * hp.bert_dim, cnt = size_t(b->xlen[i]) * hp.bert_dim * 4;
@@ -1334,11 +1354,18 @@ void synth_run(sbv2_model* mm, sbv2_device_batch* b) {
   if (b->dev_bert_rows) {
     // tts_util.rs:129-154 on the device: phoneme row i is the BERT row of its token (word2ph repeat), no transposes
     if (b->dev_bert_ready) CUDA_CHECK(cudaStreamWaitEvent(M.stream, b->dev_bert_ready, 0));
-    launch_gather_rows(ctx, bert, b->dev_bert_rows, reinterpret_cast<const int64_t*>(in + b->o_bert), int(Nx), hp.bert_dim,
-                       int(b->dev_bert_n));
+    if (b->dev_bert_means)
+      // assist texts (style_bert_vits2 extract_bert_feature): row * (1 - w) + mean(assist rows) * w
+      launch_gather_rows_blend(ctx, bert, b->dev_bert_rows, reinterpret_cast<const int64_t*>(in + b->o_bert),
+                               reinterpret_cast<const int*>(in + b->o_slot), b->dev_bert_means, reinterpret_cast<const float2*>(in + b->o_coef),
+                               int(Nx), hp.bert_dim, int(b->dev_bert_n), b->dev_bert_slots);
+    else
+      launch_gather_rows(ctx, bert, b->dev_bert_rows, reinterpret_cast<const int64_t*>(in + b->o_bert), int(Nx), hp.bert_dim,
+                         int(b->dev_bert_n));
   } else
     launch_cm_to_rm(ctx, reinterpret_cast<const float*>(in + b->o_bert), reinterpret_cast<const int64_t*>(in + b->o_bert_off),
                     nullptr, bert, hp.bert_dim, xseg);
+  M.debug["bert"] = DebugView{bert, Nx, hp.bert_dim, 4};
   F.conv(M.bert_proj, bert, hp.bert_dim, h, H, xseg);
   F.conv(M.style_proj, d_style, hp.style_dim, style_emb, H, bseg);
   launch_embed_combine(ctx, h, d_x, d_tone, d_lang, M.emb, M.tone_emb, M.lang_emb, style_emb, H, hp.n_vocab, hp.n_tones,

@@ -1,5 +1,7 @@
 #include "tts.hpp"
 
+#include <algorithm>
+#include <cmath>
 #include <cstring>
 
 namespace sbv2 {
@@ -139,6 +141,30 @@ Array2 expand_bert_features(const Array2& bert_content, const std::vector<int32_
   return out;
 }
 
+std::vector<float> assist_mean(const Array2& assist_content) {
+  if (assist_content.rows <= 0) throw Error(ErrorKind::ValueError, "assist text has no token");
+  const int64_t H = assist_content.cols;
+  std::vector<double> acc(size_t(H), 0.0);
+  for (int64_t t = 0; t < assist_content.rows; ++t)
+    for (int64_t c = 0; c < H; ++c) acc[size_t(c)] += double(assist_content.data[size_t(t * H + c)]);
+  std::vector<float> mean(static_cast<size_t>(H));
+  for (int64_t c = 0; c < H; ++c) mean[size_t(c)] = float(acc[size_t(c)] / double(assist_content.rows));
+  return mean;
+}
+
+Array2 expand_bert_features(const Array2& bert_content, const std::vector<int32_t>& word2ph, const std::vector<float>& mean,
+                            float weight) {
+  if (int64_t(mean.size()) != bert_content.cols) throw Error(ErrorKind::ValueError, "assist mean and BERT rows differ in width");
+  Array2 out = expand_bert_features(bert_content, word2ph);
+  const float c_row = float(1.0 - double(weight)), c_mean = weight;
+  for (int64_t c = 0; c < out.rows; ++c) {
+    const float m = mean[size_t(c)] * c_mean;
+    float* row = out.data.data() + size_t(c) * out.cols;
+    for (int64_t j = 0; j < out.cols; ++j) row[j] = row[j] * c_row + m;
+  }
+  return out;
+}
+
 std::vector<uint8_t> array_to_vec(const std::vector<float>& audio) {
   void* p = nullptr;
   size_t n = 0;
@@ -253,10 +279,42 @@ std::vector<float> TTSModelHolder::get_style_vector(const std::string& ident, in
   return out;
 }
 
+namespace {
+void check_assist(const AssistText& a) {
+  if (!std::isfinite(a.weight)) throw Error(ErrorKind::ValueError, "assist_text_weight must be finite");
+  if (a.token_ids.empty() || a.token_ids.size() > 32768 || a.attention_masks.size() != a.token_ids.size())
+    throw Error(ErrorKind::ValueError, "assist text must have 1 .. 32768 tokens and a mask of the same length");
+  for (int64_t m : a.attention_masks)
+    if (m == 0) throw Error(ErrorKind::ValueError, "attention_mask of an assist text must be all ones");
+}
+}  // namespace
+
 Array2 TTSModelHolder::bert_features(const std::vector<int64_t>& token_ids, const std::vector<int64_t>& attention_masks,
-                                     const std::vector<int32_t>& word2ph) {
-  Array2 content = bert::predict(bert_, token_ids, attention_masks);
-  return tts_util::expand_bert_features(content, word2ph);
+                                     const std::vector<int32_t>& word2ph, const AssistText* assist) {
+  if (assist) check_assist(*assist);
+  if (!assist || assist->weight == 0.0f) {
+    Array2 content = bert::predict(bert_, token_ids, attention_masks);
+    return tts_util::expand_bert_features(content, word2ph);
+  }
+  if (token_ids.size() != attention_masks.size()) throw Error(ErrorKind::OrtError, "input_ids and attention_mask differ in length");
+  int hidden = 0;
+  check(sbv2_bert_hidden_size(bert_.get(), &hidden));
+  const size_t t = token_ids.size(), ta = assist->token_ids.size(), s = std::max(t, ta);
+  std::vector<int64_t> ids(2 * s, 0), mask(2 * s, 0);
+  std::copy(token_ids.begin(), token_ids.end(), ids.begin());
+  std::copy(attention_masks.begin(), attention_masks.end(), mask.begin());
+  std::copy(assist->token_ids.begin(), assist->token_ids.end(), ids.begin() + long(s));
+  std::fill(mask.begin() + long(s), mask.begin() + long(s + ta), 1);
+  std::vector<float> feat(2 * s * size_t(hidden));
+  check(sbv2_bert_predict_batch(bert_.get(), ids.data(), mask.data(), 2, int64_t(s), feat.data()));
+  Array2 content, assist_content;
+  content.rows = int64_t(t);
+  content.cols = hidden;
+  content.data.assign(feat.begin(), feat.begin() + long(t * hidden));
+  assist_content.rows = int64_t(ta);
+  assist_content.cols = hidden;
+  assist_content.data.assign(feat.begin() + long(s * hidden), feat.begin() + long((s + ta) * hidden));
+  return tts_util::expand_bert_features(content, word2ph, tts_util::assist_mean(assist_content), assist->weight);
 }
 
 std::vector<uint8_t> TTSModelHolder::easy_synthesize(const std::string& ident, const std::vector<std::optional<ParsedText>>& lines,
@@ -361,10 +419,21 @@ std::vector<uint8_t> TTSModelHolder::easy_synthesize_tokens(const std::string& i
     pause.push_back(options.split_sentences && i != lines.size() - 1 ? 22050 : 0);
   }
   if (utts.empty()) throw Error(ErrorKind::NdArrayError, "NDArray error: nothing to concatenate");
+  sbv2_assist_text assist{};
+  std::vector<int32_t> assist_of;
+  if (options.assist) {
+    check_assist(*options.assist);
+    assist.input_ids = options.assist->token_ids.data();
+    assist.attention_mask = options.assist->attention_masks.data();
+    assist.t_tok = int64_t(options.assist->token_ids.size());
+    assist.weight = options.assist->weight;
+    assist_of.assign(utts.size(), 0);
+  }
   float* samples = nullptr;
   int64_t total = 0;
-  check(sbv2_synthesize_from_tokens_batch(m->vits2->get(), bert_.get(), utts.data(), int(utts.size()), pause.data(), &samples, &total,
-                                          nullptr));
+  check(sbv2_synthesize_from_tokens_assist(m->vits2->get(), bert_.get(), utts.data(), int(utts.size()), options.assist ? &assist : nullptr,
+                                           options.assist ? 1 : 0, options.assist ? assist_of.data() : nullptr, pause.data(), &samples,
+                                           &total, nullptr));
   void* wav = nullptr;
   size_t wav_n = 0;
   const int st = sbv2_wav_from_f32(samples, total, &wav, &wav_n);
@@ -506,15 +575,35 @@ int sbv2_holder_get_style_vector(sbv2_holder* h, const char* ident, int32_t styl
   });
 }
 
+namespace {
+// copies an assist text of the C ABI after the checks that make the copy safe (the rest: check_assist)
+std::optional<sbv2::host::AssistText> assist_from_c(const sbv2_assist_text* a) {
+  if (!a) return std::nullopt;
+  need(a->input_ids, "assist input_ids"), need(a->attention_mask, "assist attention_mask");
+  if (a->t_tok <= 0 || a->t_tok > 32768) throw sbv2::host::Error(sbv2::host::ErrorKind::ValueError, "assist text must have 1 .. 32768 tokens");
+  sbv2::host::AssistText t;
+  t.token_ids.assign(a->input_ids, a->input_ids + a->t_tok);
+  t.attention_masks.assign(a->attention_mask, a->attention_mask + a->t_tok);
+  t.weight = a->weight;
+  return t;
+}
+}  // namespace
+
 int sbv2_holder_bert_features(sbv2_holder* h, const int64_t* token_ids, const int64_t* attention_mask, int64_t t_tok,
                               const int32_t* word2ph, float** out, int64_t* t_x) {
+  return sbv2_holder_bert_features_assist(h, token_ids, attention_mask, t_tok, word2ph, nullptr, out, t_x);
+}
+
+int sbv2_holder_bert_features_assist(sbv2_holder* h, const int64_t* token_ids, const int64_t* attention_mask, int64_t t_tok,
+                                     const int32_t* word2ph, const sbv2_assist_text* assist, float** out, int64_t* t_x) {
   return holder_guard([&] {
     need(h, "holder"), need(token_ids, "token_ids"), need(attention_mask, "attention_mask"), need(word2ph, "word2ph"), need(out, "out"),
         need(t_x, "t_x");
     if (t_tok <= 0) throw sbv2::host::Error(sbv2::host::ErrorKind::ValueError, "t_tok must be positive");
     std::vector<int64_t> ids(token_ids, token_ids + t_tok), mask(attention_mask, attention_mask + t_tok);
     std::vector<int32_t> w(word2ph, word2ph + t_tok);
-    auto a = h->impl.bert_features(ids, mask, w);
+    const std::optional<sbv2::host::AssistText> at = assist_from_c(assist);
+    auto a = h->impl.bert_features(ids, mask, w, at ? &*at : nullptr);
     float* p = static_cast<float*>(sbv2_alloc(a.data.size() * 4 + 4));
     memcpy(p, a.data.data(), a.data.size() * 4);
     *out = p;
@@ -563,6 +652,14 @@ int sbv2_holder_easy_synthesize(sbv2_holder* h, const char* ident, const sbv2_se
 int sbv2_holder_easy_synthesize_tokens(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
                                        int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio, float length_scale,
                                        float style_weight, void** wav_bytes, size_t* wav_n) {
+  return sbv2_holder_easy_synthesize_tokens_assist(h, ident, sentences, n_sentences, total_lines, style_id, speaker_id, sdp_ratio,
+                                                   length_scale, style_weight, nullptr, wav_bytes, wav_n);
+}
+
+int sbv2_holder_easy_synthesize_tokens_assist(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
+                                              int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
+                                              float length_scale, float style_weight, const sbv2_assist_text* assist, void** wav_bytes,
+                                              size_t* wav_n) {
   return holder_guard([&] {
     using namespace sbv2::host;
     need(h, "holder"), need(ident, "ident"), need(wav_bytes, "wav_bytes"), need(wav_n, "wav_n");
@@ -587,6 +684,7 @@ int sbv2_holder_easy_synthesize_tokens(sbv2_holder* h, const char* ident, const 
     opt.length_scale = length_scale;
     opt.style_weight = style_weight;
     opt.split_sentences = true;
+    opt.assist = assist_from_c(assist);
     auto wav = h->impl.easy_synthesize_tokens(ident, lines, style_id, speaker_id, opt);
     void* p = sbv2_alloc(wav.size());
     memcpy(p, wav.data(), wav.size());

@@ -70,9 +70,23 @@ namespace bert {
 Array2 predict(Session& session, const std::vector<int64_t>& token_ids, const std::vector<int64_t>& attention_masks);
 }
 
+// Style-Bert-VITS2's assist text (assist_text / assist_text_weight): another text, normalised and tokenised like the main
+// text (CLS ... SEP), whose mean DeBERTa row is mixed into every phoneme feature with this weight.
+struct AssistText {
+  std::vector<int64_t> token_ids, attention_masks;
+  float weight = 0.0f;
+};
+
 namespace tts_util {
 // bert rows repeated word2ph[i] times, concatenated, transposed -> [hidden, sum(word2ph)]
 Array2 expand_bert_features(const Array2& bert_content, const std::vector<int32_t>& word2ph);
+// Host restatement of the device blend (include/sbv2_b200.h, sbv2_assist_text), bit for bit: the column means of an
+// assist's DeBERTa rows [n_a, hidden] with one fp64 accumulator per column summed in token order ...
+std::vector<float> assist_mean(const Array2& assist_content);
+// ... and the expansion with every row replaced by fl(fl(row * (float)(1 - (double)weight)) + fl(mean * weight)).
+// This file is compiled with -ffp-contract=off so that no fused multiply-add forms.
+Array2 expand_bert_features(const Array2& bert_content, const std::vector<int32_t>& word2ph, const std::vector<float>& mean,
+                            float weight);
 std::vector<uint8_t> array_to_vec(const std::vector<float>& audio);
 }  // namespace tts_util
 
@@ -81,6 +95,8 @@ struct SynthesizeOptions {
   float length_scale = 1.0f;
   float style_weight = 1.0f;
   bool split_sentences = true;
+  // applies to every line of the request (style_bert_vits2 TTSModel.infer passes it to each line); easy_synthesize_tokens only
+  std::optional<AssistText> assist;
 };
 
 // Output of the (out-of-scope) text frontend for one line of text.
@@ -114,9 +130,11 @@ class TTSModelHolder {
   void load(const std::string& ident, const std::vector<uint8_t>& style_vectors_bytes, const std::vector<uint8_t>& vits2_bytes);
   bool unload(const std::string& ident);
   std::vector<float> get_style_vector(const std::string& ident, int32_t style_id, float weight);
-  // device half of parse_text
+  // device half of parse_text.  With an assist text of non-zero weight DeBERTa runs once over [sentence, assist] (the
+  // layout of sbv2_synthesize_from_tokens_assist) and the blend is done on the host (tts_util::assist_mean and
+  // expand_bert_features); weight 0 is the plain path.
   Array2 bert_features(const std::vector<int64_t>& token_ids, const std::vector<int64_t>& attention_masks,
-                       const std::vector<int32_t>& word2ph);
+                       const std::vector<int32_t>& word2ph, const AssistText* assist = nullptr);
   // easy_synthesize over already-parsed lines. `lines[i]` empty optional == empty line (skipped, but
   // it still counts for the "not the last line" silence rule, tts.rs:293-320).
   std::vector<uint8_t> easy_synthesize(const std::string& ident, const std::vector<std::optional<ParsedText>>& lines, int32_t style_id,

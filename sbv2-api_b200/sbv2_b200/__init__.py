@@ -47,6 +47,11 @@ class TokenSentence(C.Structure):
                 ("lang_ids", C.POINTER(C.c_int64)), ("t_x", C.c_int64), ("line_index", C.c_int64)]
 
 
+class AssistText(C.Structure):
+    _fields_ = [("input_ids", C.POINTER(C.c_int64)), ("attention_mask", C.POINTER(C.c_int64)), ("t_tok", C.c_int64),
+                ("weight", C.c_float)]
+
+
 class Sentence(C.Structure):
     _fields_ = [("bert", C.POINTER(C.c_float)), ("phones", C.POINTER(C.c_int64)), ("tones", C.POINTER(C.c_int64)),
                 ("lang_ids", C.POINTER(C.c_int64)), ("t_x", C.c_int64), ("line_index", C.c_int64)]
@@ -80,6 +85,11 @@ def _load() -> C.CDLL:
         "sbv2_synthesize_from_tokens_batch": (C.c_int, [vp, vp, C.POINTER(TokenUtterance), C.c_int, pi64, C.POINTER(pf), pi64, pi64]),
         "sbv2_holder_easy_synthesize_tokens": (C.c_int, [vp, C.c_char_p, C.POINTER(TokenSentence), C.c_int, i64, i32, i64, f32, f32, f32,
                                                          C.POINTER(vp), C.POINTER(sz)]),
+        "sbv2_synthesize_from_tokens_assist": (C.c_int, [vp, vp, C.POINTER(TokenUtterance), C.c_int, C.POINTER(AssistText), C.c_int,
+                                                         pi32, pi64, C.POINTER(pf), pi64, pi64]),
+        "sbv2_holder_bert_features_assist": (C.c_int, [vp, pi64, pi64, i64, pi32, C.POINTER(AssistText), C.POINTER(pf), pi64]),
+        "sbv2_holder_easy_synthesize_tokens_assist": (C.c_int, [vp, C.c_char_p, C.POINTER(TokenSentence), C.c_int, i64, i32, i64, f32,
+                                                                f32, f32, C.POINTER(AssistText), C.POINTER(vp), C.POINTER(sz)]),
         "sbv2_onnx_bind_report": (C.c_int, [vp, sz, C.c_int, C.POINTER(vp)]),
         "sbv2_model_seed": (C.c_int, [vp, C.c_uint64]),
         "sbv2_synthesize_with_noise": (C.c_int, [vp, pf, pi64, pi64, pi64, i64, i64, pf, f32, f32, f32, f32, pf, pf, i64,
@@ -202,6 +212,18 @@ def _f32(a) -> np.ndarray:
 
 def _i64(a) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.int64)
+
+
+def _assist_texts(assists: Sequence[dict]):
+    """assists[k]: dict(token_ids, weight[, attention_mask]) -> (AssistText array, arrays it points into)"""
+    arr = (AssistText * max(len(assists), 1))()
+    keep = []
+    for k, a in enumerate(assists):
+        ids = _i64(a["token_ids"])
+        mask = _i64(a.get("attention_mask", np.ones_like(ids)))
+        keep += [ids, mask]
+        arr[k].input_ids, arr[k].attention_mask, arr[k].t_tok, arr[k].weight = _pi64(ids), _pi64(mask), ids.size, float(a["weight"])
+    return arr, keep
 
 
 class _Owned:
@@ -442,9 +464,12 @@ class Model:
                                                _pf(sv), sdp_ratio, length_scale, noise_scale, noise_scale_w, C.byref(p), C.byref(n)))
         return _take(p, n.value, np.float32)
 
-    def synthesize_from_tokens_batch(self, bert_model: "Model", sentences: Sequence[dict], pause_after: Optional[Sequence[int]] = None):
+    def synthesize_from_tokens_batch(self, bert_model: "Model", sentences: Sequence[dict], pause_after: Optional[Sequence[int]] = None,
+                                     assists: Optional[Sequence[dict]] = None):
         """sentences[i]: dict(token_ids, word2ph, x_tst, tones, lang_ids, style_vec[, sid, sdp_ratio, length_scale,
-        noise_scale, noise_scale_w]).  -> (audio [total] incl. the pauses, samples per sentence int64 [batch])"""
+        noise_scale, noise_scale_w, assist]).  -> (audio [total] incl. the pauses, samples per sentence int64 [batch])
+        assists: Style-Bert-VITS2 assist texts, dict(token_ids, weight[, attention_mask]) each; sentence i blends
+        assists[sentences[i]["assist"]] (no key or None: none).  assists=None calls sbv2_synthesize_from_tokens_batch."""
         B = len(sentences)
         arr = (TokenUtterance * B)()
         keep = []
@@ -462,8 +487,14 @@ class Model:
         pa = _i64(pause_after) if pause_after is not None else None
         p, total = C.POINTER(C.c_float)(), C.c_int64()
         ns = np.zeros(B, dtype=np.int64)
-        _check(lib.sbv2_synthesize_from_tokens_batch(self._h, bert_model._h, arr, B, _pi64(pa) if pa is not None else None, C.byref(p),
-                                                     C.byref(total), _pi64(ns)))
+        if assists is None:
+            _check(lib.sbv2_synthesize_from_tokens_batch(self._h, bert_model._h, arr, B, _pi64(pa) if pa is not None else None, C.byref(p),
+                                                         C.byref(total), _pi64(ns)))
+        else:
+            at, akeep = _assist_texts(assists)
+            of = np.array([-1 if u.get("assist") is None else int(u["assist"]) for u in sentences], dtype=np.int32)
+            _check(lib.sbv2_synthesize_from_tokens_assist(self._h, bert_model._h, arr, B, at, len(assists), of.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                          _pi64(pa) if pa is not None else None, C.byref(p), C.byref(total), _pi64(ns)))
         return _take(p, total.value, np.float32), ns
 
     def synthesize_with_noise(self, bert_ori, x_tst, sid: int, tones, lang_ids, style_vector, sdp_ratio, length_scale,
@@ -639,20 +670,28 @@ class TTSModelHolder:
         _check(lib.sbv2_holder_get_style_vector(self._h, ident.encode(), style_id, weight, _pf(out)))
         return out
 
-    def bert_features(self, token_ids, attention_masks, word2ph) -> np.ndarray:
+    def bert_features(self, token_ids, attention_masks, word2ph, assist: Optional[dict] = None) -> np.ndarray:
+        """assist: a Style-Bert-VITS2 assist text, dict(token_ids, weight[, attention_mask]), or None."""
         ids, mask = _i64(token_ids), _i64(attention_masks)
         w = np.ascontiguousarray(word2ph, dtype=np.int32)
         p, tx = C.POINTER(C.c_float)(), C.c_int64()
-        _check(lib.sbv2_holder_bert_features(self._h, _pi64(ids), _pi64(mask), ids.size,
-                                             w.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(p), C.byref(tx)))
+        if assist is None:
+            _check(lib.sbv2_holder_bert_features(self._h, _pi64(ids), _pi64(mask), ids.size,
+                                                 w.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(p), C.byref(tx)))
+        else:
+            at, akeep = _assist_texts([assist])
+            _check(lib.sbv2_holder_bert_features_assist(self._h, _pi64(ids), _pi64(mask), ids.size, w.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                        at, C.byref(p), C.byref(tx)))
         n = C.c_int64()  # rows = hidden size of the holder's DeBERTa: the library returns rows * t_x floats
         rows = self._bert_hidden
         return _take(p, rows * tx.value, np.float32).reshape(rows, tx.value)
 
     def easy_synthesize_tokens(self, ident: str, lines: Sequence[Optional[dict]], style_id: int, speaker_id: int,
-                               sdp_ratio: float = 0.0, length_scale: float = 1.0, style_weight: float = 1.0) -> bytes:
+                               sdp_ratio: float = 0.0, length_scale: float = 1.0, style_weight: float = 1.0,
+                               assist: Optional[dict] = None) -> bytes:
         """``lines[i]`` is None for an empty line, else dict(token_ids, word2ph, phones, tones, lang_ids): the request's
-        sentences run through DeBERTa and the synthesizer as one batch each, silences are written on the device."""
+        sentences run through DeBERTa and the synthesizer as one batch each, silences are written on the device.
+        ``assist``: a Style-Bert-VITS2 assist text, dict(token_ids, weight[, attention_mask]), applied to every line."""
         sent = [(i, l) for i, l in enumerate(lines) if l is not None]
         arr = (TokenSentence * max(len(sent), 1))()
         keep = []
@@ -665,8 +704,13 @@ class TTSModelHolder:
             a.token_ids, a.attention_mask, a.word2ph, a.t_tok = _pi64(ids), _pi64(mask), w2p.ctypes.data_as(C.POINTER(C.c_int32)), ids.size
             a.phones, a.tones, a.lang_ids, a.t_x, a.line_index = _pi64(ph), _pi64(t), _pi64(lg), ph.size, i
         p, n = C.c_void_p(), C.c_size_t()
-        _check(lib.sbv2_holder_easy_synthesize_tokens(self._h, ident.encode(), arr, len(sent), len(lines), style_id, speaker_id,
-                                                      sdp_ratio, length_scale, style_weight, C.byref(p), C.byref(n)))
+        if assist is None:
+            _check(lib.sbv2_holder_easy_synthesize_tokens(self._h, ident.encode(), arr, len(sent), len(lines), style_id, speaker_id,
+                                                          sdp_ratio, length_scale, style_weight, C.byref(p), C.byref(n)))
+        else:
+            at, akeep = _assist_texts([assist])
+            _check(lib.sbv2_holder_easy_synthesize_tokens_assist(self._h, ident.encode(), arr, len(sent), len(lines), style_id, speaker_id,
+                                                                 sdp_ratio, length_scale, style_weight, at, C.byref(p), C.byref(n)))
         out = C.string_at(p, n.value)
         lib.sbv2_free(p)
         return out
