@@ -200,6 +200,21 @@ int sbv2_synthesize_from_tokens_assist(sbv2_model* synth, sbv2_model* bert, cons
                                        const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of /* [batch] or NULL */,
                                        const int64_t* pause_after /* [batch] or NULL */, float** out_samples, int64_t* out_total,
                                        int64_t* out_n_samples /* [batch] or NULL */);
+/* Timing query of the token path (durations contract: see sbv2_predict_durations_batch below): DeBERTa, the text encoder
+ * and the duration predictors, over the same DeBERTa batch as sbv2_synthesize_from_tokens_assist.
+ * out_durations: int32 [sum t_x], caller-allocated. */
+int sbv2_predict_durations_from_tokens(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                       const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of /* [batch] or NULL */,
+                                       int32_t* out_durations);
+/* sbv2_synthesize_from_tokens_assist at given durations (durations[i] int32 [t_x] or NULL = predicted; durations NULL =
+ * all predicted).  Given durations do not change the DeBERTa batch, so the features are those of the plain call.
+ * out_durations (optional, caller-allocated int32 [sum t_x]) receives the durations used, given or predicted. */
+int sbv2_synthesize_from_tokens_with_durations(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                               const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of /* [batch] or NULL */,
+                                               const int64_t* pause_after /* [batch] or NULL */,
+                                               const int32_t* const* durations /* [batch] or NULL */,
+                                               int32_t* out_durations /* [sum t_x] or NULL */, float** out_samples, int64_t* out_total,
+                                               int64_t* out_n_samples /* [batch] or NULL */);
 
 /* Batched, variable-length extension.  Per-utterance pointer arrays of length `batch`; every
  * utterance's result is bit-identical to its own batch-1 call.  Results land in one pinned block:
@@ -222,6 +237,40 @@ typedef struct sbv2_utterance {
 int sbv2_synthesize_batch(sbv2_model* synth, const sbv2_utterance* utts, int batch, float** out_samples,
                           int64_t* out_n_samples, int32_t** out_durations /* [sum t_x] or NULL */,
                           int32_t** out_frame2ph /* [sum T_y] or NULL */);
+
+/* ---- phoneme durations: timing queries and synthesis at given durations ---------------------------------------------
+ *
+ * A duration is an integer number of latent frames; one frame is `hop` samples (the product of the decoder's upsample
+ * rates, "hop" in sbv2_model_describe: 512 for JP-Extra at 44.1 kHz).  Phoneme p of a sentence owns frames
+ * [cum(p-1), cum(p)) and samples [cum(p-1)·hop, cum(p)·hop) of that sentence's audio.
+ *
+ * Given durations d[0..t_x) of a sentence replace the duration predictors' ceil(w):
+ *   - the DP and SDP outputs are not used, so length_scale, sdp_ratio and noise_scale_w have no effect on that sentence;
+ *     noise_scale still scales the prior sample;
+ *   - T_y = max(1, sum d); all-zero durations give one frame synthesized from a zero prior mean and log-scale (frame2ph -1);
+ *   - every entry must lie in [0, 1 000 000] (the clamp applied to predicted durations); outside it, or when the call
+ *     would exceed 2^31 samples, or when explicit noise_zp has fewer than T_y frames, the call returns
+ *     SBV2_ERR_INVALID_ARGUMENT before anything runs on the device.
+ * Per sentence, durations are given or predicted (NULL entry of `durations`).  A sentence's result does not depend on
+ * which of the others are given: with explicit noise it is bit-identical to its own batch-1 call, and predicted
+ * sentences get the durations the plain call gives them.  When every sentence is given, the DP and SDP are not launched.
+ *
+ * Generator rule (internal noise): a timed call advances the model's counter-based generator exactly as the plain call
+ * with the same inputs would — it reserves the SDP noise range whenever the plain call draws it, even when it launches
+ * no SDP — and a timing query draws the SDP noise, advances by that range and draws no prior noise.  Hence
+ *   seed(s); D = query(...);  seed(s); timed(D)   ==   seed(s); plain(...)   bit for bit.
+ */
+
+/* Timing query of the features path: runs the text encoder and the duration predictors and stops after the durations
+ * (no flow, decoder or waveform).  out_durations: int32 [sum t_x], caller-allocated, utterances back to back; equal to
+ * the out_durations of sbv2_synthesize_batch on the same inputs.  noise_sdp is honoured; noise_zp is not used. */
+int sbv2_predict_durations_batch(sbv2_model* synth, const sbv2_utterance* utts, int batch, int32_t* out_durations);
+/* sbv2_synthesize_batch at given durations: durations[i] is int32 [t_x] for utterance i or NULL (predicted); durations
+ * itself may be NULL (all predicted, the plain call).  Outputs as sbv2_synthesize_batch. */
+int sbv2_synthesize_batch_with_durations(sbv2_model* synth, const sbv2_utterance* utts, int batch,
+                                         const int32_t* const* durations /* [batch] or NULL */, float** out_samples,
+                                         int64_t* out_n_samples, int32_t** out_durations /* [sum t_x] or NULL */,
+                                         int32_t** out_frame2ph /* [sum T_y] or NULL */);
 
 /* Device-resident variant used by the benchmark's kernel-only timing: inputs already uploaded with
  * sbv2_batch_upload; runs the whole synthesizer and leaves the waveforms on the device. */
@@ -343,6 +392,28 @@ int sbv2_holder_easy_synthesize_tokens_assist(sbv2_holder* h, const char* ident,
                                               int n_sentences, int64_t total_lines, int32_t style_id, int64_t speaker_id,
                                               float sdp_ratio, float length_scale, float style_weight,
                                               const sbv2_assist_text* assist, void** wav_bytes, size_t* wav_n);
+/* Timing of a request ("audio query"): the durations easy_synthesize_tokens_timed with durations = NULL would use, int32
+ * [sum t_x] caller-allocated, sentences concatenated in sentences[] order (durations contract: see
+ * sbv2_predict_durations_batch).  Runs DeBERTa, the text encoder and the duration predictors only.  Each line_index may
+ * appear once. */
+int sbv2_holder_predict_durations_tokens(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
+                                         int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
+                                         float length_scale, float style_weight, const sbv2_assist_text* assist,
+                                         int32_t* out_durations);
+/* sbv2_holder_easy_synthesize_tokens_assist at given durations and with the timing of the result.
+ *   durations: [n_sentences] in sentences[] order, each int32 [t_x] or NULL (predicted); NULL = all predicted, which
+ *     returns the same WAV bytes as sbv2_holder_easy_synthesize_tokens_assist.
+ *   out_durations (optional): int32 [sum t_x], the durations used, in sentences[] order.
+ *   out_phoneme_start (optional): int64 [sum t_x], in sentences[] order; entry p is the index, in the WAV's sample data,
+ *     of phoneme p's first sample.  It accounts for the earlier lines and the 22 050-sample pauses; the phoneme ends at
+ *     start + d·hop.  Character or token spans follow from these and word2ph.
+ * Each line_index may appear once. */
+int sbv2_holder_easy_synthesize_tokens_timed(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
+                                             int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
+                                             float length_scale, float style_weight, const sbv2_assist_text* assist,
+                                             const int32_t* const* durations /* [n_sentences] or NULL */,
+                                             int32_t* out_durations /* [sum t_x] or NULL */,
+                                             int64_t* out_phoneme_start /* [sum t_x] or NULL */, void** wav_bytes, size_t* wav_n);
 
 #ifdef __cplusplus
 }

@@ -15,6 +15,147 @@ const char* last_error_cstr();
 
 using namespace sbv2;
 
+namespace {
+
+// One implementation of the token path: sbv2_synthesize_from_tokens_assist (and through it _batch) and
+// sbv2_synthesize_from_tokens_with_durations synthesize, sbv2_predict_durations_from_tokens (query = true) stops after
+// the durations kernel and writes them to out_durations.
+void tokens_call(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch, const sbv2_assist_text* assists,
+                 int n_assists, const int32_t* assist_of, const int64_t* pause_after, const int32_t* const* durations, bool query,
+                 int32_t* out_durations, float** out_samples, int64_t* out_total, int64_t* out_n_samples) {
+  SBV2_REQUIRE(synth && bert && utts && (query ? out_durations != nullptr : out_samples && out_total), "null argument");
+  SBV2_REQUIRE(!synth->is_bert, "synthesize called on a BERT model");
+  SBV2_REQUIRE(bert->is_bert, "bert_predict called on a synthesizer model");
+  SBV2_REQUIRE(synth->device == bert->device, "the BERT and synthesizer models must live on the same device");
+  SBV2_REQUIRE(batch > 0, "empty batch");
+  SBV2_REQUIRE(n_assists >= 0 && (assists || n_assists == 0), "null assists with n_assists > 0");
+  if (!query) {
+    *out_samples = nullptr;
+    *out_total = 0;
+  }
+  for (int a = 0; a < n_assists; ++a) {
+    const sbv2_assist_text& x = assists[a];
+    SBV2_REQUIRE(x.input_ids && x.attention_mask, "null assist-text input");
+    SBV2_REQUIRE(x.t_tok > 0 && x.t_tok <= kMaxBertTokens, "assist text must have 1 .. 32768 tokens");
+    SBV2_REQUIRE(std::isfinite(x.weight), "assist_text_weight must be finite");
+    for (int64_t t = 0; t < x.t_tok; ++t)
+      SBV2_REQUIRE(x.attention_mask[t] != 0, "attention_mask of an assist text must be all ones (padding is added by the library)");
+  }
+  // DeBERTa batch: [sentences..., used assists...] right-padded to the longest row.  An assist is used when some
+  // sentence names it with a non-zero weight; used assists follow in index order and take slots 0, 1, ...
+  std::vector<char> named(size_t(n_assists), 0);
+  for (int i = 0; i < batch; ++i) {
+    const int a = assist_of ? assist_of[i] : -1;
+    SBV2_REQUIRE(a >= -1 && a < n_assists, "assist_of entry out of range");
+    if (a >= 0 && assists[a].weight != 0.f) named[size_t(a)] = 1;
+  }
+  std::vector<int> slot_of(size_t(n_assists), -1), used;
+  for (int a = 0; a < n_assists; ++a)
+    if (named[size_t(a)]) {
+      slot_of[size_t(a)] = int(used.size());
+      used.push_back(a);
+    }
+  const int rows_b = batch + int(used.size());
+  int64_t s_max = 0, nx = 0;
+  for (int i = 0; i < batch; ++i) {
+    SBV2_REQUIRE(utts[i].input_ids && utts[i].attention_mask && utts[i].word2ph && utts[i].t_tok > 0 && utts[i].t_x > 0, "empty input");
+    s_max = std::max(s_max, utts[i].t_tok);
+    nx += utts[i].t_x;
+  }
+  for (int a : used) s_max = std::max(s_max, assists[a].t_tok);
+  std::vector<int64_t> ids(size_t(rows_b) * s_max, 0), mask(size_t(rows_b) * s_max, 0), ph2tok;
+  std::vector<int32_t> ph_slot;
+  ph2tok.reserve(size_t(nx));
+  if (!used.empty()) ph_slot.reserve(size_t(nx));
+  for (int i = 0; i < batch; ++i) {
+    const sbv2_token_utterance& u = utts[i];
+    const int32_t slot = assist_of && assist_of[i] >= 0 ? slot_of[size_t(assist_of[i])] : -1;
+    int64_t n_ph = 0;
+    for (int64_t t = 0; t < u.t_tok; ++t) {
+      SBV2_REQUIRE(u.attention_mask[t] != 0, "attention_mask of a sentence must be all ones (padding is added by the library)");
+      ids[size_t(i) * s_max + t] = u.input_ids[t];
+      mask[size_t(i) * s_max + t] = 1;
+      SBV2_REQUIRE(u.word2ph[t] >= 0, "negative word2ph entry");
+      // tts_util.rs:129-154: token t is repeated word2ph[t] times
+      for (int32_t j = 0; j < u.word2ph[t]; ++j) ph2tok.push_back(int64_t(i) * s_max + t);
+      n_ph += u.word2ph[t];
+    }
+    SBV2_REQUIRE(n_ph == u.t_x, "sum(word2ph) must equal the number of phonemes");
+    if (!used.empty()) ph_slot.insert(ph_slot.end(), size_t(n_ph), slot);
+  }
+  std::vector<float> coef(used.size() * 2);
+  for (size_t k = 0; k < used.size(); ++k) {
+    const sbv2_assist_text& x = assists[used[k]];
+    for (int64_t t = 0; t < x.t_tok; ++t) {
+      ids[(size_t(batch) + k) * s_max + t] = x.input_ids[t];
+      mask[(size_t(batch) + k) * s_max + t] = 1;
+    }
+    coef[2 * k] = float(1.0 - double(x.weight));
+    coef[2 * k + 1] = x.weight;
+  }
+  std::vector<sbv2_utterance> su;
+  su.resize(size_t(batch));
+  for (int i = 0; i < batch; ++i) {
+    const sbv2_token_utterance& u = utts[i];
+    sbv2_utterance& o = su[size_t(i)];
+    o = sbv2_utterance{};
+    o.x_tst = u.x_tst;
+    o.tones = u.tones;
+    o.lang_ids = u.lang_ids;
+    o.t_x = u.t_x;
+    o.sid = u.sid;
+    o.style_vec = u.style_vec;
+    o.sdp_ratio = u.sdp_ratio;
+    o.length_scale = u.length_scale;
+    o.noise_scale = u.noise_scale;
+    o.noise_scale_w = u.noise_scale_w;
+  }
+  synth_check_durations(synth, su.data(), batch, durations);  // before DeBERTa launches anything
+  const float* rows = bert_forward_device(bert, ids.data(), mask.data(), rows_b, s_max);
+  SBV2_REQUIRE(rows != nullptr, "attention_mask selects no token");
+  DeviceBert dev;
+  if (!used.empty()) {
+    dev.n_slots = int(used.size());
+    dev.means = bert_token_mean(bert, batch, int(used.size()));
+    dev.slot = ph_slot.data();
+    dev.coef = coef.data();
+  }
+  cudaEvent_t ready = nullptr;
+  CUDA_CHECK(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
+  struct EventGuard {
+    cudaEvent_t e;
+    ~EventGuard() { cudaEventDestroy(e); }
+  } guard{ready};
+  CUDA_CHECK(cudaEventRecord(ready, bert->stream));
+  dev.rows = rows;
+  dev.n_rows = int64_t(rows_b) * s_max;
+  dev.hidden = bert_hidden(bert);
+  dev.ph2tok = ph2tok.data();
+  dev.ready = ready;
+  // given durations change nothing above: the DeBERTa batch and the gathered features are those of the plain call
+  std::unique_ptr<sbv2_device_batch, void (*)(sbv2_device_batch*)> b(synth_upload(synth, su.data(), batch, &dev, durations),
+                                                                     synth_batch_free);
+  if (query) {
+    synth_set_query(b.get());
+    synth_run(synth, b.get());
+    synth_query_durations(synth, b.get(), out_durations);  // synchronises: the BERT rows are free again
+    return;
+  }
+  if (pause_after) synth_set_pauses(b.get(), pause_after);
+  synth_run(synth, b.get());
+  std::vector<int64_t> n(size_t(batch), 0);
+  int32_t* dur = nullptr;
+  synth_download(synth, b.get(), out_samples, n.data(), out_durations ? &dur : nullptr, nullptr);  // synchronises: the BERT rows are free again
+  if (dur) {
+    memcpy(out_durations, dur, size_t(synth_batch_phonemes(b.get())) * 4);
+    free_out(dur);
+  }
+  *out_total = synth_wave_total(b.get());
+  if (out_n_samples) memcpy(out_n_samples, n.data(), size_t(batch) * 8);
+}
+
+}  // namespace
+
 extern "C" {
 
 const char* sbv2_last_error(void) { return last_error_cstr(); }
@@ -149,15 +290,32 @@ int sbv2_model_seed(sbv2_model* synth, uint64_t seed) {
 
 int sbv2_synthesize_batch(sbv2_model* synth, const sbv2_utterance* utts, int batch, float** out_samples, int64_t* out_n_samples,
                           int32_t** out_durations, int32_t** out_frame2ph) {
+  return sbv2_synthesize_batch_with_durations(synth, utts, batch, nullptr, out_samples, out_n_samples, out_durations, out_frame2ph);
+}
+
+int sbv2_synthesize_batch_with_durations(sbv2_model* synth, const sbv2_utterance* utts, int batch, const int32_t* const* durations,
+                                         float** out_samples, int64_t* out_n_samples, int32_t** out_durations, int32_t** out_frame2ph) {
   return guarded([&] {
     SBV2_REQUIRE(synth && out_samples && out_n_samples, "null argument");
     SBV2_REQUIRE(!synth->is_bert, "synthesize called on a BERT model");
     *out_samples = nullptr;
     if (out_durations) *out_durations = nullptr;
     if (out_frame2ph) *out_frame2ph = nullptr;
-    std::unique_ptr<sbv2_device_batch, void (*)(sbv2_device_batch*)> b(synth_upload(synth, utts, batch), synth_batch_free);
+    std::unique_ptr<sbv2_device_batch, void (*)(sbv2_device_batch*)> b(synth_upload(synth, utts, batch, nullptr, durations),
+                                                                       synth_batch_free);
     synth_run(synth, b.get());
     synth_download(synth, b.get(), out_samples, out_n_samples, out_durations, out_frame2ph);
+  });
+}
+
+int sbv2_predict_durations_batch(sbv2_model* synth, const sbv2_utterance* utts, int batch, int32_t* out_durations) {
+  return guarded([&] {
+    SBV2_REQUIRE(synth && out_durations, "null argument");
+    SBV2_REQUIRE(!synth->is_bert, "synthesize called on a BERT model");
+    std::unique_ptr<sbv2_device_batch, void (*)(sbv2_device_batch*)> b(synth_upload(synth, utts, batch), synth_batch_free);
+    synth_set_query(b.get());
+    synth_run(synth, b.get());
+    synth_query_durations(synth, b.get(), out_durations);
   });
 }
 
@@ -258,120 +416,24 @@ int sbv2_synthesize_from_tokens_batch(sbv2_model* synth, sbv2_model* bert, const
 int sbv2_synthesize_from_tokens_assist(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
                                        const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of,
                                        const int64_t* pause_after, float** out_samples, int64_t* out_total, int64_t* out_n_samples) {
+  return sbv2_synthesize_from_tokens_with_durations(synth, bert, utts, batch, assists, n_assists, assist_of, pause_after, nullptr, nullptr,
+                                                    out_samples, out_total, out_n_samples);
+}
+
+int sbv2_synthesize_from_tokens_with_durations(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                               const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of,
+                                               const int64_t* pause_after, const int32_t* const* durations, int32_t* out_durations,
+                                               float** out_samples, int64_t* out_total, int64_t* out_n_samples) {
   return guarded([&] {
-    SBV2_REQUIRE(synth && bert && utts && out_samples && out_total, "null argument");
-    SBV2_REQUIRE(!synth->is_bert, "synthesize called on a BERT model");
-    SBV2_REQUIRE(bert->is_bert, "bert_predict called on a synthesizer model");
-    SBV2_REQUIRE(synth->device == bert->device, "the BERT and synthesizer models must live on the same device");
-    SBV2_REQUIRE(batch > 0, "empty batch");
-    SBV2_REQUIRE(n_assists >= 0 && (assists || n_assists == 0), "null assists with n_assists > 0");
-    *out_samples = nullptr;
-    *out_total = 0;
-    for (int a = 0; a < n_assists; ++a) {
-      const sbv2_assist_text& x = assists[a];
-      SBV2_REQUIRE(x.input_ids && x.attention_mask, "null assist-text input");
-      SBV2_REQUIRE(x.t_tok > 0 && x.t_tok <= kMaxBertTokens, "assist text must have 1 .. 32768 tokens");
-      SBV2_REQUIRE(std::isfinite(x.weight), "assist_text_weight must be finite");
-      for (int64_t t = 0; t < x.t_tok; ++t)
-        SBV2_REQUIRE(x.attention_mask[t] != 0, "attention_mask of an assist text must be all ones (padding is added by the library)");
-    }
-    // DeBERTa batch: [sentences..., used assists...] right-padded to the longest row.  An assist is used when some
-    // sentence names it with a non-zero weight; used assists follow in index order and take slots 0, 1, ...
-    std::vector<char> named(size_t(n_assists), 0);
-    for (int i = 0; i < batch; ++i) {
-      const int a = assist_of ? assist_of[i] : -1;
-      SBV2_REQUIRE(a >= -1 && a < n_assists, "assist_of entry out of range");
-      if (a >= 0 && assists[a].weight != 0.f) named[size_t(a)] = 1;
-    }
-    std::vector<int> slot_of(size_t(n_assists), -1), used;
-    for (int a = 0; a < n_assists; ++a)
-      if (named[size_t(a)]) {
-        slot_of[size_t(a)] = int(used.size());
-        used.push_back(a);
-      }
-    const int rows_b = batch + int(used.size());
-    int64_t s_max = 0, nx = 0;
-    for (int i = 0; i < batch; ++i) {
-      SBV2_REQUIRE(utts[i].input_ids && utts[i].attention_mask && utts[i].word2ph && utts[i].t_tok > 0 && utts[i].t_x > 0, "empty input");
-      s_max = std::max(s_max, utts[i].t_tok);
-      nx += utts[i].t_x;
-    }
-    for (int a : used) s_max = std::max(s_max, assists[a].t_tok);
-    std::vector<int64_t> ids(size_t(rows_b) * s_max, 0), mask(size_t(rows_b) * s_max, 0), ph2tok;
-    std::vector<int32_t> ph_slot;
-    ph2tok.reserve(size_t(nx));
-    if (!used.empty()) ph_slot.reserve(size_t(nx));
-    for (int i = 0; i < batch; ++i) {
-      const sbv2_token_utterance& u = utts[i];
-      const int32_t slot = assist_of && assist_of[i] >= 0 ? slot_of[size_t(assist_of[i])] : -1;
-      int64_t n_ph = 0;
-      for (int64_t t = 0; t < u.t_tok; ++t) {
-        SBV2_REQUIRE(u.attention_mask[t] != 0, "attention_mask of a sentence must be all ones (padding is added by the library)");
-        ids[size_t(i) * s_max + t] = u.input_ids[t];
-        mask[size_t(i) * s_max + t] = 1;
-        SBV2_REQUIRE(u.word2ph[t] >= 0, "negative word2ph entry");
-        // tts_util.rs:129-154: token t is repeated word2ph[t] times
-        for (int32_t j = 0; j < u.word2ph[t]; ++j) ph2tok.push_back(int64_t(i) * s_max + t);
-        n_ph += u.word2ph[t];
-      }
-      SBV2_REQUIRE(n_ph == u.t_x, "sum(word2ph) must equal the number of phonemes");
-      if (!used.empty()) ph_slot.insert(ph_slot.end(), size_t(n_ph), slot);
-    }
-    std::vector<float> coef(used.size() * 2);
-    for (size_t k = 0; k < used.size(); ++k) {
-      const sbv2_assist_text& x = assists[used[k]];
-      for (int64_t t = 0; t < x.t_tok; ++t) {
-        ids[(size_t(batch) + k) * s_max + t] = x.input_ids[t];
-        mask[(size_t(batch) + k) * s_max + t] = 1;
-      }
-      coef[2 * k] = float(1.0 - double(x.weight));
-      coef[2 * k + 1] = x.weight;
-    }
-    const float* rows = bert_forward_device(bert, ids.data(), mask.data(), rows_b, s_max);
-    SBV2_REQUIRE(rows != nullptr, "attention_mask selects no token");
-    DeviceBert dev;
-    if (!used.empty()) {
-      dev.n_slots = int(used.size());
-      dev.means = bert_token_mean(bert, batch, int(used.size()));
-      dev.slot = ph_slot.data();
-      dev.coef = coef.data();
-    }
-    cudaEvent_t ready = nullptr;
-    CUDA_CHECK(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-    struct EventGuard {
-      cudaEvent_t e;
-      ~EventGuard() { cudaEventDestroy(e); }
-    } guard{ready};
-    CUDA_CHECK(cudaEventRecord(ready, bert->stream));
-    dev.rows = rows;
-    dev.n_rows = int64_t(rows_b) * s_max;
-    dev.hidden = bert_hidden(bert);
-    dev.ph2tok = ph2tok.data();
-    dev.ready = ready;
-    std::vector<sbv2_utterance> su;
-    su.resize(size_t(batch));
-    for (int i = 0; i < batch; ++i) {
-      const sbv2_token_utterance& u = utts[i];
-      sbv2_utterance& o = su[size_t(i)];
-      o = sbv2_utterance{};
-      o.x_tst = u.x_tst;
-      o.tones = u.tones;
-      o.lang_ids = u.lang_ids;
-      o.t_x = u.t_x;
-      o.sid = u.sid;
-      o.style_vec = u.style_vec;
-      o.sdp_ratio = u.sdp_ratio;
-      o.length_scale = u.length_scale;
-      o.noise_scale = u.noise_scale;
-      o.noise_scale_w = u.noise_scale_w;
-    }
-    std::unique_ptr<sbv2_device_batch, void (*)(sbv2_device_batch*)> b(synth_upload(synth, su.data(), batch, &dev), synth_batch_free);
-    if (pause_after) synth_set_pauses(b.get(), pause_after);
-    synth_run(synth, b.get());
-    std::vector<int64_t> n(size_t(batch), 0);
-    synth_download(synth, b.get(), out_samples, n.data(), nullptr, nullptr);  // synchronises: the BERT rows are free again
-    *out_total = synth_wave_total(b.get());
-    if (out_n_samples) memcpy(out_n_samples, n.data(), size_t(batch) * 8);
+    tokens_call(synth, bert, utts, batch, assists, n_assists, assist_of, pause_after, durations, false, out_durations, out_samples,
+                out_total, out_n_samples);
+  });
+}
+
+int sbv2_predict_durations_from_tokens(sbv2_model* synth, sbv2_model* bert, const sbv2_token_utterance* utts, int batch,
+                                       const sbv2_assist_text* assists, int n_assists, const int32_t* assist_of, int32_t* out_durations) {
+  return guarded([&] {
+    tokens_call(synth, bert, utts, batch, assists, n_assists, assist_of, nullptr, nullptr, true, out_durations, nullptr, nullptr, nullptr);
   });
 }
 

@@ -144,6 +144,12 @@ void launch_sdp_affine(const LaunchCtx& ctx, float* z, const float* m, const flo
 void launch_durations(const LaunchCtx& ctx, const float* logw_dp, const float* z_sdp /*[rows,2] or null*/,
                       const float* sdp_ratio_utt, const float* length_scale_utt, float* w_out, int* dur, int* cum,
                       int* ylen, const Segs& seg);
+// launch_durations with caller-given durations: utterance b takes given[start .. start + len) (int32, [0, 1e6]) when
+// given_flag[b] != 0 and the predicted durations otherwise (logw_dp may be null when every flag is set); same scan,
+// cum and ylen rules.  w_out of a given phoneme is its duration.
+void launch_durations_given(const LaunchCtx& ctx, const float* logw_dp, const float* z_sdp /*[rows,2] or null*/,
+                            const float* sdp_ratio_utt, const float* length_scale_utt, const int* given /*[rows]*/,
+                            const int* given_flag /*[B]*/, float* w_out, int* dur, int* cum, int* ylen, const Segs& seg);
 // frame2ph + gather + prior sample: z_p[j,c] = m_p[i,c] + eps[j,c]*exp(logs_p[i,c])*noise_scale[b]
 void launch_expand(const LaunchCtx& ctx, float* z_p, int* frame2ph, const float* stats /*[rows_x, 2C]: m_p | logs_p*/,
                    const int* cum, const float* eps_rm /*[rows_y, C]*/, const float* noise_scale_utt, int C,

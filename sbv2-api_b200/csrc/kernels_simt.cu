@@ -657,21 +657,30 @@ __global__ void sdp_affine_kernel(float* z, const float* m, const float* logs, i
 // ---------------------------------------------------------------------------------------------
 // length regulator
 // ---------------------------------------------------------------------------------------------
-__global__ void durations_kernel(const float* logw_dp, const float* z_sdp, const float* sdp_ratio, const float* length_scale,
-                                 float* w_out, int* dur, int* cum, int* ylen, Segs seg) {
+// kGiven: utterance b takes the caller's integers given[] when given_flag[b] != 0 (the DP / SDP outputs are not read
+// for it) and the predicted durations otherwise; both go through the same clamp, scan, cum and ylen rules.
+template <bool kGiven>
+__device__ __forceinline__ void durations_body(const float* logw_dp, const float* z_sdp, const float* sdp_ratio, const float* length_scale,
+                                               const int* given, const int* given_flag, float* w_out, int* dur, int* cum, int* ylen,
+                                               const Segs& seg) {
   // one warp per utterance: chunked inclusive scan
   int b = blockIdx.x;
   int lane = threadIdx.x;
   int len = seg.len[b];
   int base = seg.start[b];
   float ratio = sdp_ratio[b], ls = length_scale[b];
+  const bool use_given = kGiven && given_flag[b] != 0;
   // 64-bit total: 2^20 phonemes of up to 1e6 frames each exceed int32.  ylen saturates at INT_MAX, which the host
   // rejects as too long; whenever it accepts the batch, every prefix in cum fits in int32.
   long long carry = 0;
   for (int t0 = 0; t0 < len; t0 += 32) {
     int t = t0 + lane;
     int d = 0;
-    if (t < len) {
+    if (t < len && use_given) {
+      d = min(max(given[base + t], 0), 1000000);
+      if (w_out) w_out[base + t] = (float)d;
+      dur[base + t] = d;
+    } else if (t < len) {
       float dp = logw_dp[base + t];
       float logw;
       if (z_sdp) {
@@ -698,6 +707,16 @@ __global__ void durations_kernel(const float* logw_dp, const float* z_sdp, const
     carry += __shfl_sync(0xffffffffu, s, 31);  // one chunk: at most 32e6
   }
   if (lane == 0) ylen[b] = (int)min(max(carry, 1LL), (long long)INT_MAX);
+}
+
+__global__ void durations_kernel(const float* logw_dp, const float* z_sdp, const float* sdp_ratio, const float* length_scale,
+                                 float* w_out, int* dur, int* cum, int* ylen, Segs seg) {
+  durations_body<false>(logw_dp, z_sdp, sdp_ratio, length_scale, nullptr, nullptr, w_out, dur, cum, ylen, seg);
+}
+
+__global__ void durations_given_kernel(const float* logw_dp, const float* z_sdp, const float* sdp_ratio, const float* length_scale,
+                                       const int* given, const int* given_flag, float* w_out, int* dur, int* cum, int* ylen, Segs seg) {
+  durations_body<true>(logw_dp, z_sdp, sdp_ratio, length_scale, given, given_flag, w_out, dur, cum, ylen, seg);
 }
 
 __global__ void expand_kernel(float* z_p, int* frame2ph, const float* stats, const int* cum, const float* eps,
@@ -1044,6 +1063,15 @@ void launch_durations(const LaunchCtx& ctx, const float* logw_dp, const float* z
                       const float* length_scale_utt, float* w_out, int* dur, int* cum, int* ylen, const Segs& seg) {
   if (seg.n <= 0) return;
   durations_kernel<<<seg.n, 32, 0, ctx.stream>>>(logw_dp, z_sdp, sdp_ratio_utt, length_scale_utt, w_out, dur, cum, ylen, seg);
+  POST_LAUNCH(ctx);
+}
+
+void launch_durations_given(const LaunchCtx& ctx, const float* logw_dp, const float* z_sdp, const float* sdp_ratio_utt,
+                            const float* length_scale_utt, const int* given, const int* given_flag, float* w_out, int* dur, int* cum,
+                            int* ylen, const Segs& seg) {
+  if (seg.n <= 0) return;
+  durations_given_kernel<<<seg.n, 32, 0, ctx.stream>>>(logw_dp, z_sdp, sdp_ratio_utt, length_scale_utt, given, given_flag, w_out, dur,
+                                                       cum, ylen, seg);
   POST_LAUNCH(ctx);
 }
 

@@ -108,10 +108,21 @@ struct DeviceBert {
   const int32_t* slot = nullptr;    // host [sum t_x]: assist slot of each phoneme, -1 = the plain row
   const float* coef = nullptr;      // host [n_slots][2]: (c_row, c_mean) = ((float)(1 - (double)w), w)
 };
-sbv2_device_batch* synth_upload(sbv2_model* m, const sbv2_utterance* utts, int batch, const DeviceBert* dev_bert = nullptr);
+// durations (optional, [batch]): caller-given integer durations of utterance i ([t_x], each in [0, 1e6]) or null for the
+// predicted ones; they replace the DP / SDP outputs of that utterance (include/sbv2_b200.h, sbv2_synthesize_batch_with_durations)
+sbv2_device_batch* synth_upload(sbv2_model* m, const sbv2_utterance* utts, int batch, const DeviceBert* dev_bert = nullptr,
+                                const int32_t* const* durations = nullptr);
+// Host checks of given durations (synth_upload runs them too): each entry in [0, 1e6], the given utterances' samples
+// < 2^31, explicit noise_zp long enough.  Callers that launch work before synth_upload call it first.
+void synth_check_durations(sbv2_model* m, const sbv2_utterance* utts, int batch, const int32_t* const* durations);
 void synth_run(sbv2_model* m, sbv2_device_batch* b);
+// Timing query: synth_run on a batch marked here stops after the durations kernel (no expand, flow, decoder or waveform
+// buffer) and synth_query_durations copies the durations [sum t_x] into caller memory.
+void synth_set_query(sbv2_device_batch* b);
+void synth_query_durations(sbv2_model* m, sbv2_device_batch* b, int32_t* out);
 void synth_download(sbv2_model* m, sbv2_device_batch* b, float** out_samples, int64_t* out_n, int32_t** out_dur,
                     int32_t** out_f2p);
+int64_t synth_batch_phonemes(const sbv2_device_batch* b);                     // sum t_x
 int64_t synth_total_samples(sbv2_model* m, const sbv2_device_batch* b);
 int64_t synth_wave_total(const sbv2_device_batch* b);                        // samples of the output buffer incl. pauses
 void synth_set_pauses(sbv2_device_batch* b, const int64_t* pause_after);     // before synth_run: zeros after each utterance

@@ -180,6 +180,10 @@ struct sbv2_device_batch {
   std::vector<int> xlen, xstart, ylen, ystart;
   std::vector<int64_t> zp_frames;
   bool has_noise_sdp = false, has_noise_zp = false, any_sdp = false;
+  // caller-given durations: int32 [sum t_x] at o_given, int32 [B] flags (1 = given) at o_gflag; any_given == false
+  // leaves both regions empty and the batch on the plain durations kernel
+  bool any_given = false, all_given = false;
+  bool query = false;  // timing query: synth_run stops after the durations kernel
   BatchBuffers* bufs = nullptr;  // borrowed from / returned to the owner's pool
   sbv2_model* owner = nullptr;
   sbv2::DBuf &in, &zp, &ymeta, &wave, &dur, &cum, &f2p, &ylen_dev;
@@ -187,7 +191,7 @@ struct sbv2_device_batch {
       : bufs(b), owner(o), in(b->in), zp(b->zp), ymeta(b->ymeta), wave(b->wave), dur(b->dur), cum(b->cum), f2p(b->f2p), ylen_dev(b->ylen_dev) {}
   // offsets (bytes) into `in`
   size_t o_x = 0, o_tone = 0, o_lang = 0, o_sid = 0, o_sdp_ratio = 0, o_ls = 0, o_ns = 0, o_nsw = 0, o_xstart = 0, o_xlen = 0,
-         o_bert_off = 0, o_nsdp_off = 0, o_style = 0, o_bert = 0, o_nsdp = 0, o_zp_off = 0, o_zp_ld = 0;
+         o_bert_off = 0, o_nsdp_off = 0, o_given = 0, o_gflag = 0, o_style = 0, o_bert = 0, o_nsdp = 0, o_zp_off = 0, o_zp_ld = 0;
   bool ran = false;
   bool decode_only = false;
   bool borrowed_host = false;  // some H2D copies read the caller's (pinned) buffers directly: synchronise before returning to it
@@ -963,7 +967,34 @@ void synth_set_seed(sbv2_model* m, uint64_t seed) {
 // ---------------------------------------------------------------------------------------------
 // upload
 // ---------------------------------------------------------------------------------------------
-sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int batch, const DeviceBert* dev_bert) {
+void synth_check_durations(sbv2_model* mm, const sbv2_utterance* utts, int batch, const int32_t* const* durations) {
+  if (!durations) return;
+  const HParams& hp = static_cast<SynthModel*>(mm)->hp;
+  // the range is the clamp durations_kernel applies to predicted durations; the given utterances alone must already fit
+  // the 2^31-sample output and their explicit prior noise
+  int64_t given_samples = 0;
+  for (int i = 0; i < batch; ++i) {
+    const int32_t* d = durations[i];
+    if (!d) continue;
+    SBV2_REQUIRE(utts[i].t_x > 0, "t_x must be positive");
+    int64_t sum = 0;
+    for (int64_t t = 0; t < utts[i].t_x; ++t) {
+      if (d[t] < 0 || d[t] > 1000000)
+        fail(SBV2_ERR_INVALID_ARGUMENT, "duration " + std::to_string(d[t]) + " of phoneme " + std::to_string(t) + " of utterance " +
+                                            std::to_string(i) + " is outside [0, 1000000] frames");
+      sum += d[t];
+    }
+    const int64_t ty = std::max<int64_t>(sum, 1);
+    given_samples += ty * hp.hop;
+    if (given_samples > (int64_t(1) << 31) - 1) fail(SBV2_ERR_INVALID_ARGUMENT, "given durations too long: more than 2^31 samples in one call");
+    if (utts[i].noise_zp && utts[i].noise_zp_frames < ty)
+      fail(SBV2_ERR_INVALID_ARGUMENT, "noise_zp has " + std::to_string(utts[i].noise_zp_frames) + " frames but utterance " +
+                                          std::to_string(i) + " needs T_y = " + std::to_string(ty));
+  }
+}
+
+sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int batch, const DeviceBert* dev_bert,
+                                const int32_t* const* durations) {
   auto* M = static_cast<SynthModel*>(mm);
   SBV2_REQUIRE(!M->is_bert, "synthesize called on a BERT model");
   SBV2_REQUIRE(utts && batch > 0, "empty batch");
@@ -1005,6 +1036,13 @@ sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int 
   b->has_noise_sdp = n_nsdp > 0;
   b->has_noise_zp = n_nzp > 0;
   b->Nx = nx;
+  if (durations) {
+    synth_check_durations(M, utts, batch, durations);
+    int n_given = 0;
+    for (int i = 0; i < batch; ++i) n_given += durations[i] ? 1 : 0;
+    b->any_given = n_given > 0;
+    b->all_given = n_given == batch;
+  }
   if (dev_bert) {
     SBV2_REQUIRE(dev_bert->rows && dev_bert->ph2tok && dev_bert->hidden == hp.bert_dim, "BERT hidden size does not match the synthesizer");
     for (int64_t t = 0; t < nx; ++t)
@@ -1040,6 +1078,8 @@ sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int 
   b->o_xlen = take(batch * 4);
   b->o_bert_off = take(batch * 8);
   b->o_nsdp_off = take(batch * 8);
+  b->o_given = take(b->any_given ? size_t(nx) * 4 : 0);  // empty regions leave the plain layout unchanged
+  b->o_gflag = take(b->any_given ? size_t(batch) * 4 : 0);
   b->o_style = take(size_t(batch) * hp.style_dim * 4);
   b->o_bert = take(size_t(nx) * hp.bert_dim * 4);
   b->o_nsdp = take(size_t(nx) * 2 * 4);
@@ -1082,6 +1122,12 @@ sbv2_device_batch* synth_upload(sbv2_model* mm, const sbv2_utterance* utts, int 
     hnoff[i] = int64_t(s) * 2;
     memcpy(hstyle + size_t(i) * hp.style_dim, u.style_vec, size_t(hp.style_dim) * 4);
     if (u.noise_sdp) memcpy(hnsdp + size_t(s) * 2, u.noise_sdp, size_t(n) * 2 * 4);
+    if (b->any_given) {
+      int32_t* hgiven = reinterpret_cast<int32_t*>(h + b->o_given);
+      reinterpret_cast<int32_t*>(h + b->o_gflag)[i] = durations[i] ? 1 : 0;
+      if (durations[i]) memcpy(hgiven + s, durations[i], size_t(n) * 4);
+      else memset(hgiven + s, 0, size_t(n) * 4);
+    }
   }
   b->in.stream = M->stream;
   b->in.ensure(total);
@@ -1375,8 +1421,8 @@ void synth_run(sbv2_model* mm, sbv2_device_batch* b) {
   M.debug["enc_x"] = DebugView{h, Nx, H, 4};
   M.debug["stats"] = DebugView{stats, Nx, 2 * hp.inter, 4};
 
-  // ---- duration predictor -------------------------------------------------------------------
-  {
+  // ---- duration predictor (not run when every utterance brings its own durations) -----------
+  if (!b->all_given) {
     float* gc = M.ws[W_GG].as<float>();
     F.conv(M.dp_cond, g, hp.gin, gc, H, bseg);
     launch_add_utt_vec(ctx, dpx, h, gc, H, H, xseg);
@@ -1390,7 +1436,11 @@ void synth_run(sbv2_model* mm, sbv2_device_batch* b) {
 
   // ---- stochastic duration predictor (reverse) -----------------------------------------------
   float* zs = nullptr;
-  if (b->any_sdp) {
+  if (b->any_sdp && b->all_given) {
+    // no SDP to run, but the generator advances as the plain call's would: the z_p noise below then lands on the same
+    // counters, so given durations equal to the predicted ones give the plain call's audio bit for bit
+    if (!b->has_noise_sdp) M.rng_offset += uint64_t(Nx) * 2;
+  } else if (b->any_sdp) {
     float* sx = ens(W_SDPX, size_t(Nx) * H);
     float* sh = ens(W_SDPH, size_t(Nx) * H);
     float* t1 = ens(W_SDPT, size_t(Nx) * H * 2);
@@ -1431,9 +1481,17 @@ void synth_run(sbv2_model* mm, sbv2_device_batch* b) {
   b->dur.stream = b->cum.stream = M.stream;
   b->dur.ensure(size_t(Nx) * 4);
   b->cum.ensure(size_t(Nx) * 4);
-  launch_durations(ctx, logw, zs, d_ratio, d_ls, wbuf, b->dur.as<int>(), b->cum.as<int>(), d_ylen, xseg);
+  if (b->any_given)
+    launch_durations_given(ctx, b->all_given ? nullptr : logw, zs, d_ratio, d_ls, reinterpret_cast<const int*>(in + b->o_given),
+                           reinterpret_cast<const int*>(in + b->o_gflag), wbuf, b->dur.as<int>(), b->cum.as<int>(), d_ylen, xseg);
+  else
+    launch_durations(ctx, logw, zs, d_ratio, d_ls, wbuf, b->dur.as<int>(), b->cum.as<int>(), d_ylen, xseg);
   M.debug["w"] = DebugView{wbuf, Nx, 1, 4};
   M.region_end("text");
+  if (b->query) {
+    b->ran = true;
+    return;
+  }
   M.pin_ylen.ensure(size_t(B) * 4);
   CUDA_CHECK(cudaMemcpyAsync(M.pin_ylen.p, d_ylen, size_t(B) * 4, cudaMemcpyDeviceToHost, M.stream));
   M.wait_stream(/*yield=*/B >= 8);
@@ -1713,6 +1771,17 @@ void synth_run(sbv2_model* mm, sbv2_device_batch* b) {
   b->ran = true;
 }
 
+void synth_set_query(sbv2_device_batch* b) { b->query = true; }
+
+void synth_query_durations(sbv2_model* mm, sbv2_device_batch* b, int32_t* out) {
+  auto* M = static_cast<SynthModel*>(mm);
+  SBV2_REQUIRE(b->ran && b->query, "timing query has not been run");
+  M->bind_device();
+  CUDA_CHECK(cudaMemcpyAsync(out, b->dur.p, size_t(b->Nx) * 4, cudaMemcpyDeviceToHost, M->stream));
+  M->wait_stream(/*yield=*/b->B >= 8);
+}
+
+int64_t synth_batch_phonemes(const sbv2_device_batch* b) { return b->Nx; }
 int64_t synth_total_samples(sbv2_model* m, const sbv2_device_batch* b) { return b->Ny * static_cast<SynthModel*>(m)->hp.hop; }
 int64_t synth_wave_total(const sbv2_device_batch* b) { return b->wave_total; }
 void synth_set_pauses(sbv2_device_batch* b, const int64_t* pause_after) {

@@ -380,17 +380,28 @@ std::vector<uint8_t> TTSModelHolder::easy_synthesize(const std::string& ident, c
   return tts_util::array_to_vec(audio);
 }
 
-std::vector<uint8_t> TTSModelHolder::easy_synthesize_tokens(const std::string& ident,
-                                                            const std::vector<std::optional<ParsedTokens>>& lines, int32_t style_id,
-                                                            int64_t speaker_id, const SynthesizeOptions& options) {
+struct TokenBatch {
+  std::vector<float> style_vector;
+  std::vector<sbv2_token_utterance> utts;  // the non-empty lines in line order
+  std::vector<int64_t> pause;
+  sbv2_assist_text assist{};
+  std::vector<int32_t> assist_of;
+  std::vector<const int32_t*> durations;  // [utts] or empty: all predicted
+  int64_t n_phonemes = 0;
+  const sbv2_assist_text* assist_ptr() const { return assist_of.empty() ? nullptr : &assist; }
+  const int32_t* assist_of_ptr() const { return assist_of.empty() ? nullptr : assist_of.data(); }
+};
+
+sbv2_model* TTSModelHolder::token_batch(const std::string& ident, const std::vector<std::optional<ParsedTokens>>& lines,
+                                        int32_t style_id, int64_t speaker_id, const SynthesizeOptions& options, TokenBatch& out) {
   find_and_load_model(ident);
-  std::vector<float> style_vector = get_style_vector(ident, style_id, options.style_weight);
+  out.style_vector = get_style_vector(ident, style_id, options.style_weight);
   TTSModel* m = find_model(ident);
   if (!m || !m->vits2) throw Error(ErrorKind::ModelNotFoundError, "model not found error: " + ident);
   if (!options.split_sentences && (lines.size() != 1 || !lines[0]))
     throw Error(ErrorKind::ValueError, "split_sentences=false expects exactly one parsed text");
-  std::vector<sbv2_token_utterance> utts;
-  std::vector<int64_t> pause;
+  if (!options.durations.empty() && options.durations.size() != lines.size())
+    throw Error(ErrorKind::ValueError, "durations must have one entry per line of the request");
   for (size_t i = 0; i < lines.size(); ++i) {
     if (!lines[i]) continue;  // empty line (tts.rs:293-295)
     const ParsedTokens& t = *lines[i];
@@ -409,31 +420,63 @@ std::vector<uint8_t> TTSModelHolder::easy_synthesize_tokens(const std::string& i
     u.lang_ids = t.lang_ids.data();
     u.t_x = t_x;
     u.sid = speaker_id;
-    u.style_vec = style_vector.data();
+    u.style_vec = out.style_vector.data();
     u.sdp_ratio = options.sdp_ratio;
     u.length_scale = options.length_scale;
     u.noise_scale = 0.677f;
     u.noise_scale_w = 0.8f;
-    utts.push_back(u);
+    out.utts.push_back(u);
+    out.n_phonemes += t_x;
     // tts.rs:318-320: half a second of silence after every line but the last one of the text
-    pause.push_back(options.split_sentences && i != lines.size() - 1 ? 22050 : 0);
+    out.pause.push_back(options.split_sentences && i != lines.size() - 1 ? 22050 : 0);
+    if (!options.durations.empty()) {
+      const auto& d = options.durations[i];
+      if (d && int64_t(d->size()) != t_x) throw Error(ErrorKind::ValueError, "durations of a line must have one entry per phoneme");
+      out.durations.push_back(d ? d->data() : nullptr);
+    }
   }
-  if (utts.empty()) throw Error(ErrorKind::NdArrayError, "NDArray error: nothing to concatenate");
-  sbv2_assist_text assist{};
-  std::vector<int32_t> assist_of;
+  if (out.utts.empty()) throw Error(ErrorKind::NdArrayError, "NDArray error: nothing to concatenate");
   if (options.assist) {
     check_assist(*options.assist);
-    assist.input_ids = options.assist->token_ids.data();
-    assist.attention_mask = options.assist->attention_masks.data();
-    assist.t_tok = int64_t(options.assist->token_ids.size());
-    assist.weight = options.assist->weight;
-    assist_of.assign(utts.size(), 0);
+    out.assist.input_ids = options.assist->token_ids.data();
+    out.assist.attention_mask = options.assist->attention_masks.data();
+    out.assist.t_tok = int64_t(options.assist->token_ids.size());
+    out.assist.weight = options.assist->weight;
+    out.assist_of.assign(out.utts.size(), 0);
   }
+  return m->vits2->get();
+}
+
+std::vector<uint8_t> TTSModelHolder::easy_synthesize_tokens(const std::string& ident,
+                                                            const std::vector<std::optional<ParsedTokens>>& lines, int32_t style_id,
+                                                            int64_t speaker_id, const SynthesizeOptions& options, TokenTiming* timing) {
+  TokenBatch tb;
+  sbv2_model* synth = token_batch(ident, lines, style_id, speaker_id, options, tb);
+  const size_t B = tb.utts.size();
+  std::vector<int32_t> dur(timing ? size_t(tb.n_phonemes) : 0);
+  std::vector<int64_t> n(B, 0);
   float* samples = nullptr;
   int64_t total = 0;
-  check(sbv2_synthesize_from_tokens_assist(m->vits2->get(), bert_.get(), utts.data(), int(utts.size()), options.assist ? &assist : nullptr,
-                                           options.assist ? 1 : 0, options.assist ? assist_of.data() : nullptr, pause.data(), &samples,
-                                           &total, nullptr));
+  check(sbv2_synthesize_from_tokens_with_durations(synth, bert_.get(), tb.utts.data(), int(B), tb.assist_ptr(), tb.assist_of.empty() ? 0 : 1,
+                                                   tb.assist_of_ptr(), tb.pause.data(), tb.durations.empty() ? nullptr : tb.durations.data(),
+                                                   timing ? dur.data() : nullptr, &samples, &total, n.data()));
+  if (timing) {
+    // sentence k starts after the samples and pauses of the sentences before it; hop = samples / T_y, T_y = max(1, sum d)
+    timing->phoneme_start.assign(size_t(tb.n_phonemes), 0);
+    int64_t start = 0, p = 0;
+    for (size_t k = 0; k < B; ++k) {
+      int64_t ty = 0;
+      for (int64_t t = 0; t < tb.utts[k].t_x; ++t) ty += dur[size_t(p + t)];
+      const int64_t hop = n[k] / std::max<int64_t>(ty, 1);
+      int64_t cum = 0;
+      for (int64_t t = 0; t < tb.utts[k].t_x; ++t, ++p) {
+        timing->phoneme_start[size_t(p)] = start + cum * hop;
+        cum += dur[size_t(p)];
+      }
+      start += n[k] + tb.pause[k];
+    }
+    timing->durations = std::move(dur);
+  }
   void* wav = nullptr;
   size_t wav_n = 0;
   const int st = sbv2_wav_from_f32(samples, total, &wav, &wav_n);
@@ -442,6 +485,17 @@ std::vector<uint8_t> TTSModelHolder::easy_synthesize_tokens(const std::string& i
   std::vector<uint8_t> out(static_cast<uint8_t*>(wav), static_cast<uint8_t*>(wav) + wav_n);
   sbv2_free(wav);
   return out;
+}
+
+std::vector<int32_t> TTSModelHolder::predict_durations_tokens(const std::string& ident,
+                                                              const std::vector<std::optional<ParsedTokens>>& lines, int32_t style_id,
+                                                              int64_t speaker_id, const SynthesizeOptions& options) {
+  TokenBatch tb;
+  sbv2_model* synth = token_batch(ident, lines, style_id, speaker_id, options, tb);
+  std::vector<int32_t> dur(size_t(tb.n_phonemes));
+  check(sbv2_predict_durations_from_tokens(synth, bert_.get(), tb.utts.data(), int(tb.utts.size()), tb.assist_ptr(),
+                                           tb.assist_of.empty() ? 0 : 1, tb.assist_of_ptr(), dur.data()));
+  return dur;
 }
 
 }  // namespace host
@@ -660,32 +714,108 @@ int sbv2_holder_easy_synthesize_tokens_assist(sbv2_holder* h, const char* ident,
                                               int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
                                               float length_scale, float style_weight, const sbv2_assist_text* assist, void** wav_bytes,
                                               size_t* wav_n) {
+  return sbv2_holder_easy_synthesize_tokens_timed(h, ident, sentences, n_sentences, total_lines, style_id, speaker_id, sdp_ratio,
+                                                  length_scale, style_weight, assist, nullptr, nullptr, nullptr, wav_bytes, wav_n);
+}
+
+namespace {
+// sentences of the C ABI -> one entry per line of the request (empty optional = empty line); `unique` rejects a
+// line_index named twice (the timing arrays have one slot per sentence)
+std::vector<std::optional<sbv2::host::ParsedTokens>> token_lines(const sbv2_token_sentence* sentences, int n_sentences, int64_t total_lines,
+                                                                 bool unique) {
+  using namespace sbv2::host;
+  if (n_sentences > 0) need(sentences, "sentences");
+  std::vector<std::optional<ParsedTokens>> lines(size_t(total_lines > 0 ? total_lines : 0));
+  for (int i = 0; i < n_sentences; ++i) {
+    const sbv2_token_sentence& s = sentences[i];
+    if (s.line_index < 0 || s.line_index >= total_lines) throw Error(ErrorKind::ValueError, "line_index out of range");
+    if (!s.token_ids || !s.attention_mask || !s.word2ph || !s.phones || !s.tones || !s.lang_ids || s.t_tok <= 0 || s.t_x <= 0)
+      throw Error(ErrorKind::ValueError, "sentence with null or empty input");
+    if (unique && lines[size_t(s.line_index)]) throw Error(ErrorKind::ValueError, "two sentences name the same line_index");
+    ParsedTokens t;
+    t.token_ids.assign(s.token_ids, s.token_ids + s.t_tok);
+    t.attention_masks.assign(s.attention_mask, s.attention_mask + s.t_tok);
+    t.word2ph.assign(s.word2ph, s.word2ph + s.t_tok);
+    t.phones.assign(s.phones, s.phones + s.t_x);
+    t.tones.assign(s.tones, s.tones + s.t_x);
+    t.lang_ids.assign(s.lang_ids, s.lang_ids + s.t_x);
+    lines[size_t(s.line_index)] = std::move(t);
+  }
+  return lines;
+}
+
+sbv2::host::SynthesizeOptions token_options(float sdp_ratio, float length_scale, float style_weight, const sbv2_assist_text* assist) {
+  sbv2::host::SynthesizeOptions opt;
+  opt.sdp_ratio = sdp_ratio;
+  opt.length_scale = length_scale;
+  opt.style_weight = style_weight;
+  opt.split_sentences = true;
+  opt.assist = assist_from_c(assist);
+  return opt;
+}
+
+// first phoneme of each sentence (sentences[] order) in the line-order concatenation the holder returns
+std::vector<int64_t> line_order_offsets(const sbv2_token_sentence* sentences, int n_sentences) {
+  std::vector<int> order(static_cast<size_t>(n_sentences));
+  for (int i = 0; i < n_sentences; ++i) order[size_t(i)] = i;
+  std::sort(order.begin(), order.end(), [&](int a, int b) { return sentences[a].line_index < sentences[b].line_index; });
+  std::vector<int64_t> off(static_cast<size_t>(n_sentences), 0);
+  int64_t o = 0;
+  for (int k : order) {
+    off[size_t(k)] = o;
+    o += sentences[k].t_x;
+  }
+  return off;
+}
+}  // namespace
+
+int sbv2_holder_predict_durations_tokens(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
+                                         int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
+                                         float length_scale, float style_weight, const sbv2_assist_text* assist,
+                                         int32_t* out_durations) {
+  return holder_guard([&] {
+    need(h, "holder"), need(ident, "ident"), need(out_durations, "out_durations");
+    auto lines = token_lines(sentences, n_sentences, total_lines, true);
+    const std::vector<int32_t> d = h->impl.predict_durations_tokens(ident, lines, style_id, speaker_id,
+                                                                    token_options(sdp_ratio, length_scale, style_weight, assist));
+    const std::vector<int64_t> off = line_order_offsets(sentences, n_sentences);
+    int64_t o = 0;
+    for (int i = 0; i < n_sentences; ++i) {
+      std::copy(d.begin() + off[size_t(i)], d.begin() + off[size_t(i)] + sentences[i].t_x, out_durations + o);
+      o += sentences[i].t_x;
+    }
+  });
+}
+
+int sbv2_holder_easy_synthesize_tokens_timed(sbv2_holder* h, const char* ident, const sbv2_token_sentence* sentences, int n_sentences,
+                                             int64_t total_lines, int32_t style_id, int64_t speaker_id, float sdp_ratio,
+                                             float length_scale, float style_weight, const sbv2_assist_text* assist,
+                                             const int32_t* const* durations, int32_t* out_durations, int64_t* out_phoneme_start,
+                                             void** wav_bytes, size_t* wav_n) {
   return holder_guard([&] {
     using namespace sbv2::host;
     need(h, "holder"), need(ident, "ident"), need(wav_bytes, "wav_bytes"), need(wav_n, "wav_n");
-    if (n_sentences > 0) need(sentences, "sentences");
-    std::vector<std::optional<ParsedTokens>> lines(size_t(total_lines > 0 ? total_lines : 0));
-    for (int i = 0; i < n_sentences; ++i) {
-      const sbv2_token_sentence& s = sentences[i];
-      if (s.line_index < 0 || s.line_index >= total_lines) throw Error(ErrorKind::ValueError, "line_index out of range");
-      if (!s.token_ids || !s.attention_mask || !s.word2ph || !s.phones || !s.tones || !s.lang_ids || s.t_tok <= 0 || s.t_x <= 0)
-        throw Error(ErrorKind::ValueError, "sentence with null or empty input");
-      ParsedTokens t;
-      t.token_ids.assign(s.token_ids, s.token_ids + s.t_tok);
-      t.attention_masks.assign(s.attention_mask, s.attention_mask + s.t_tok);
-      t.word2ph.assign(s.word2ph, s.word2ph + s.t_tok);
-      t.phones.assign(s.phones, s.phones + s.t_x);
-      t.tones.assign(s.tones, s.tones + s.t_x);
-      t.lang_ids.assign(s.lang_ids, s.lang_ids + s.t_x);
-      lines[size_t(s.line_index)] = std::move(t);
+    const bool timed = durations || out_durations || out_phoneme_start;
+    auto lines = token_lines(sentences, n_sentences, total_lines, timed);
+    SynthesizeOptions opt = token_options(sdp_ratio, length_scale, style_weight, assist);
+    if (durations) {
+      opt.durations.resize(lines.size());
+      for (int i = 0; i < n_sentences; ++i)
+        if (durations[i]) opt.durations[size_t(sentences[i].line_index)].emplace(durations[i], durations[i] + sentences[i].t_x);
     }
-    SynthesizeOptions opt;
-    opt.sdp_ratio = sdp_ratio;
-    opt.length_scale = length_scale;
-    opt.style_weight = style_weight;
-    opt.split_sentences = true;
-    opt.assist = assist_from_c(assist);
-    auto wav = h->impl.easy_synthesize_tokens(ident, lines, style_id, speaker_id, opt);
+    TokenTiming timing;
+    auto wav = h->impl.easy_synthesize_tokens(ident, lines, style_id, speaker_id, opt, timed ? &timing : nullptr);
+    if (timed) {
+      const std::vector<int64_t> off = line_order_offsets(sentences, n_sentences);
+      int64_t o = 0;
+      for (int i = 0; i < n_sentences; ++i) {
+        const size_t a = size_t(off[size_t(i)]), n = size_t(sentences[i].t_x);
+        if (out_durations) std::copy(timing.durations.begin() + long(a), timing.durations.begin() + long(a + n), out_durations + o);
+        if (out_phoneme_start)
+          std::copy(timing.phoneme_start.begin() + long(a), timing.phoneme_start.begin() + long(a + n), out_phoneme_start + o);
+        o += int64_t(n);
+      }
+    }
     void* p = sbv2_alloc(wav.size());
     memcpy(p, wav.data(), wav.size());
     *wav_bytes = p;

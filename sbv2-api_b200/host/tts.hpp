@@ -97,7 +97,17 @@ struct SynthesizeOptions {
   bool split_sentences = true;
   // applies to every line of the request (style_bert_vits2 TTSModel.infer passes it to each line); easy_synthesize_tokens only
   std::optional<AssistText> assist;
+  // given phoneme durations in latent frames, per line of the request (include/sbv2_b200.h states the contract): empty =
+  // all predicted, an empty optional = that line predicted; easy_synthesize_tokens only
+  std::vector<std::optional<std::vector<int32_t>>> durations;
 };
+
+// Where the phonemes of a request land (easy_synthesize_tokens): both [sum t_x] over the non-empty lines in line order.
+struct TokenTiming {
+  std::vector<int32_t> durations;      // frames per phoneme, given or predicted
+  std::vector<int64_t> phoneme_start;  // index of the phoneme's first sample in the WAV's sample data (ends at start + d * hop)
+};
+struct TokenBatch;  // one request's sentences as the C ABI takes them (tts.cpp)
 
 // Output of the (out-of-scope) text frontend for one line of text.
 struct ParsedText {
@@ -142,14 +152,22 @@ class TTSModelHolder {
   // easy_synthesize with bert::predict folded in: every non-empty line of the request goes through DeBERTa as ONE
   // right-padded batch and through the synthesizer as ONE batch (features never leave the device), the 22 050-sample
   // pauses of tts.rs:318-320 are written on the device, and the WAV is one header + one copy of the pinned result.
+  // timing (optional) receives the durations used and where each phoneme starts in the WAV.
   std::vector<uint8_t> easy_synthesize_tokens(const std::string& ident, const std::vector<std::optional<ParsedTokens>>& lines,
-                                              int32_t style_id, int64_t speaker_id, const SynthesizeOptions& options);
+                                              int32_t style_id, int64_t speaker_id, const SynthesizeOptions& options,
+                                              TokenTiming* timing = nullptr);
+  // "audio query": the durations easy_synthesize_tokens would use without given durations ([sum t_x], line order); runs
+  // DeBERTa, the text encoder and the duration predictors only.
+  std::vector<int32_t> predict_durations_tokens(const std::string& ident, const std::vector<std::optional<ParsedTokens>>& lines,
+                                                int32_t style_id, int64_t speaker_id, const SynthesizeOptions& options);
   size_t loaded_count() const;
   Session& bert_session() { return bert_; }
 
  private:
   TTSModel* find_model(const std::string& ident);
   bool find_and_load_model(const std::string& ident);
+  sbv2_model* token_batch(const std::string& ident, const std::vector<std::optional<ParsedTokens>>& lines, int32_t style_id,
+                          int64_t speaker_id, const SynthesizeOptions& options, TokenBatch& out);
   std::vector<uint8_t> tokenizer_;
   Session bert_;
   std::vector<TTSModel> models_;

@@ -90,6 +90,18 @@ def _load() -> C.CDLL:
         "sbv2_holder_bert_features_assist": (C.c_int, [vp, pi64, pi64, i64, pi32, C.POINTER(AssistText), C.POINTER(pf), pi64]),
         "sbv2_holder_easy_synthesize_tokens_assist": (C.c_int, [vp, C.c_char_p, C.POINTER(TokenSentence), C.c_int, i64, i32, i64, f32,
                                                                 f32, f32, C.POINTER(AssistText), C.POINTER(vp), C.POINTER(sz)]),
+        "sbv2_predict_durations_batch": (C.c_int, [vp, C.POINTER(Utterance), C.c_int, pi32]),
+        "sbv2_synthesize_batch_with_durations": (C.c_int, [vp, C.POINTER(Utterance), C.c_int, C.POINTER(pi32), C.POINTER(pf), pi64,
+                                                           C.POINTER(pi32), C.POINTER(pi32)]),
+        "sbv2_predict_durations_from_tokens": (C.c_int, [vp, vp, C.POINTER(TokenUtterance), C.c_int, C.POINTER(AssistText), C.c_int,
+                                                         pi32, pi32]),
+        "sbv2_synthesize_from_tokens_with_durations": (C.c_int, [vp, vp, C.POINTER(TokenUtterance), C.c_int, C.POINTER(AssistText),
+                                                                 C.c_int, pi32, pi64, C.POINTER(pi32), pi32, C.POINTER(pf), pi64, pi64]),
+        "sbv2_holder_predict_durations_tokens": (C.c_int, [vp, C.c_char_p, C.POINTER(TokenSentence), C.c_int, i64, i32, i64, f32, f32,
+                                                           f32, C.POINTER(AssistText), pi32]),
+        "sbv2_holder_easy_synthesize_tokens_timed": (C.c_int, [vp, C.c_char_p, C.POINTER(TokenSentence), C.c_int, i64, i32, i64, f32,
+                                                               f32, f32, C.POINTER(AssistText), C.POINTER(pi32), pi32, pi64,
+                                                               C.POINTER(vp), C.POINTER(sz)]),
         "sbv2_onnx_bind_report": (C.c_int, [vp, sz, C.c_int, C.POINTER(vp)]),
         "sbv2_model_seed": (C.c_int, [vp, C.c_uint64]),
         "sbv2_synthesize_with_noise": (C.c_int, [vp, pf, pi64, pi64, pi64, i64, i64, pf, f32, f32, f32, f32, pf, pf, i64,
@@ -224,6 +236,35 @@ def _assist_texts(assists: Sequence[dict]):
         keep += [ids, mask]
         arr[k].input_ids, arr[k].attention_mask, arr[k].t_tok, arr[k].weight = _pi64(ids), _pi64(mask), ids.size, float(a["weight"])
     return arr, keep
+
+
+def _pi32(a: np.ndarray):
+    return a.ctypes.data_as(C.POINTER(C.c_int32))
+
+
+def _duration_ptrs(durations, t_x: Sequence[int]):
+    """durations[i]: int array [t_x[i]] or None (predicted) -> (int32* [B] for the C ABI, arrays it points into)"""
+    if len(durations) != len(t_x):
+        raise Sbv2Error(ERR_INVALID_ARGUMENT, "durations must have one entry per utterance")
+    arr = (C.POINTER(C.c_int32) * max(len(durations), 1))()
+    keep = []
+    for i, d in enumerate(durations):
+        if d is None:
+            continue
+        d = np.asarray(d)
+        if d.shape != (t_x[i],):
+            raise Sbv2Error(ERR_INVALID_ARGUMENT, f"durations of utterance {i} must have shape ({t_x[i]},)")
+        if not np.issubdtype(d.dtype, np.integer) or (d.size and (d.min() < -2**31 or d.max() >= 2**31)):
+            raise Sbv2Error(ERR_INVALID_ARGUMENT, f"durations of utterance {i} must be int32 integers")
+        d = np.ascontiguousarray(d, dtype=np.int32)
+        keep.append(d)
+        arr[i] = _pi32(d)
+    return arr, keep
+
+
+def _split(flat: np.ndarray, lens: Sequence[int]) -> List[np.ndarray]:
+    offs = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
+    return [flat[offs[i]:offs[i + 1]] for i in range(len(lens))]
 
 
 class _Owned:
@@ -464,6 +505,63 @@ class Model:
                                                _pf(sv), sdp_ratio, length_scale, noise_scale, noise_scale_w, C.byref(p), C.byref(n)))
         return _take(p, n.value, np.float32)
 
+    @staticmethod
+    def _token_utterances(sentences: Sequence[dict]):
+        arr = (TokenUtterance * max(len(sentences), 1))()
+        keep = []
+        for i, u in enumerate(sentences):
+            ids, w2p = _i64(u["token_ids"]), np.ascontiguousarray(u["word2ph"], dtype=np.int32)
+            mask = _i64(u.get("attention_mask", np.ones_like(ids)))
+            x, t, l, sv = _i64(u["x_tst"]), _i64(u["tones"]), _i64(u["lang_ids"]), _f32(u["style_vec"])
+            keep += [ids, mask, w2p, x, t, l, sv]
+            a = arr[i]
+            a.input_ids, a.attention_mask, a.t_tok, a.word2ph = _pi64(ids), _pi64(mask), ids.size, _pi32(w2p)
+            a.x_tst, a.tones, a.lang_ids, a.t_x = _pi64(x), _pi64(t), _pi64(l), x.size
+            a.sid, a.style_vec = int(u.get("sid", 0)), _pf(sv)
+            a.sdp_ratio, a.length_scale = float(u.get("sdp_ratio", 0.0)), float(u.get("length_scale", 1.0))
+            a.noise_scale, a.noise_scale_w = float(u.get("noise_scale", 0.677)), float(u.get("noise_scale_w", 0.8))
+        return arr, keep
+
+    @staticmethod
+    def _assist_args(sentences: Sequence[dict], assists: Optional[Sequence[dict]]):
+        """-> (AssistText array or None, n_assists, int32* assist_of or None, arrays to keep alive)"""
+        if assists is None:
+            return None, 0, None, []
+        at, akeep = _assist_texts(assists)
+        of = np.array([-1 if u.get("assist") is None else int(u["assist"]) for u in sentences], dtype=np.int32)
+        return at, len(assists), _pi32(of), akeep + [of]
+
+    def predict_durations_from_tokens(self, bert_model: "Model", sentences: Sequence[dict],
+                                      assists: Optional[Sequence[dict]] = None) -> List[np.ndarray]:
+        """Timing query of the token path (sbv2_predict_durations_from_tokens): DeBERTa, the text encoder and the duration
+        predictors only.  sentences / assists as in synthesize_from_tokens_batch.  -> durations int32 [t_x] per sentence."""
+        arr, keep = self._token_utterances(sentences)
+        at, na, of, akeep = self._assist_args(sentences, assists)
+        tx = [int(np.asarray(u["x_tst"]).size) for u in sentences]
+        out = np.zeros(sum(tx), dtype=np.int32)
+        _check(lib.sbv2_predict_durations_from_tokens(self._h, bert_model._h, arr, len(sentences), at, na, of, _pi32(out)))
+        return _split(out, tx)
+
+    def synthesize_from_tokens_with_durations(self, bert_model: "Model", sentences: Sequence[dict],
+                                              durations: Optional[Sequence[Optional[np.ndarray]]],
+                                              pause_after: Optional[Sequence[int]] = None, assists: Optional[Sequence[dict]] = None):
+        """synthesize_from_tokens_batch at given durations (durations[i]: frames per phoneme [t_x] or None = predicted;
+        durations=None: all predicted).  -> (audio [total] incl. the pauses, samples per sentence int64 [batch],
+        the durations used int32 [t_x] per sentence)"""
+        B = len(sentences)
+        arr, keep = self._token_utterances(sentences)
+        at, na, of, akeep = self._assist_args(sentences, assists)
+        tx = [int(np.asarray(u["x_tst"]).size) for u in sentences]
+        dp, dkeep = _duration_ptrs(durations, tx) if durations is not None else (None, [])
+        pa = _i64(pause_after) if pause_after is not None else None
+        p, total = C.POINTER(C.c_float)(), C.c_int64()
+        ns = np.zeros(B, dtype=np.int64)
+        dur = np.zeros(sum(tx), dtype=np.int32)
+        _check(lib.sbv2_synthesize_from_tokens_with_durations(self._h, bert_model._h, arr, B, at, na, of,
+                                                              _pi64(pa) if pa is not None else None, dp, _pi32(dur), C.byref(p),
+                                                              C.byref(total), _pi64(ns)))
+        return _take(p, total.value, np.float32), ns, _split(dur, tx)
+
     def synthesize_from_tokens_batch(self, bert_model: "Model", sentences: Sequence[dict], pause_after: Optional[Sequence[int]] = None,
                                      assists: Optional[Sequence[dict]] = None):
         """sentences[i]: dict(token_ids, word2ph, x_tst, tones, lang_ids, style_vec[, sid, sdp_ratio, length_scale,
@@ -560,6 +658,32 @@ class Model:
         xo = np.concatenate([[0], np.cumsum(tx)])
         yo = offs // hop
         return audios, [d[xo[i]:xo[i + 1]] for i in range(B)], [f[yo[i]:yo[i + 1]] for i in range(B)]
+
+    def predict_durations_batch(self, utts: Sequence[dict]) -> List[np.ndarray]:
+        """Timing query of the features path (sbv2_predict_durations_batch): the text encoder and the duration predictors
+        only.  utts as in synthesize_batch.  -> durations int32 [t_x] per utterance."""
+        arr, keep = self._utterances(utts)
+        tx = [int(u_.t_x) for u_ in arr]
+        out = np.zeros(sum(tx), dtype=np.int32)
+        _check(lib.sbv2_predict_durations_batch(self._h, arr, len(utts), _pi32(out)))
+        return _split(out, tx)
+
+    def synthesize_batch_with_durations(self, utts: Sequence[dict], durations: Optional[Sequence[Optional[np.ndarray]]]):
+        """synthesize_batch at given durations (durations[i]: frames per phoneme [t_x] or None = predicted).
+        -> (audio list, durations list, frame2ph list)"""
+        arr, keep = self._utterances(utts)
+        B = len(utts)
+        tx = [int(u_.t_x) for u_ in arr]
+        dp, dkeep = _duration_ptrs(durations, tx) if durations is not None else (None, [])
+        p = C.POINTER(C.c_float)()
+        ns = np.zeros(B, dtype=np.int64)
+        pd, pf2 = C.POINTER(C.c_int32)(), C.POINTER(C.c_int32)()
+        _check(lib.sbv2_synthesize_batch_with_durations(self._h, arr, B, dp, C.byref(p), _pi64(ns), C.byref(pd), C.byref(pf2)))
+        flat = _take(p, int(ns.sum()), np.float32)
+        hop = self.describe()["hop"]
+        d = _take(pd, sum(tx), np.int32)
+        f = _take(pf2, int(ns.sum() // hop), np.int32)
+        return _split(flat, ns), _split(d, tx), _split(f, ns // hop)
 
     def decode_batch(self, zs: Sequence[np.ndarray], sids: Optional[Sequence[int]] = None) -> List[np.ndarray]:
         """HiFi-GAN decoder alone: zs[b] float32 [192, T_y[b]]."""
@@ -714,6 +838,54 @@ class TTSModelHolder:
         out = C.string_at(p, n.value)
         lib.sbv2_free(p)
         return out
+
+    @staticmethod
+    def _token_sentences(lines: Sequence[Optional[dict]]):
+        sent = [(i, l) for i, l in enumerate(lines) if l is not None]
+        arr = (TokenSentence * max(len(sent), 1))()
+        keep = []
+        for j, (i, l) in enumerate(sent):
+            ids, w2p = _i64(l["token_ids"]), np.ascontiguousarray(l["word2ph"], dtype=np.int32)
+            mask = _i64(l.get("attention_mask", np.ones_like(ids)))
+            ph, t, lg = _i64(l["phones"]), _i64(l["tones"]), _i64(l["lang_ids"])
+            keep += [ids, mask, w2p, ph, t, lg]
+            a = arr[j]
+            a.token_ids, a.attention_mask, a.word2ph, a.t_tok = _pi64(ids), _pi64(mask), _pi32(w2p), ids.size
+            a.phones, a.tones, a.lang_ids, a.t_x, a.line_index = _pi64(ph), _pi64(t), _pi64(lg), ph.size, i
+        return sent, arr, keep
+
+    def predict_durations_tokens(self, ident: str, lines: Sequence[Optional[dict]], style_id: int, speaker_id: int,
+                                 sdp_ratio: float = 0.0, length_scale: float = 1.0, style_weight: float = 1.0,
+                                 assist: Optional[dict] = None) -> List[np.ndarray]:
+        """Timing of a request ("audio query"), lines as in easy_synthesize_tokens.  -> durations int32 [t_x] per non-empty
+        line, in frames of ``hop`` samples."""
+        sent, arr, keep = self._token_sentences(lines)
+        at, akeep = _assist_texts([assist]) if assist is not None else (None, [])
+        tx = [int(np.asarray(l["phones"]).size) for _, l in sent]
+        out = np.zeros(sum(tx), dtype=np.int32)
+        _check(lib.sbv2_holder_predict_durations_tokens(self._h, ident.encode(), arr, len(sent), len(lines), style_id, speaker_id,
+                                                        sdp_ratio, length_scale, style_weight, at, _pi32(out)))
+        return _split(out, tx)
+
+    def easy_synthesize_tokens_timed(self, ident: str, lines: Sequence[Optional[dict]], style_id: int, speaker_id: int,
+                                     sdp_ratio: float = 0.0, length_scale: float = 1.0, style_weight: float = 1.0,
+                                     assist: Optional[dict] = None, durations: Optional[Sequence[Optional[np.ndarray]]] = None):
+        """easy_synthesize_tokens at given durations (one entry per non-empty line: frames per phoneme [t_x] or None =
+        predicted; durations=None: all predicted).  -> (WAV bytes, durations int32 [t_x] per non-empty line, index of each
+        phoneme's first sample in the WAV's sample data int64 [t_x] per non-empty line)"""
+        sent, arr, keep = self._token_sentences(lines)
+        at, akeep = _assist_texts([assist]) if assist is not None else (None, [])
+        tx = [int(np.asarray(l["phones"]).size) for _, l in sent]
+        dp, dkeep = _duration_ptrs(durations, tx) if durations is not None else (None, [])
+        dur = np.zeros(sum(tx), dtype=np.int32)
+        start = np.zeros(sum(tx), dtype=np.int64)
+        p, n = C.c_void_p(), C.c_size_t()
+        _check(lib.sbv2_holder_easy_synthesize_tokens_timed(self._h, ident.encode(), arr, len(sent), len(lines), style_id, speaker_id,
+                                                            sdp_ratio, length_scale, style_weight, at, dp, _pi32(dur), _pi64(start),
+                                                            C.byref(p), C.byref(n)))
+        out = C.string_at(p, n.value)
+        lib.sbv2_free(p)
+        return out, _split(dur, tx), _split(start, tx)
 
     def easy_synthesize(self, ident: str, lines: Sequence[Optional[dict]], style_id: int, speaker_id: int,
                         sdp_ratio: float = 0.0, length_scale: float = 1.0, style_weight: float = 1.0) -> bytes:
