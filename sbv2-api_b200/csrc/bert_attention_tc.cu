@@ -610,7 +610,7 @@ __global__ void __launch_bounds__(160, 1) deberta_attention_tc_multi_kernel(__ha
 // two-term fp16 split x = h0 + h1 (the plane blocks [h0 | h1 | h0] the split GEMMs exchange), every product is the three
 // cross terms h0 g0 + h0 g1 + h1 g0 accumulated in fp32, the position-bias windows go through ONE fp32 shared-memory tile
 // (c2p written, p2c added), and the probabilities are split as well before P V.  Replaces the fp32 CUDA-core kernel
-// (deberta_attention_kernel<true>) there; measured error against it: see tests/test_gpu_bert.py.
+// (deberta_attention_kernel<true>) there; both against float64: tests/test_gpu_bert_attention_short.py.
 //   qkv_s : split planar [h0 | h1 | h0] x [3 * heads * 8 planes][rows][8], values scaled by sc (power of two)
 //   pos_*_s: fp16 [2 terms][heads][8][n_pos][8], scaled by sc
 //   out_s : split planar ctx [h0 | h1 | h0] x [heads * 8 planes], scaled by sc (= V's scale: O needs no rescaling)

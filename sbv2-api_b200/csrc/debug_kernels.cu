@@ -670,70 +670,98 @@ extern "C" int sbv2_debug_bert_bucket_table(int span, int* max_rel, int* out) {
   });
 }
 
+namespace {
+
+// fp32 position table [n_pos][H] -> [H][n_pos], the layout the CUDA-core kernels read
+std::vector<float> transpose_pos(const float* pos, int n_pos, int H) {
+  std::vector<float> t(size_t(H) * n_pos);
+  for (int r = 0; r < n_pos; ++r)
+    for (int c = 0; c < H; ++c) t[size_t(c) * n_pos + r] = pos[size_t(r) * H + c];
+  return t;
+}
+
+// Ragged batch of DeBERTa utterances (1 ... kMaxBertTokens tokens each) and the planar segments the attention reads.
+PlanarSegs deberta_ragged(sbv2_model& owner, const int* lens, int n, Ragged* R) {
+  SBV2_REQUIRE(lens && n > 0, "need at least one utterance");
+  for (int b = 0; b < n; ++b) SBV2_REQUIRE(lens[b] >= 1 && lens[b] <= kMaxBertTokens, "utterance lengths must be in [1, 32768]");
+  ragged(owner, lens, n, R);
+  return planar_segs(*R, n);
+}
+
+}  // namespace
+
 // One DeBERTa disentangled attention launch (head dim 64) on a ragged batch, with the bucket table of `span`.
 //   qkv   fp16 row-major [terms][sum(lens)][3 * heads * 64] (q | k | v, channel h * 64 + d)
 //   pos_k, pos_q  fp16 row-major [terms][2 * span][heads * 64]: the position projections
 //   mode  0: single-tile tensor-core kernel (<= 128 tokens), 1: multi-tile tensor-core kernel, 2: its exact variant, whose
-//         operands are the two fp16 terms (terms = 2) of values scaled by sc, 3: CUDA-core kernel; terms = 1 except in mode 2
+//         operands are the two fp16 terms (terms = 2) of values scaled by sc, 3: CUDA-core kernel, 4: the exact single-tile
+//         kernel (<= 128 tokens; operands as mode 2); terms = 2 in modes 2 and 4, else 1
 //   far_pairs  modes 1 and 2: far tile pairs take the reduced path (0: the generic path for every pair)
-//   out   fp16 row-major [terms][sum(lens)][heads * 64]: the context (mode 2: the two terms of context * sc)
+//   pad_seed  0: the planar input rows of no utterance (the gaps and the tail) hold zeros, as a freshly cleared buffer;
+//         else they hold finite fp16 values drawn from this seed, as rows that an earlier, longer batch left behind
+//   out   fp16 row-major [blocks][sum(lens)][heads * 64]: the context (modes 2 and 4: the plane blocks [h0 | h1 | h0] of
+//         context * sc); blocks = 1, or in modes 2 and 4 out_blocks = 2 (the two terms) or 3 (all three blocks)
 //   reps > 0: the launch is then repeated `reps` times between two CUDA events and *ms receives the mean time per launch
-// The planar rows of no utterance hold zeros, as the model keeps them.
+//   stray (or null): stray[0] <- planar rows outside every utterance written into any of the three output blocks, which
+//         hold kHalfSentinel before the launch
 extern "C" int sbv2_debug_deberta_attention(const uint16_t* qkv, const uint16_t* pos_k, const uint16_t* pos_q, const int* lens, int n,
-                                            int heads, int span, int mode, int far_pairs, float sc, int reps, float* ms, uint16_t* out) {
+                                            int heads, int span, int mode, int far_pairs, float sc, unsigned long long pad_seed,
+                                            int out_blocks, int reps, float* ms, uint16_t* out, long long* stray) {
   return guarded([&] {
-    SBV2_REQUIRE(qkv && pos_k && pos_q && lens && out && n > 0 && heads > 0 && mode >= 0 && mode <= 3, "bad arguments");
-    SBV2_REQUIRE(mode != 2 || sc > 0.f, "the exact kernel needs the split scale");
+    SBV2_REQUIRE(qkv && pos_k && pos_q && lens && out && n > 0 && heads > 0 && mode >= 0 && mode <= 4, "bad arguments");
+    const bool exact = mode == 2 || mode == 4;
+    SBV2_REQUIRE(!exact || sc > 0.f, "the exact kernels need the split scale");
+    SBV2_REQUIRE(exact ? (out_blocks == 2 || out_blocks == 3) : out_blocks == 1, "out_blocks: 2 or 3 in modes 2 and 4, else 1");
     SBV2_REQUIRE(reps <= 0 || ms != nullptr, "timing needs *ms");
     sbv2_model owner;
     open_owner(owner);
     const LaunchCtx ctx = owner.ctx();
-    std::vector<int> ystart(lens, lens + n), ylen(lens, lens + n), muls{1};
-    long long rows = 0;
-    for (int b = 0; b < n; ++b) {
-      SBV2_REQUIRE(lens[b] >= 1 && lens[b] <= kMaxBertTokens, "utterance lengths must be in [1, 32768]");
-      ystart[size_t(b)] = int(rows);
-      rows += lens[b];
-      SBV2_REQUIRE(rows < INT_MAX, "too many rows");
-    }
+    Ragged R;
+    const PlanarSegs ps = deberta_ragged(owner, lens, n, &R);
+    const Geom& G = R.g();
+    const long long rows = R.rows;
     int max_rel = 0;
     const std::vector<int> tab = bert_bucket_table(span, &max_rel);
-    DBuf meta;
-    PinnedBuf pin;
-    meta.stream = owner.stream;
-    BatchGeom bg = build_geoms(&owner, meta, pin, ystart, ylen, muls);
-    const Geom& G = bg.g[0];
-    const int H = heads * 64, C3 = 3 * H, terms = mode == 2 ? 2 : 1, n_pos = 2 * span;
+    const int H = heads * 64, C3 = 3 * H, terms = exact ? 2 : 1, n_pos = 2 * span;
     const size_t plane = size_t(G.rows_tot) * 8, qkv_blk = size_t(C3 / 8) * plane, ctx_blk = size_t(H / 8) * plane;
     std::vector<uint16_t> hq(terms * qkv_blk, 0);
+    if (pad_seed != 0) {
+      uint64_t st = pad_seed;
+      for (int term = 0; term < terms; ++term)
+        for (int pl = 0; pl < C3 / 8; ++pl)
+          for (size_t pr = 0; pr < size_t(G.rows_tot); ++pr) {
+            if (R.in_utt[pr]) continue;
+            for (int e = 0; e < 8; ++e) {
+              st += 0x9E3779B97F4A7C15ull;  // splitmix64
+              uint64_t z = st;
+              z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+              z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+              uint16_t u = uint16_t(z ^ (z >> 31));
+              if ((u & 0x7C00) == 0x7C00) u ^= 0x4000;  // Inf / NaN exponent -> a finite value
+              hq[term * qkv_blk + size_t(pl) * plane + pr * 8 + e] = u;
+            }
+          }
+    }
     for (int term = 0; term < terms; ++term)
       for (int b = 0; b < n; ++b)
         for (int t = 0; t < lens[b]; ++t) {
           const size_t pr = size_t(G.pstart[size_t(b)]) + t;
-          const uint16_t* src = qkv + (size_t(term) * rows + ystart[size_t(b)] + t) * C3;
+          const uint16_t* src = qkv + (size_t(term) * rows + R.ystart[size_t(b)] + t) * C3;
           for (int c = 0; c < C3; ++c) hq[term * qkv_blk + size_t(c / 8) * plane + pr * 8 + c % 8] = src[c];
         }
-    std::vector<uint16_t> ho(3 * ctx_blk, 0);
+    std::vector<uint16_t> ho(3 * ctx_blk, kHalfSentinel);
     const __half* d_qkv = reinterpret_cast<const __half*>(upload(owner, hq.data(), hq.size()));
     __half* d_out = reinterpret_cast<__half*>(upload(owner, ho.data(), ho.size()));
     const int* d_tab = upload(owner, tab.data(), tab.size());
-    PlanarSegs ps;
-    ps.start = bg.d_ystart;
-    ps.pstart = G.d_pstart;
-    ps.len = G.d_len;
-    ps.order = bg.d_order;
-    ps.n = n;
-    ps.max_len = G.max_len;
-    ps.plane_stride = G.rows_tot * 8;
     std::function<void()> launch;
     if (mode == 3) {
       // the CUDA-core kernel reads fp32 tables transposed to [heads * 64][n_pos]
-      std::vector<float> tk(size_t(H) * n_pos), tq(tk.size());
-      for (int r = 0; r < n_pos; ++r)
-        for (int c = 0; c < H; ++c) {
-          tk[size_t(c) * n_pos + r] = __half2float(__ushort_as_half(pos_k[size_t(r) * H + c]));
-          tq[size_t(c) * n_pos + r] = __half2float(__ushort_as_half(pos_q[size_t(r) * H + c]));
-        }
+      std::vector<float> fk(size_t(n_pos) * H), fq(fk.size());
+      for (size_t i = 0; i < fk.size(); ++i) {
+        fk[i] = __half2float(__ushort_as_half(pos_k[i]));
+        fq[i] = __half2float(__ushort_as_half(pos_q[i]));
+      }
+      const std::vector<float> tk = transpose_pos(fk.data(), n_pos, H), tq = transpose_pos(fq.data(), n_pos, H);
       const float* d_tk = upload(owner, tk.data(), tk.size());
       const float* d_tq = upload(owner, tq.data(), tq.size());
       launch = [&, d_tk, d_tq] { launch_deberta_attention(ctx, d_out, d_qkv, d_tk, d_tq, n_pos, d_tab, max_rel, heads, 64, ps); };
@@ -752,9 +780,11 @@ extern "C" int sbv2_debug_deberta_attention(const uint16_t* qkv, const uint16_t*
       launch = [&, d_pk, d_pq] {
         if (mode == 0) launch_deberta_attention_tc(ctx, d_out, d_qkv, d_pk, d_pq, n_pos, span, heads, ps);
         else if (mode == 1) launch_deberta_attention_tc_multi(ctx, d_out, d_qkv, d_pk, d_pq, n_pos, d_tab, max_rel, heads, far_pairs != 0, ps);
-        else
+        else if (mode == 2)
           launch_deberta_attention_tc_exact_multi(ctx, d_out, (long long)ctx_blk, d_qkv, (long long)qkv_blk, d_pk, d_pq, n_pos, d_tab, max_rel,
                                                   heads, sc, far_pairs != 0, ps);
+        else
+          launch_deberta_attention_tc_exact(ctx, d_out, (long long)ctx_blk, d_qkv, (long long)qkv_blk, d_pk, d_pq, n_pos, span, heads, sc, ps);
       };
     }
     launch();
@@ -772,12 +802,71 @@ extern "C" int sbv2_debug_deberta_attention(const uint16_t* qkv, const uint16_t*
       CUDA_CHECK(cudaEventDestroy(e1));
     }
     download(owner, ho.data(), reinterpret_cast<const uint16_t*>(d_out), ho.size());
-    for (int term = 0; term < terms; ++term)
-      for (int b = 0; b < n; ++b)
-        for (int t = 0; t < lens[b]; ++t) {
-          const size_t pr = size_t(G.pstart[size_t(b)]) + t;
-          uint16_t* dst = out + (size_t(term) * rows + ystart[size_t(b)] + t) * H;
-          for (int c = 0; c < H; ++c) dst[c] = ho[term * ctx_blk + size_t(c / 8) * plane + pr * 8 + c % 8];
-        }
+    std::vector<uint16_t> blk(ctx_blk);
+    for (int k = 0; k < out_blocks; ++k) {
+      std::copy(ho.begin() + k * ctx_blk, ho.begin() + (k + 1) * ctx_blk, blk.begin());
+      unplanar(out + size_t(k) * rows * H, blk, H / 8, R, n);
+    }
+    if (stray) stray[0] = stray_rows(ho, 3 * H / 8, R);
+  });
+}
+
+// The fp32 CUDA-core attention (launch_deberta_attention_f32, deberta_attention_kernel<true>: the exact mode's kernel
+// beyond what the exact tensor-core kernels take, and their cross-check) on a ragged batch, with the bucket table of `span`.
+//   qkv   fp32 row-major [sum(lens)][3 * heads * 64] (q | k | v, channel h * 64 + d)
+//   pos_k, pos_q  fp32 row-major [2 * span][heads * 64], transposed on the host to the [heads * 64][2 * span] it reads
+//   out   (or null) fp32 row-major [sum(lens)][heads * 64] <- the context; the buffer holds an fp32 NaN payload before,
+//         and 128 rows past the last utterance more
+//   split (or null) fp16 [3][sum(lens)][heads * 64] <- the plane blocks [h0 | h1 | h0] of context * split_scale that the
+//         split output (ctx_split) writes, from a launch of its own
+//   stray (or null): stray[0] <- planar rows outside every utterance written into the split planes (kHalfSentinel before)
+//         plus the rows past the last utterance written into out
+extern "C" int sbv2_debug_deberta_attention_f32(const float* qkv, const float* pos_k, const float* pos_q, const int* lens, int n, int heads,
+                                                int span, float split_scale, float* out, uint16_t* split, long long* stray) {
+  return guarded([&] {
+    SBV2_REQUIRE(qkv && pos_k && pos_q && (out || split) && heads > 0, "bad arguments");
+    SBV2_REQUIRE(!split || split_scale > 0.f, "the split output needs its scale");
+    sbv2_model owner;
+    open_owner(owner);
+    const LaunchCtx ctx = owner.ctx();
+    Ragged R;
+    const PlanarSegs ps = deberta_ragged(owner, lens, n, &R);
+    const long long rows = R.rows;
+    int max_rel = 0;
+    const std::vector<int> tab = bert_bucket_table(span, &max_rel);
+    const int H = heads * 64, n_pos = 2 * span;
+    const float* d_qkv = upload(owner, qkv, size_t(rows) * 3 * H);
+    const std::vector<float> tk = transpose_pos(pos_k, n_pos, H), tq = transpose_pos(pos_q, n_pos, H);
+    const float* d_tk = upload(owner, tk.data(), tk.size());
+    const float* d_tq = upload(owner, tq.data(), tq.size());
+    const int* d_tab = upload(owner, tab.data(), tab.size());
+    long long written = 0;
+    if (out) {
+      const size_t tail = size_t(128) * H, elems = size_t(rows) * H;
+      std::vector<uint32_t> ho(elems + tail, kFloatSentinel);
+      float* d_out = reinterpret_cast<float*>(upload(owner, ho.data(), ho.size()));
+      launch_deberta_attention_f32(ctx, d_out, nullptr, 0.f, d_qkv, d_tk, d_tq, n_pos, d_tab, max_rel, heads, 64, ps);
+      download(owner, ho.data(), reinterpret_cast<const uint32_t*>(d_out), ho.size());
+      memcpy(out, ho.data(), elems * sizeof(float));
+      for (size_t r = 0; r < 128; ++r) {
+        bool w = false;
+        for (int c = 0; c < H; ++c) w |= ho[elems + r * H + c] != kFloatSentinel;
+        written += w ? 1 : 0;
+      }
+    }
+    if (split) {
+      const size_t ctx_blk = size_t(H / 8) * R.g().rows_tot * 8;
+      std::vector<uint16_t> hs(3 * ctx_blk, kHalfSentinel);
+      __half* d_s = reinterpret_cast<__half*>(upload(owner, hs.data(), hs.size()));
+      launch_deberta_attention_f32(ctx, nullptr, d_s, split_scale, d_qkv, d_tk, d_tq, n_pos, d_tab, max_rel, heads, 64, ps);
+      download(owner, hs.data(), reinterpret_cast<const uint16_t*>(d_s), hs.size());
+      std::vector<uint16_t> blk(ctx_blk);
+      for (int k = 0; k < 3; ++k) {
+        std::copy(hs.begin() + k * ctx_blk, hs.begin() + (k + 1) * ctx_blk, blk.begin());
+        unplanar(split + size_t(k) * rows * H, blk, H / 8, R, n);
+      }
+      written += stray_rows(hs, 3 * H / 8, R);
+    }
+    if (stray) stray[0] = written;
   });
 }

@@ -155,7 +155,7 @@ _debug_lib = None
 def debug_lib() -> C.CDLL:
     """libsbv2_b200_debug.so: the same objects plus the kernel unit-test / tracing hooks (sbv2_debug_conv_compare,
     _conv_trace, _pair_compare, _attn_trace, _mma_rate*, _flow_attention, _rel_attention, _convflow_spline, _durations,
-    _umma_layer, _dec_post, _bert_bucket_table, _deberta_attention), which the product library does not export."""
+    _umma_layer, _dec_post, _bert_bucket_table, _deberta_attention, _deberta_attention_f32), which the product library does not export."""
     global _debug_lib
     if _debug_lib is None:
         path = os.path.join(_HERE, "libsbv2_b200_debug.so")
@@ -182,27 +182,56 @@ def debug_bert_bucket_table(span: int) -> np.ndarray:
     return out
 
 
-DEBERTA_ATTN_MODES = {"single": 0, "multi": 1, "exact-multi": 2, "simt": 3}
+DEBERTA_ATTN_MODES = {"single": 0, "multi": 1, "exact-multi": 2, "simt": 3, "exact-single": 4}
+DEBERTA_ATTN_EXACT = ("exact-multi", "exact-single")
 
 
 def debug_deberta_attention(qkv: np.ndarray, pos_k: np.ndarray, pos_q: np.ndarray, lens, heads: int, mode: str,
-                            far_pairs: bool = True, sc: float = 16.0, reps: int = 0):
+                            far_pairs: bool = True, sc: float = 16.0, reps: int = 0, *, all_blocks: bool = False,
+                            pad_seed: int = 0, with_stray: bool = False):
     """One DeBERTa attention launch (sbv2_debug_deberta_attention) on a ragged batch: qkv fp16 [terms, sum(lens), 3*heads*64],
-    pos_k / pos_q fp16 [terms, 2*span, heads*64]; terms = 2 (the split terms of values scaled by sc) for mode "exact-multi",
-    else 1.  Returns the context, fp16 [terms, sum(lens), heads*64] (exact-multi: the two terms of context * sc); with
-    reps > 0, (context, mean ms of `reps` more launches timed with CUDA events)."""
-    terms = 2 if mode == "exact-multi" else 1
+    pos_k / pos_q fp16 [terms, 2*span, heads*64]; terms = 2 (the split terms of values scaled by sc) for the exact modes
+    ("exact-multi", "exact-single"), else 1.  Returns the context, fp16 [terms, sum(lens), heads*64] (exact modes: the two
+    terms of context * sc; with all_blocks, the three plane blocks [h0 | h1 | h0]); with reps > 0, (context, mean ms of
+    `reps` more launches timed with CUDA events).  pad_seed != 0 fills the planar input rows outside every utterance with
+    finite fp16 values drawn from it (else zeros).  with_stray appends the number of planar rows outside every utterance
+    that the launch wrote to the returned tuple."""
+    exact = mode in DEBERTA_ATTN_EXACT
+    terms = 2 if exact else 1
+    blocks = (3 if all_blocks else 2) if exact else 1
     lens_a = np.ascontiguousarray(lens, dtype=np.int32)
     qkv = np.ascontiguousarray(qkv, dtype=np.float16).reshape(terms, int(lens_a.sum()), 3 * heads * 64)
     pos_k = np.ascontiguousarray(pos_k, dtype=np.float16).reshape(terms, -1, heads * 64)
     pos_q = np.ascontiguousarray(pos_q, dtype=np.float16).reshape(pos_k.shape)
-    out = np.zeros((terms, int(lens_a.sum()), heads * 64), np.float16)
-    u16, ms = C.POINTER(C.c_uint16), C.c_float(0.0)
+    out = np.zeros((blocks, int(lens_a.sum()), heads * 64), np.float16)
+    u16, ms, stray = C.POINTER(C.c_uint16), C.c_float(0.0), C.c_longlong(0)
     _debug_check(debug_lib().sbv2_debug_deberta_attention(
         qkv.ctypes.data_as(u16), pos_k.ctypes.data_as(u16), pos_q.ctypes.data_as(u16), lens_a.ctypes.data_as(C.POINTER(C.c_int)),
-        len(lens_a), heads, pos_k.shape[1] // 2, DEBERTA_ATTN_MODES[mode], int(bool(far_pairs)), C.c_float(sc), reps, C.byref(ms),
-        out.ctypes.data_as(u16)))
-    return (out, ms.value) if reps > 0 else out
+        len(lens_a), heads, pos_k.shape[1] // 2, DEBERTA_ATTN_MODES[mode], int(bool(far_pairs)), C.c_float(sc),
+        C.c_ulonglong(pad_seed), blocks, reps, C.byref(ms), out.ctypes.data_as(u16), C.byref(stray)))
+    res = (out,) + ((ms.value,) if reps > 0 else ()) + ((stray.value,) if with_stray else ())
+    return res[0] if len(res) == 1 else res
+
+
+def debug_deberta_attention_f32(qkv: np.ndarray, pos_k: np.ndarray, pos_q: np.ndarray, lens, heads: int, *, out: bool = True,
+                                split_scale: float = 0.0):
+    """The fp32 CUDA-core DeBERTa attention (sbv2_debug_deberta_attention_f32) on a ragged batch: qkv fp32
+    [sum(lens), 3*heads*64], pos_k / pos_q fp32 [2*span, heads*64].  Returns (context fp32 [sum(lens), heads*64] or None
+    when not `out`, the split output fp16 [3, sum(lens), heads*64] = the plane blocks [h0 | h1 | h0] of context *
+    split_scale or None when split_scale is 0, rows written outside the utterances)."""
+    lens_a = np.ascontiguousarray(lens, dtype=np.int32)
+    H = heads * 64
+    qkv = np.ascontiguousarray(qkv, dtype=np.float32).reshape(int(lens_a.sum()), 3 * H)
+    pos_k = np.ascontiguousarray(pos_k, dtype=np.float32).reshape(-1, H)
+    pos_q = np.ascontiguousarray(pos_q, dtype=np.float32).reshape(pos_k.shape)
+    ctx = np.zeros((int(lens_a.sum()), H), np.float32) if out else None
+    split = np.zeros((3, int(lens_a.sum()), H), np.float16) if split_scale > 0 else None
+    f32p, stray = C.POINTER(C.c_float), C.c_longlong(0)
+    _debug_check(debug_lib().sbv2_debug_deberta_attention_f32(
+        qkv.ctypes.data_as(f32p), pos_k.ctypes.data_as(f32p), pos_q.ctypes.data_as(f32p), lens_a.ctypes.data_as(C.POINTER(C.c_int)),
+        len(lens_a), heads, pos_k.shape[0] // 2, C.c_float(split_scale), None if ctx is None else ctx.ctypes.data_as(f32p),
+        None if split is None else split.ctypes.data_as(C.POINTER(C.c_uint16)), C.byref(stray)))
+    return ctx, split, stray.value
 
 
 def _check(status: int) -> None:
